@@ -10,6 +10,12 @@ batch of 64 synthetic 2-channel 48x48 LR tiles per GPU: bicubic down of the HR b
 loss, backward, fused Adam.  Prints ONE JSON line (rank 0).  Besides the headline (BASELINE config 2 / 3) the line
 carries `infer_region` (config 4: tile extraction, batched forward, stitching of a 3000 x 17280 region, host images out)
 and `x8` (config 5: x8 upscaling of 4-channel 96 x 96 tiles); `--skip-extras` leaves them out.
+
+`--dump-outputs DIR` (CUDA arm, rank 0) writes what the last timed training step computed to DIR/*.npy, float32:
+`loss` (what train_step returned), `prediction` (the model output it was computed from, 64 x 2 x 192 x 192), and
+`params_sample` / `grads_sample` (the updated parameters and their gradients at a fixed, seeded set of 2^20 of the
+16.3 M flat indices).  Inputs and initial weights are seeded, so two builds run with the same arguments can be compared
+output for output.
 """
 import argparse
 import json
@@ -77,6 +83,21 @@ def synth_hr(B, C, S, seed):
     import torch
     g = torch.Generator().manual_seed(seed)
     return torch.randn(B, C, S, S, generator=g)
+
+
+DUMP_SAMPLE = 1 << 20   # parameters / gradients sampled per dump: the full flat buffers are 65 MB each
+
+
+def dump_outputs(dirname, loss, prediction, eng):
+    """Write the last training step's results as float32 .npy files (see the module docstring)."""
+    import numpy as np
+    import torch
+    idx = torch.randperm(eng.n_params, generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values
+    idx = idx.to(eng.flat.device)
+    arrays = {"loss": loss.reshape(1), "prediction": prediction, "params_sample": eng.flat[idx], "grads_sample": eng.flat_grad[idx]}
+    os.makedirs(dirname, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), t.detach().float().cpu().numpy())
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -353,13 +374,19 @@ def run_cuda(args):
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
+    captured, hook = {}, None
+    if args.dump_outputs and rank == 0:   # keeps the model output of each step (train_step returns only the loss)
+        hook = model.register_forward_hook(lambda mod, inp, out: captured.update(prediction=out.detach()))
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for i in range(args.steps):
-        step(resident[i % nbuf])
+        loss = step(resident[i % nbuf])
     e1.record()
     sync_all()
     clocks = sampler.stop() if rank == 0 else None
+    if hook is not None:
+        hook.remove()
+        dump_outputs(args.dump_outputs, loss, captured.pop("prediction"), eng)
     ms = e0.elapsed_time(e1)
     t = torch.tensor([ms], device=dev, dtype=torch.float64)
     if world > 1:
@@ -515,7 +542,13 @@ def main():
     ap.add_argument("--impl", default="cuda", choices=["cuda", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--skip-extras", action="store_true", help="leave out the config-4 / config-5 keys (and config 1 of the reference arm)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's loss, prediction and parameter / gradient "
+                                                          "samples to DIR/*.npy (CUDA arm)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "cuda":
+        ap.error("--dump-outputs applies to the CUDA arm")
     args.warmup = max(args.warmup, 3) if args.impl == "cuda" else args.warmup
     if args.impl == "reference":
         run_reference(args)
