@@ -191,7 +191,7 @@ typedef struct sres_wgrad_job {
   const void* dy_bf16;     /* gradient of the conv output, bf16 PTL                              */
   float* dw_oihw;          /* fp32 (cout_total, 64, 3, 3)                                        */
   float* dbias;            /* fp32 (cout_total) or NULL                                          */
-  int32_t cout_total, oc_stride, oc_offset, accumulate;
+  int32_t cout_total, oc_stride, oc_offset, accumulate;   /* cout_total >= 1, oc_stride >= 1, 0 <= oc_offset < oc_stride */
   float scale;             /* result multiplier (1 for a plain conv; EDSR's res_scale for conv2) */
 } sres_wgrad_job;
 SRES_API int sres_conv3x3_wgrad_batch(const sres_wgrad_job* jobs, int njobs, int B, int H, int W, void* workspace,

@@ -16,7 +16,7 @@
 // reads from shared memory -- the resource that bounds this kernel.  (dY's padding rows are zero, so the rows the
 // shifted window drops at the very end of the buffer contribute nothing.)
 //
-// Up to 4 independent weight gradients ("jobs": different layers of the backward pass) share one
+// Up to SRES_WGRAD_MAX_JOBS (8) independent weight gradients ("jobs": different layers of the backward pass) share one
 // launch: CTA c works on job c % njobs and reduces every nsplit-th 128-position chunk of it.  Fewer
 // split-K partials per job means less partial traffic and the per-launch cost (prologue, accumulator
 // drain) is paid once per batch.  Each CTA TMA-stores its fp32 partial [5][128][64] (+ the bias-gradient
@@ -346,6 +346,14 @@ extern "C" int sres_conv3x3_wgrad_batch(const sres_wgrad_job* jobs, int njobs, i
   if (!jobs || njobs < 1 || njobs > kWgMaxJobs) return set_error(SRES_ERR_INVALID_ARG, "wgrad: 1..8 jobs per batch");
   if (!workspace) return set_error(SRES_ERR_INVALID_ARG, "wgrad: null workspace");
   if (B <= 0 || H <= 0 || W <= 0) return set_error(SRES_ERR_INVALID_ARG, "wgrad: bad geometry");
+  // Checked before anything touches the device: with oc_stride 0 the reduce's 64 threads of a row would race on one
+  // element, and an offset outside [0, oc_stride) would write into another sub-convolution's rows.
+  for (int j = 0; j < njobs; ++j) {
+    const sres_wgrad_job& J = jobs[j];
+    if (!J.x_bf16 || !J.dy_bf16 || !J.dw_oihw) return set_error(SRES_ERR_INVALID_ARG, "wgrad: null pointer in job");
+    if (J.cout_total < 1 || J.oc_stride < 1 || J.oc_offset < 0 || J.oc_offset >= J.oc_stride)
+      return set_error(SRES_ERR_INVALID_ARG, "wgrad: need cout_total >= 1, oc_stride >= 1 and 0 <= oc_offset < oc_stride");
+  }
   WgradKParams p{};
   p.P = W + 1;
   const long long npos = (long long)B * (H + 1) * (W + 1);
@@ -407,7 +415,6 @@ extern "C" int sres_conv3x3_wgrad_batch(const sres_wgrad_job* jobs, int njobs, i
   WgMaps maps;
   for (int j = 0; j < kWgMaxJobs; ++j) {
     const sres_wgrad_job& J = jobs[j < njobs ? j : 0];
-    if (!J.x_bf16 || !J.dy_bf16 || !J.dw_oihw) return set_error(SRES_ERR_INVALID_ARG, "wgrad: null pointer in job");
     int rc = make_tmap_rows64(&maps.x[j], J.x_bf16, (uint64_t)p.npos, (uint32_t)p.xbox);
     if (rc) return rc;
     rc = make_tmap_rows64(&maps.dy[j], J.dy_bf16, (uint64_t)p.npos, (uint32_t)p.dybox);

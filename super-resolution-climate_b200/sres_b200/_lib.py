@@ -56,6 +56,15 @@ class ChainArgs(C.Structure):
     ]
 
 
+class WgradJob(C.Structure):
+    """sres_wgrad_job (include/sres_b200.h)."""
+    _fields_ = [
+        ("x_bf16", C.c_void_p), ("dy_bf16", C.c_void_p), ("dw_oihw", C.c_void_p), ("dbias", C.c_void_p),
+        ("cout_total", C.c_int32), ("oc_stride", C.c_int32), ("oc_offset", C.c_int32), ("accumulate", C.c_int32),
+        ("scale", C.c_float),
+    ]
+
+
 _lib = None
 
 

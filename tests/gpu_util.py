@@ -30,6 +30,36 @@ def rel_l2(a: torch.Tensor, b: torch.Tensor) -> float:
     return ((a.double() - b.double()).norm() / (b.double().norm() + 1e-30)).item()
 
 
+def conv3x3_wgrad_ref(x: torch.Tensor, dy: torch.Tensor):
+    """Weight gradient of a 3x3, padding-1 convolution in float64 as nine shifted reductions,
+    dW[o,i,ky,kx] = sum_{b,y,x} dy[b,o,y,x] * xpad[b,i,y+ky,x+kx], and the same reduction over |x|, |dy| (the scale
+    against which the fp32 rounding of each element is judged).  x (B,Ci,H,W), dy (B,Co,H,W) -> two (Co,Ci,3,3)."""
+    H, W = dy.shape[2:]
+    xp = torch.nn.functional.pad(x.double(), (1, 1, 1, 1))
+    d = dy.double()
+    dw = torch.empty(dy.shape[1], x.shape[1], 3, 3, dtype=torch.float64, device=dy.device)
+    A = torch.empty_like(dw)
+    for ky in range(3):
+        for kx in range(3):
+            xs = xp[:, :, ky:ky + H, kx:kx + W]
+            dw[:, :, ky, kx] = torch.tensordot(d, xs, dims=([0, 2, 3], [0, 2, 3]))
+            A[:, :, ky, kx] = torch.tensordot(d.abs(), xs.abs(), dims=([0, 2, 3], [0, 2, 3]))
+    return dw, A
+
+
+def check_grad(name, got, ref, A, rel_bound, elem=2.0 ** -12):
+    """Compare a kernel's gradient tensor with its float64 reference: rel-L2 below `rel_bound` and every element within
+    `elem` * A (A = the reduction over absolute values).  Prints both measured numbers (visible with pytest -s)."""
+    d = (got.double() - ref.double()).abs()
+    rel = (d.norm() / (ref.double().norm() + 1e-300)).item()
+    worst = (d / A.double().clamp_min(1e-300)).max().item()
+    print(f"  {name:<44s} rel-L2 {rel:.2e} (bound {rel_bound:.0e})   max|err|/A {worst:.2e}")
+    assert torch.isfinite(got).all(), f"{name}: non-finite values"
+    assert rel < rel_bound, f"{name}: rel-L2 {rel:.3e} >= {rel_bound:.0e}"
+    assert bool((d <= elem * A.double()).all()), f"{name}: worst element |err|/A = {worst:.3e} > {elem:.3e}"
+    return rel
+
+
 def pack(lib, w: torch.Tensor, mode: int, n_rows=64, stride=1, offset=0) -> torch.Tensor:
     out = torch.empty(9 * n_rows * 64, device=w.device, dtype=torch.bfloat16)
     _KEEP.append(w)

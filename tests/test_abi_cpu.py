@@ -129,6 +129,19 @@ def test_invalid_arguments_fail_loudly(lib):
         L.check(lib.sres_pack_conv_weights(None, None, 0, 64, 64, 64, 1, 0, None), "pack")
     assert lib.sres_adam_step_flat(None, None, None, None, C.c_int64(8), C.c_int64(1), C.c_double(1e-3), C.c_double(0.9),
                                    C.c_double(0.999), C.c_double(1e-8), C.c_double(0.0), None) == 1
+    # weight-gradient jobs whose output-channel mapping is malformed are refused before the device is touched (the
+    # pointers are never dereferenced): oc_stride 0 would have 64 threads race on one element
+    for cout_total, stride, offset in ((64, 0, 0), (64, -1, 0), (256, 4, 4), (256, 4, -1), (0, 1, 0), (-64, 1, 0)):
+        job = L.WgradJob(16, 16, 16, 16, cout_total, stride, offset, 0, 1.0)
+        assert lib.sres_conv3x3_wgrad_batch(C.byref(job), 1, 2, 8, 8, C.c_void_p(16), C.c_size_t(1 << 30), None) == 1
+        assert b"oc_stride" in lib.sres_last_error(), (cout_total, stride, offset)
+    good = L.WgradJob(16, 16, 16, 16, 256, 4, 3, 0, 1.0)
+    bad = L.WgradJob(16, 16, 16, 16, 256, 4, 0, 0, 1.0)
+    bad.oc_stride = 0
+    jobs = (L.WgradJob * 2)(good, bad)                                          # the second job of a batch is checked too
+    assert lib.sres_conv3x3_wgrad_batch(jobs, 2, 2, 8, 8, C.c_void_p(16), C.c_size_t(1 << 30), None) == 1
+    assert lib.sres_conv3x3_wgrad(C.c_void_p(16), C.c_void_p(16), 2, 8, 8, C.c_void_p(16), None, 64, 0, 0, 0, C.c_void_p(16),
+                                  C.c_size_t(1 << 30), None) == 1
 
 
 def test_no_cpu_fallback():
