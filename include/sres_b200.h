@@ -203,7 +203,8 @@ SRES_API int sres_conv3x3_wgrad(const void* x_bf16, const void* dy_bf16, int B, 
 /* ------------------------------------------------------------------------------------------ */
 /* Narrow 3x3 convolutions at the ends of the network (CUDA cores, HBM-bound)                 */
 /* ------------------------------------------------------------------------------------------ */
-/* planar fp32 (B,Cs,H,W), Cs = 1..4  ->  64-feature PTL rows (fp32 and/or bf16).
+/* Cs = 1..16 image channels in all five entry points below (SRES_ERR_UNSUPPORTED beyond).
+ * planar fp32 (B,Cs,H,W)  ->  64-feature PTL rows (fp32 and/or bf16).
  *   transposed == 0: w (64,Cs,3,3) + bias: the head conv forward (sres/model/rcan/network.py:13,23)
  *   transposed == 1: w (Cs,64,3,3): input-gradient of the tail conv 64->Cs (network.py:16)
  *   unshuffle  > 1 : store with PixelUnshuffle(unshuffle) addressing (sub-grid-major PTL)          */
@@ -214,6 +215,7 @@ SRES_API int sres_conv3x3_small_in(const float* in_nchw, const float* w, const f
  * tensor-core kernel's halo window; w (Cs,64,3,3)                                                       */
 SRES_API int sres_conv3x3_small_out(const void* u_bf16, const float* w, const float* bias, int B, int Cs, int H, int W,
                                     float* out_nchw, void* stream);
+/* workspace of the two weight gradients below, for any Cs (channel chunks run in stream order and reuse it) */
 SRES_API size_t sres_small_wgrad_workspace_bytes(void);
 /* head conv weight/bias gradient; the output gradient is g1 (+ g2 when not NULL), fp32 PTL      */
 SRES_API int sres_small_in_wgrad(const float* g1_f32, const float* g2_f32, const float* in_nchw, int B, int Cs,
@@ -306,7 +308,7 @@ SRES_API int sres_adam_step_flat(float* p, const float* g, float* m, float* v, i
 #define SRES_ARCH_EDSR 1
 typedef struct sres_rcan_desc {
   int32_t B, H, W;         /* low-resolution tile batch                                         */
-  int32_t cin, cout;       /* image channels (nchannels_in / nchannels_out, manager.py:52)       */
+  int32_t cin, cout;       /* image channels, 1..16 each (nchannels_in / nchannels_out, manager.py:52) */
   int32_t nfeatures;       /* 64                                                                 */
   int32_t n_groups;        /* nlayers  (residual groups)                                         */
   int32_t n_blocks;        /* nblocks  (RCABs per group)                                         */

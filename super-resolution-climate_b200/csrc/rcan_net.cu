@@ -147,8 +147,9 @@ static int build_net(Net* n, const sres_rcan_desc* d, int training) {
   if (!d) return set_error(SRES_ERR_INVALID_ARG, "rcan: null description");
   if (d->B <= 0 || d->H <= 0 || d->W <= 0) return set_error(SRES_ERR_INVALID_ARG, "rcan: bad tile geometry");
   if (d->nfeatures != 64) return set_error(SRES_ERR_UNSUPPORTED, "rcan: kernels are specialised for nfeatures == 64");
-  if (d->cin < 1 || d->cin > 4 || d->cout < 1 || d->cout > 4)
-    return set_error(SRES_ERR_UNSUPPORTED, "rcan: 1..4 image channels supported");
+  // 16: the narrow CUDA-core head / tail kernels (small_conv.cu) and the n_out = 16 tensor-core tail conv
+  if (d->cin < 1 || d->cin > 16 || d->cout < 1 || d->cout > 16)
+    return set_error(SRES_ERR_UNSUPPORTED, "rcan: 1..16 image channels supported");
   if (d->n_groups < 1 || d->n_blocks < 1) return set_error(SRES_ERR_INVALID_ARG, "rcan: need >= 1 group and block");
   if (d->arch != SRES_ARCH_RCAN && d->arch != SRES_ARCH_EDSR) return set_error(SRES_ERR_INVALID_ARG, "rcan: unknown arch");
   const bool edsr = d->arch == SRES_ARCH_EDSR;

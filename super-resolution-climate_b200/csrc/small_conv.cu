@@ -1,17 +1,24 @@
 // The narrow 3x3 convolutions at the two ends of RCAN, on CUDA cores (they are HBM-bound: K or N
-// is only 9*C with C = 1..4 image channels, SURVEY.md section 2 op inventory).
+// is only 9*C with C = 1..16 image channels, SURVEY.md section 2 op inventory).
 //
 //   conv3x3_small_in   : planar fp32 NCHW (C_s channels) -> 64-feature PTL rows.
 //                        head conv forward (sres/model/rcan/network.py:13,23) and, with transposed +
 //                        flipped weights, the input-gradient of the tail conv (network.py:16).
 //   small_in_wgrad     : weight/bias gradient of the head conv (reduction over all positions).
 //   small_out_wgrad    : weight/bias gradient of the tail conv 64 -> C_s.
+//
+// The kernels are written for at most kChunkC = 4 channels.  More channels (up to kMaxSmallC = 16):
+//   * the weight gradients and the CUDA-core tail forward compute every output element from one image channel, so they
+//     run as ceil(C_s / 4) launches over channel chunks (Ctot = the image's channel count, c0 = the chunk's first);
+//   * the head forward and the tail input-gradient sum over the channels: conv3x3_small_in_wide_kernel (weights in
+//     shared memory, narrower column strips) takes 5..16 channels in one launch.
 #include "internal.h"
 #include "ptx.cuh"
 
 namespace sres {
 
-constexpr int kMaxSmallC = 4;
+constexpr int kChunkC = 4;
+constexpr int kMaxSmallC = 16;
 
 // ---------------------------------------------------------------------------------------------
 // planar (B,Cs,H,W) fp32  ->  PTL [rows][64]
@@ -32,19 +39,19 @@ __host__ __device__ inline int strip_cols(int W) {
   return (((W + n - 1) / n) + 3) & ~3;
 }
 
-// Stage the planar fp32 band rows [y0-1, y0+kBandRows] x columns [x_lo-1, x_lo+S] of image b (zero outside the image) as
-// s[c][r][i], i = column - (x_lo - 1), pitch SWp.  One warp per (channel, row): coalesced, no per-element division.
+// Stage the planar fp32 band rows [y0-1, y0+kBandRows] x columns [x_lo-1, x_lo+S] of channels c0 .. c0+nch-1 of image b
+// (Ctot channels an image; zero outside the image) as s[c - c0][r][i], i = column - (x_lo - 1), pitch SWp.  One warp per
+// (channel, row): coalesced, no per-element division.
 // Asynchronous copies (cp.async, zero-fill outside the image): the callers stage item i+1 into the other half of a double
 // buffer while they compute item i -- staged synchronously, the ~40 dependent global loads per thread and item took as
 // long as the item's arithmetic.
-template <int CS>
-__device__ __forceinline__ void stage_band_async(float* s, const float* __restrict__ in, int b, int H, int W, int y0,
-                                                 int x_lo, int SWp) {
+__device__ __forceinline__ void stage_band_async(float* s, const float* __restrict__ in, int nch, int Ctot, int c0, int b,
+                                                 int H, int W, int y0, int x_lo, int SWp) {
   const int lane = threadIdx.x & 31, wrp = threadIdx.x >> 5;
-  for (int cr = wrp; cr < CS * (kBandRows + 2); cr += 8) {
+  for (int cr = wrp; cr < nch * (kBandRows + 2); cr += 8) {
     const int c = cr / (kBandRows + 2), r = cr - c * (kBandRows + 2), yy = y0 - 1 + r;
     const bool yin = yy >= 0 && yy < H;
-    const float* src = in + (((size_t)b * CS + c) * H + (yin ? yy : 0)) * W;
+    const float* src = in + (((size_t)b * Ctot + c0 + c) * H + (yin ? yy : 0)) * W;
     float* dst = s + cr * SWp;
     for (int i = lane; i < SWp; i += 32) {
       const int xx = x_lo - 1 + i;
@@ -103,7 +110,7 @@ conv3x3_small_in_kernel(const float* __restrict__ in, const float* __restrict__ 
   const int n_items = B * bands * nstrips, buf_floats = CS * (kBandRows + 2) * SWp;
   if ((int)blockIdx.x < n_items) {
     const BandItem it = band_item(blockIdx.x, bands, nstrips, S);
-    stage_band_async<CS>(s_buf, in, it.b, H, W, it.y0, it.x_lo, SWp);
+    stage_band_async(s_buf, in, CS, CS, 0, it.b, H, W, it.y0, it.x_lo, SWp);
   }
   cp_async_commit();
   int parity = 0;
@@ -115,7 +122,7 @@ conv3x3_small_in_kernel(const float* __restrict__ in, const float* __restrict__ 
     __syncthreads();   // every warp is done with the previous item: its buffer is free for the prefetch
     if (item + (int)gridDim.x < n_items) {
       const BandItem nx = band_item(item + gridDim.x, bands, nstrips, S);
-      stage_band_async<CS>(s_buf + (parity ^ 1) * buf_floats, in, nx.b, H, W, nx.y0, nx.x_lo, SWp);
+      stage_band_async(s_buf + (parity ^ 1) * buf_floats, in, CS, CS, 0, nx.b, H, W, nx.y0, nx.x_lo, SWp);
     }
     cp_async_commit();
     cp_async_wait<1>();
@@ -206,14 +213,142 @@ conv3x3_small_in_kernel(const float* __restrict__ in, const float* __restrict__ 
 }
 
 // ---------------------------------------------------------------------------------------------
+// conv3x3_small_in for 5..16 channels (same math, same PTL row mappings, same padding rows).  The kernel above cannot
+// simply be instantiated with CS = 16: its 2*CS*9 weights a thread would be 288 registers, and its double-buffered
+// 256-column band 333 KB.  Here
+//   * the weights sit in shared memory as feature pairs, float2 sw[c*9 + t][32] (lane l holds features 2l, 2l+1): a
+//     warp reads one 256-byte row per tap and channel, shared by four positions;
+//   * the column strips are at most kWideStrip pixels: at 16 channels the two band buffers and the weights take 98.5 KB,
+//     so two blocks share an SM;
+//   * a warp walks groups of four consecutive positions of the whole band (W % 4 == 0), any unshuffle factor, or single
+//     positions otherwise; the channel loop is not unrolled (its body is 36 FFMA2 for 18 shared loads).
+// Accumulation is fp32, channel by channel and tap by tap, as above.
+// ---------------------------------------------------------------------------------------------
+constexpr int kWideStrip = 48;
+
+__host__ __device__ inline int strip_cols_wide(int W) {
+  const int n = (W + kWideStrip - 1) / kWideStrip;
+  return (((W + n - 1) / n) + 3) & ~3;
+}
+
+__host__ __device__ inline size_t small_in_wide_smem_bytes(int Cs, int W) {
+  return (2 * (size_t)Cs * (kBandRows + 2) * (strip_cols_wide(W) + 2) + (size_t)Cs * 9 * 64) * sizeof(float);
+}
+
+__global__ void __launch_bounds__(256, 2)
+conv3x3_small_in_wide_kernel(const float* __restrict__ in, const float* __restrict__ w, const float* __restrict__ bias,
+                             int B, int Cs, int H, int W, int transposed, int unshuffle, float* __restrict__ out_f32,
+                             uint16_t* __restrict__ out_bf16) {
+  extern __shared__ float s_buf[];  // 2 x [Cs][kBandRows+2][S+2], then the weights [Cs*9][64]
+  const int lane = threadIdx.x & 31, wrp = threadIdx.x >> 5;
+  const int n0 = lane * 2;
+  const int S = strip_cols_wide(W), nstrips = (W + S - 1) / S, SWp = S + 2;   // even pitch: 8-byte aligned pairs
+  const int buf_floats = Cs * (kBandRows + 2) * SWp;
+  float* const s_w = s_buf + 2 * buf_floats;
+  for (int i = threadIdx.x; i < Cs * 9 * 64; i += blockDim.x) {
+    const int n = i & 63, ct = i >> 6, c = ct / 9, t = ct - c * 9;
+    s_w[i] = transposed ? w[(c * 64 + n) * 9 + (8 - t)] : w[(n * Cs + c) * 9 + t];
+  }
+  const float2* const sw2 = reinterpret_cast<const float2*>(s_w) + lane;
+  const float2 br = (bias && !transposed) ? make_float2(bias[n0], bias[n0 + 1]) : make_float2(0.f, 0.f);
+  const int P = W + 1, RP = (H + 1) * P;
+  const int bands = (H + 1 + kBandRows - 1) / kBandRows;  // the zero row y == H belongs to the last band
+  const int f = unshuffle > 1 ? unshuffle : 1;
+  const int Pl = W / f + 1, Rl = H / f + 1;
+  auto row_of = [&](int b, int y, int subx) -> long long {
+    if (f == 1) return (long long)b * RP + (long long)y * P;
+    return ((long long)((y % f) * f + subx) * B + b) * Rl * Pl + (long long)(y / f) * Pl;
+  };
+  auto store = [&](int b, int y, int x, float a0, float a1) {
+    const long long oq = row_of(b, y, x % f) + x / f;
+    if (out_f32) *reinterpret_cast<float2*>(out_f32 + oq * 64 + n0) = make_float2(a0, a1);
+    if (out_bf16) *reinterpret_cast<uint32_t*>(out_bf16 + oq * 64 + n0) = pack_bf16x2(a0, a1);
+  };
+  const int n_items = B * bands * nstrips;
+  if ((int)blockIdx.x < n_items) {
+    const BandItem it = band_item(blockIdx.x, bands, nstrips, S);
+    stage_band_async(s_buf, in, Cs, Cs, 0, it.b, H, W, it.y0, it.x_lo, SWp);
+  }
+  cp_async_commit();
+  int parity = 0;
+  for (int item = blockIdx.x; item < n_items; item += gridDim.x, parity ^= 1) {
+    const BandItem it = band_item(item, bands, nstrips, S);
+    const int b = it.b, y0 = it.y0, x_lo = it.x_lo, x_hi = min(W, x_lo + S);
+    const bool last_strip = x_lo + S >= W;
+    const float* s_in = s_buf + parity * buf_floats;
+    __syncthreads();   // every warp is done with the previous item (and the weights are in place, first time round)
+    if (item + (int)gridDim.x < n_items) {
+      const BandItem nx = band_item(item + gridDim.x, bands, nstrips, S);
+      stage_band_async(s_buf + (parity ^ 1) * buf_floats, in, Cs, Cs, 0, nx.b, H, W, nx.y0, nx.x_lo, SWp);
+    }
+    cp_async_commit();
+    cp_async_wait<1>();
+    __syncthreads();
+    const int rows = min(kBandRows, H + 1 - y0);
+    const int img_rows = min(kBandRows, H - y0);   // rows above the zero row y == H
+    const int ncol = x_hi - x_lo + (last_strip ? 1 : 0);   // + the padding column x == W
+    if ((W & 3) == 0) {
+      const int ng = (x_hi - x_lo) >> 2;
+      for (int g = wrp; g < img_rows * ng; g += 8) {
+        const int yl = g / ng, xr = (g - yl * ng) * 4;
+        float2 a[4];
+#pragma unroll
+        for (int j = 0; j < 4; ++j) a[j] = br;
+#pragma unroll 1
+        for (int c = 0; c < Cs; ++c) {
+          const float* srow = s_in + (c * (kBandRows + 2) + yl) * SWp + xr;
+          const float2* wc = sw2 + c * 9 * 32;
+#pragma unroll
+          for (int ty = 0; ty < 3; ++ty) {
+            const float* dr = srow + ty * SWp;
+            const float2 d01 = *reinterpret_cast<const float2*>(dr);
+            const float2 d23 = *reinterpret_cast<const float2*>(dr + 2);
+            const float2 d45 = *reinterpret_cast<const float2*>(dr + 4);
+            const float d6[6] = {d01.x, d01.y, d23.x, d23.y, d45.x, d45.y};
+#pragma unroll
+            for (int tx = 0; tx < 3; ++tx) {
+              const float2 wv = wc[(ty * 3 + tx) * 32];
+#pragma unroll
+              for (int j = 0; j < 4; ++j) ffma2_bcast(a[j], wv, d6[j + tx]);
+            }
+          }
+        }
+#pragma unroll
+        for (int j = 0; j < 4; ++j) store(b, y0 + yl, x_lo + xr + j, a[j].x, a[j].y);
+      }
+      // zeros: the padding column of the image rows, then the zero row y == H if it is in this band
+      if (last_strip)
+        for (int yl = wrp; yl < img_rows; yl += 8) store(b, y0 + yl, W, 0.f, 0.f);
+      if (rows > img_rows)
+        for (int xr = wrp; xr < ncol; xr += 8) store(b, H, x_lo + xr, 0.f, 0.f);
+      continue;
+    }
+    for (int pos = wrp; pos < rows * ncol; pos += 8) {
+      const int yl = pos / ncol, xr = pos - yl * ncol, x = x_lo + xr, y = y0 + yl;
+      float2 a = make_float2(0.f, 0.f);
+      if (x != W && y != H) {
+        a = br;
+#pragma unroll 1
+        for (int c = 0; c < Cs; ++c)
+#pragma unroll
+          for (int t = 0; t < 9; ++t)
+            ffma2_bcast(a, sw2[(c * 9 + t) * 32], s_in[(c * (kBandRows + 2) + yl + t / 3) * SWp + xr + t % 3]);
+      }
+      store(b, y, x, a.x, a.y);
+    }
+  }
+}
+
+// ---------------------------------------------------------------------------------------------
 // head-conv weight gradient: dW[n][c][t] = sum_q (g1+g2)[q][n] * in[c][q+off(t)],  db[n] = sum_q g[q][n]
 // block = 64 features x 4 position lanes; per-block partials then a fixed-order reduce.
+// One launch covers Cs <= kChunkC channels c0 .. c0+Cs-1 of an image with Ctot channels.
 // ---------------------------------------------------------------------------------------------
-constexpr int kSwAcc = kMaxSmallC * 9 + 1;
+constexpr int kSwAcc = kChunkC * 9 + 1;
 
 __global__ void __launch_bounds__(256)
 small_in_wgrad_kernel(const float* __restrict__ g1, const float* __restrict__ g2, const float* __restrict__ in, int B,
-                      int Cs, int H, int W, float* __restrict__ part) {
+                      int Cs, int Ctot, int c0, int H, int W, float* __restrict__ part) {
   __shared__ float sm[4][64][kSwAcc];
   const int n = threadIdx.x & 63, ln = threadIdx.x >> 6;
   const int P = W + 1, RP = (H + 1) * P;
@@ -229,7 +364,7 @@ small_in_wgrad_kernel(const float* __restrict__ g1, const float* __restrict__ g2
     if (g2) gv += g2[q * 64 + n];
     acc[kSwAcc - 1] += gv;
     for (int c = 0; c < Cs; ++c) {
-      const float* ip = in + ((size_t)b * Cs + c) * H * W;
+      const float* ip = in + ((size_t)b * Ctot + c0 + c) * H * W;
 #pragma unroll
       for (int t = 0; t < 9; ++t) {
         const int yy = y + t / 3 - 1, xx = x + t % 3 - 1;
@@ -254,7 +389,7 @@ small_in_wgrad_kernel(const float* __restrict__ g1, const float* __restrict__ g2
 template <int CS>
 __global__ void __launch_bounds__(256)
 small_in_wgrad_band_kernel(const float* __restrict__ g1, const float* __restrict__ g2, const float* __restrict__ in, int B,
-                           int H, int W, float* __restrict__ part) {
+                           int Ctot, int c0, int H, int W, float* __restrict__ part) {
   extern __shared__ float s_x[];  // [CS][kBandRows+2][SW], then the cross-warp reduction buffer
   const int lane = threadIdx.x & 31, wrp = threadIdx.x >> 5;
   const int n0 = lane * 2;
@@ -271,7 +406,7 @@ small_in_wgrad_band_kernel(const float* __restrict__ g1, const float* __restrict
     __syncthreads();
     for (int i = threadIdx.x; i < CS * (kBandRows + 2) * SW; i += blockDim.x) {
       const int xx = i % SW - 1, yy = (i / SW) % (kBandRows + 2) + y0 - 1, c = i / (SW * (kBandRows + 2));
-      s_x[i] = (yy >= 0 && yy < H && xx >= 0 && xx < W) ? __ldg(in + (((size_t)b * CS + c) * H + yy) * W + xx) : 0.f;
+      s_x[i] = (yy >= 0 && yy < H && xx >= 0 && xx < W) ? __ldg(in + (((size_t)b * Ctot + c0 + c) * H + yy) * W + xx) : 0.f;
     }
     __syncthreads();
     const int rows = min(kBandRows, H - y0);
@@ -326,7 +461,7 @@ small_in_wgrad_band_kernel(const float* __restrict__ g1, const float* __restrict
   }
 }
 
-__global__ void small_in_wgrad_reduce_kernel(const float* __restrict__ part, int nparts, int Cs,
+__global__ void small_in_wgrad_reduce_kernel(const float* __restrict__ part, int nparts, int Cs, int Ctot, int c0,
                                              float* __restrict__ dw, float* __restrict__ db, int accumulate) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= 64 * kSwAcc) return;
@@ -336,7 +471,7 @@ __global__ void small_in_wgrad_reduce_kernel(const float* __restrict__ part, int
   if (e == kSwAcc - 1) {
     if (db) db[n] = accumulate ? db[n] + s : s;
   } else if (e < Cs * 9) {
-    float* o = dw + (size_t)n * Cs * 9 + e;
+    float* o = dw + (size_t)n * Ctot * 9 + c0 * 9 + e;
     *o = accumulate ? *o + s : s;
   }
 }
@@ -348,11 +483,12 @@ __global__ void small_in_wgrad_reduce_kernel(const float* __restrict__ part, int
 // A block owns bands of kBandRows image rows: the planar dout band (+halo, zero outside) is staged in
 // shared memory; a thread owns 2 input features k (one bf16x2 load per U row, a warp reads one full
 // 128-byte row) and 8 warps walk the band's rows.  Per-block partials, then a fixed-order reduce.
+// One launch covers CS <= kChunkC channels c0 .. c0+CS-1 of an output gradient with Ctot channels.
 // ---------------------------------------------------------------------------------------------
 template <int CS>
 __global__ void __launch_bounds__(256, 2)
-small_out_wgrad_kernel(const float* __restrict__ dout, const uint16_t* __restrict__ u, int B, int H, int W,
-                       float* __restrict__ part) {
+small_out_wgrad_kernel(const float* __restrict__ dout, const uint16_t* __restrict__ u, int B, int Ctot, int c0, int H,
+                       int W, float* __restrict__ part) {
   extern __shared__ float s_buf[];  // 2 x [CS][kBandRows+2][S+2] (column strips, see strip_cols), then the cross-warp reduction buffer
   const int lane = threadIdx.x & 31, wrp = threadIdx.x >> 5;
   const int k0 = lane * 2;
@@ -372,7 +508,7 @@ small_out_wgrad_kernel(const float* __restrict__ dout, const uint16_t* __restric
   const int n_items = B * bands * nstrips, buf_floats = CS * (kBandRows + 2) * SWp;
   if ((int)blockIdx.x < n_items) {
     const BandItem it = band_item(blockIdx.x, bands, nstrips, S);
-    stage_band_async<CS>(s_buf, dout, it.b, H, W, it.y0, it.x_lo, SWp);
+    stage_band_async(s_buf, dout, CS, Ctot, c0, it.b, H, W, it.y0, it.x_lo, SWp);
   }
   cp_async_commit();
   int parity = 0;
@@ -383,7 +519,7 @@ small_out_wgrad_kernel(const float* __restrict__ dout, const uint16_t* __restric
     __syncthreads();   // every warp is done with the previous item: its buffer is free for the prefetch
     if (item + (int)gridDim.x < n_items) {
       const BandItem nx = band_item(item + gridDim.x, bands, nstrips, S);
-      stage_band_async<CS>(s_buf + (parity ^ 1) * buf_floats, dout, nx.b, H, W, nx.y0, nx.x_lo, SWp);
+      stage_band_async(s_buf + (parity ^ 1) * buf_floats, dout, CS, Ctot, c0, nx.b, H, W, nx.y0, nx.x_lo, SWp);
     }
     cp_async_commit();
     cp_async_wait<1>();
@@ -474,7 +610,7 @@ small_out_wgrad_kernel(const float* __restrict__ dout, const uint16_t* __restric
   }
 }
 
-__global__ void small_out_wgrad_reduce_kernel(const float* __restrict__ part, int nparts, int Cs,
+__global__ void small_out_wgrad_reduce_kernel(const float* __restrict__ part, int nparts, int Cs, int c0,
                                               float* __restrict__ dw, float* __restrict__ db, int accumulate) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= 64 * kSwAcc) return;
@@ -482,9 +618,9 @@ __global__ void small_out_wgrad_reduce_kernel(const float* __restrict__ part, in
   for (int p = 0; p < nparts; ++p) s += part[(size_t)p * 64 * kSwAcc + i];
   const int k = i / kSwAcc, e = i % kSwAcc;
   if (e == kSwAcc - 1) {
-    if (db && k < Cs) db[k] = accumulate ? db[k] + s : s;
+    if (db && k < Cs) db[c0 + k] = accumulate ? db[c0 + k] + s : s;
   } else if (e < Cs * 9) {
-    const int c = e / 9, t = e % 9;
+    const int c = c0 + e / 9, t = e % 9;
     float* o = dw + ((size_t)c * 64 + k) * 9 + t;
     *o = accumulate ? *o + s : s;
   }
@@ -494,20 +630,21 @@ __global__ void small_out_wgrad_reduce_kernel(const float* __restrict__ part, in
 // tail conv forward on CUDA cores: 64-feature bf16 PTL -> planar fp32 (B,Cs,H,W).  Used when the image is too
 // wide for the tensor-core kernel's flat halo window (W > ~700: the x8 up-scaling of 96x96 tiles); the op is
 // HBM-bound either way (it reads 128 B per pixel and writes 4*Cs).  One warp per output pixel: lanes split
-// the 64 input features (2 each), 9 taps, shuffle reduction.
+// the 64 input features (2 each), 9 taps, shuffle reduction.  One launch writes CS <= kChunkC output planes
+// c0 .. c0+CS-1 of Ctot.
 // ---------------------------------------------------------------------------------------------
 template <int CS>
 __global__ void __launch_bounds__(256)
 small_out_fwd_kernel(const uint16_t* __restrict__ u, const float* __restrict__ w, const float* __restrict__ bias, int B,
-                     int H, int W, float* __restrict__ out) {
+                     int Ctot, int c0, int H, int W, float* __restrict__ out) {
   const int lane = threadIdx.x & 31;
   float wr[CS][9][2];
 #pragma unroll
   for (int c = 0; c < CS; ++c)
 #pragma unroll
     for (int t = 0; t < 9; ++t) {
-      wr[c][t][0] = w[(c * 64 + 2 * lane) * 9 + t];
-      wr[c][t][1] = w[(c * 64 + 2 * lane + 1) * 9 + t];
+      wr[c][t][0] = w[((c0 + c) * 64 + 2 * lane) * 9 + t];
+      wr[c][t][1] = w[((c0 + c) * 64 + 2 * lane + 1) * 9 + t];
     }
   const int P = W + 1;
   const long long RP = (long long)(H + 1) * P;
@@ -532,7 +669,7 @@ small_out_fwd_kernel(const uint16_t* __restrict__ u, const float* __restrict__ w
       float a = acc[c];
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
-      if (lane == 0) out[(((long long)b * CS + c) * H + y) * W + x] = a + (bias ? bias[c] : 0.f);
+      if (lane == 0) out[(((long long)b * Ctot + c0 + c) * H + y) * W + x] = a + (bias ? bias[c0 + c] : 0.f);
     }
   }
 }
@@ -551,17 +688,26 @@ extern "C" int sres_conv3x3_small_in(const float* in_nchw, const float* w, const
                                      int W, int transposed, int unshuffle, float* out_f32, void* out_bf16,
                                      void* stream) {
   if (!in_nchw || !w || (!out_f32 && !out_bf16)) return set_error(SRES_ERR_INVALID_ARG, "small_in: null pointer");
-  if (Cs < 1 || Cs > kMaxSmallC) return set_error(SRES_ERR_UNSUPPORTED, "small_in: 1..4 image channels supported");
+  if (Cs < 1 || Cs > kMaxSmallC) return set_error(SRES_ERR_UNSUPPORTED, "small_in: 1..16 image channels supported");
   if (B <= 0 || H <= 0 || W <= 0) return set_error(SRES_ERR_INVALID_ARG, "small_in: bad geometry");
   if (unshuffle > 1 && (H % unshuffle || W % unshuffle))
     return set_error(SRES_ERR_INVALID_ARG, "small_in: unshuffle factor must divide H and W");
   const int bands = (H + 1 + kBandRows - 1) / kBandRows;
-  const int S = strip_cols(W), nstrips = (W + S - 1) / S;
+  const bool wide = Cs > kChunkC;
+  const int S = wide ? strip_cols_wide(W) : strip_cols(W), nstrips = (W + S - 1) / S;
   long long items = (long long)B * bands * nstrips;
   const int blocks = (int)(items > small_grid() * 2 ? small_grid() * 2 : items);
-  const size_t smem = 2 * (size_t)Cs * (kBandRows + 2) * (S + 2) * sizeof(float);   // double buffer, <= 83 KB
   cudaStream_t st = (cudaStream_t)stream;
   uint16_t* o16 = (uint16_t*)out_bf16;
+  if (wide) {
+    const size_t smem = small_in_wide_smem_bytes(Cs, W);   // <= 98.5 KB at 16 channels
+    cudaFuncSetAttribute(conv3x3_small_in_wide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    conv3x3_small_in_wide_kernel<<<blocks, 256, smem, st>>>(in_nchw, w, bias, B, Cs, H, W, transposed, unshuffle, out_f32,
+                                                            o16);
+    SRES_CHECK_LAUNCH("small_in: launch");
+    return SRES_OK;
+  }
+  const size_t smem = 2 * (size_t)Cs * (kBandRows + 2) * (S + 2) * sizeof(float);   // double buffer, <= 83 KB
 #define SRES_LAUNCH_SMALL_IN(CS)                                                                                   \
   do {                                                                                                             \
     if (smem > 48 * 1024)                                                                                          \
@@ -579,90 +725,104 @@ extern "C" int sres_conv3x3_small_in(const float* in_nchw, const float* w, const
   return SRES_OK;
 }
 
+// The weight-gradient launches of the channel chunks run one after the other on the caller's stream and reuse the same
+// partials, so the workspace is the size of one chunk's, whatever the channel count.
 extern "C" size_t sres_small_wgrad_workspace_bytes(void) { return (size_t)small_grid() * 64 * kSwAcc * sizeof(float); }
 
 extern "C" int sres_small_in_wgrad(const float* g1_f32, const float* g2_f32, const float* in_nchw, int B, int Cs,
                                    int H, int W, float* dw, float* db, int accumulate, void* workspace,
                                    size_t workspace_bytes, void* stream) {
   if (!g1_f32 || !in_nchw || !dw || !workspace) return set_error(SRES_ERR_INVALID_ARG, "small_in_wgrad: null pointer");
-  if (Cs < 1 || Cs > kMaxSmallC) return set_error(SRES_ERR_UNSUPPORTED, "small_in_wgrad: 1..4 image channels supported");
+  if (Cs < 1 || Cs > kMaxSmallC) return set_error(SRES_ERR_UNSUPPORTED, "small_in_wgrad: 1..16 image channels supported");
   const int grid = small_grid();
   if (workspace_bytes < (size_t)grid * 64 * kSwAcc * sizeof(float))
     return set_error(SRES_ERR_INVALID_ARG, "small_in_wgrad: workspace too small");
-  size_t smem = (size_t)Cs * (kBandRows + 2) * ((W + 3) & ~1) * sizeof(float);
-  const size_t red = (size_t)8 * 64 * kSwAcc * sizeof(float);
-  if (smem < red) smem = red;
-  if ((W & 3) == 0 && smem <= 200 * 1024) {
-    cudaStream_t st = (cudaStream_t)stream;
-    float* partp = (float*)workspace;
+  cudaStream_t st = (cudaStream_t)stream;
+  float* partp = (float*)workspace;
+  // chunks of <= 4 channels; each recomputes the bias gradient, the first one writes it
+  for (int c0 = 0; c0 < Cs; c0 += kChunkC) {
+    const int cc = Cs - c0 < kChunkC ? Cs - c0 : kChunkC;
+    size_t smem = (size_t)cc * (kBandRows + 2) * ((W + 3) & ~1) * sizeof(float);
+    const size_t red = (size_t)8 * 64 * kSwAcc * sizeof(float);
+    if (smem < red) smem = red;
+    if ((W & 3) == 0 && smem <= 200 * 1024) {
 #define SRES_LAUNCH_HEAD_WG(CS)                                                                                       \
   do {                                                                                                                \
     cudaFuncSetAttribute(small_in_wgrad_band_kernel<CS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);      \
-    small_in_wgrad_band_kernel<CS><<<grid, 256, smem, st>>>(g1_f32, g2_f32, in_nchw, B, H, W, partp);                  \
+    small_in_wgrad_band_kernel<CS><<<grid, 256, smem, st>>>(g1_f32, g2_f32, in_nchw, B, Cs, c0, H, W, partp);          \
   } while (0)
-    switch (Cs) {
-      case 1: SRES_LAUNCH_HEAD_WG(1); break;
-      case 2: SRES_LAUNCH_HEAD_WG(2); break;
-      case 3: SRES_LAUNCH_HEAD_WG(3); break;
-      default: SRES_LAUNCH_HEAD_WG(4); break;
-    }
+      switch (cc) {
+        case 1: SRES_LAUNCH_HEAD_WG(1); break;
+        case 2: SRES_LAUNCH_HEAD_WG(2); break;
+        case 3: SRES_LAUNCH_HEAD_WG(3); break;
+        default: SRES_LAUNCH_HEAD_WG(4); break;
+      }
 #undef SRES_LAUNCH_HEAD_WG
-  } else {
-    small_in_wgrad_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(g1_f32, g2_f32, in_nchw, B, Cs, H, W, (float*)workspace);
+    } else {
+      small_in_wgrad_kernel<<<grid, 256, 0, st>>>(g1_f32, g2_f32, in_nchw, B, cc, Cs, c0, H, W, partp);
+    }
+    SRES_CHECK_LAUNCH("small_in_wgrad: launch");
+    small_in_wgrad_reduce_kernel<<<(64 * kSwAcc + 255) / 256, 256, 0, st>>>(partp, grid, cc, Cs, c0, dw,
+                                                                             c0 == 0 ? db : nullptr, accumulate);
+    SRES_CHECK_LAUNCH("small_in_wgrad: reduce launch");
   }
-  SRES_CHECK_LAUNCH("small_in_wgrad: launch");
-  small_in_wgrad_reduce_kernel<<<(64 * kSwAcc + 255) / 256, 256, 0, (cudaStream_t)stream>>>((const float*)workspace, grid,
-                                                                                            Cs, dw, db, accumulate);
-  SRES_CHECK_LAUNCH("small_in_wgrad: reduce launch");
   return SRES_OK;
 }
 
 extern "C" int sres_small_out_wgrad(const float* dout_nchw, const void* u_bf16, int B, int Cs, int H, int W, float* dw,
                                     float* db, int accumulate, void* workspace, size_t workspace_bytes, void* stream) {
   if (!dout_nchw || !u_bf16 || !dw || !workspace) return set_error(SRES_ERR_INVALID_ARG, "small_out_wgrad: null pointer");
-  if (Cs < 1 || Cs > kMaxSmallC) return set_error(SRES_ERR_UNSUPPORTED, "small_out_wgrad: 1..4 image channels supported");
+  if (Cs < 1 || Cs > kMaxSmallC) return set_error(SRES_ERR_UNSUPPORTED, "small_out_wgrad: 1..16 image channels supported");
   const int grid = small_grid();
   if (workspace_bytes < (size_t)grid * 64 * kSwAcc * sizeof(float))
     return set_error(SRES_ERR_INVALID_ARG, "small_out_wgrad: workspace too small");
-  size_t smem = 2 * (size_t)Cs * (kBandRows + 2) * (strip_cols(W) + 2) * sizeof(float);   // double buffer
-  const size_t red = (size_t)8 * 64 * kSwAcc * sizeof(float);
-  if (smem < red) smem = red;
   cudaStream_t st = (cudaStream_t)stream;
   const uint16_t* u16 = (const uint16_t*)u_bf16;
   float* partp = (float*)workspace;
+  // chunks of <= 4 channels: each one reads all of U again (the 64-feature operand), see DESIGN.md section 3.3.  Past 4
+  // channels a remainder of 3 runs as 2 + 1: the 3-channel instance keeps 27 accumulator pairs a thread and spills.
+  for (int c0 = 0, cc; c0 < Cs; c0 += cc) {
+    cc = Cs - c0 < kChunkC ? Cs - c0 : kChunkC;
+    if (Cs > kChunkC && cc == 3) cc = 2;
+    size_t smem = 2 * (size_t)cc * (kBandRows + 2) * (strip_cols(W) + 2) * sizeof(float);   // double buffer
+    const size_t red = (size_t)8 * 64 * kSwAcc * sizeof(float);
+    if (smem < red) smem = red;
 #define SRES_LAUNCH_SMALL_OUT(CS)                                                                               \
   do {                                                                                                          \
     cudaFuncSetAttribute(small_out_wgrad_kernel<CS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);   \
-    small_out_wgrad_kernel<CS><<<grid, 256, smem, st>>>(dout_nchw, u16, B, H, W, partp);                        \
+    small_out_wgrad_kernel<CS><<<grid, 256, smem, st>>>(dout_nchw, u16, B, Cs, c0, H, W, partp);                \
   } while (0)
-  switch (Cs) {
-    case 1: SRES_LAUNCH_SMALL_OUT(1); break;
-    case 2: SRES_LAUNCH_SMALL_OUT(2); break;
-    case 3: SRES_LAUNCH_SMALL_OUT(3); break;
-    default: SRES_LAUNCH_SMALL_OUT(4); break;
-  }
+    switch (cc) {
+      case 1: SRES_LAUNCH_SMALL_OUT(1); break;
+      case 2: SRES_LAUNCH_SMALL_OUT(2); break;
+      case 3: SRES_LAUNCH_SMALL_OUT(3); break;
+      default: SRES_LAUNCH_SMALL_OUT(4); break;
+    }
 #undef SRES_LAUNCH_SMALL_OUT
-  SRES_CHECK_LAUNCH("small_out_wgrad: launch");
-  small_out_wgrad_reduce_kernel<<<(64 * kSwAcc + 255) / 256, 256, 0, (cudaStream_t)stream>>>((const float*)workspace, grid,
-                                                                                             Cs, dw, db, accumulate);
-  SRES_CHECK_LAUNCH("small_out_wgrad: reduce launch");
+    SRES_CHECK_LAUNCH("small_out_wgrad: launch");
+    small_out_wgrad_reduce_kernel<<<(64 * kSwAcc + 255) / 256, 256, 0, st>>>(partp, grid, cc, c0, dw, db, accumulate);
+    SRES_CHECK_LAUNCH("small_out_wgrad: reduce launch");
+  }
   return SRES_OK;
 }
 
 extern "C" int sres_conv3x3_small_out(const void* u_bf16, const float* w, const float* bias, int B, int Cs, int H, int W,
                                       float* out_nchw, void* stream) {
   if (!u_bf16 || !w || !out_nchw) return set_error(SRES_ERR_INVALID_ARG, "small_out: null pointer");
-  if (Cs < 1 || Cs > kMaxSmallC) return set_error(SRES_ERR_UNSUPPORTED, "small_out: 1..4 image channels supported");
+  if (Cs < 1 || Cs > kMaxSmallC) return set_error(SRES_ERR_UNSUPPORTED, "small_out: 1..16 image channels supported");
   if (B <= 0 || H <= 0 || W <= 0) return set_error(SRES_ERR_INVALID_ARG, "small_out: bad geometry");
   const int grid = small_grid() * 4;
   cudaStream_t st = (cudaStream_t)stream;
   const uint16_t* u16 = (const uint16_t*)u_bf16;
-  switch (Cs) {
-    case 1: small_out_fwd_kernel<1><<<grid, 256, 0, st>>>(u16, w, bias, B, H, W, out_nchw); break;
-    case 2: small_out_fwd_kernel<2><<<grid, 256, 0, st>>>(u16, w, bias, B, H, W, out_nchw); break;
-    case 3: small_out_fwd_kernel<3><<<grid, 256, 0, st>>>(u16, w, bias, B, H, W, out_nchw); break;
-    default: small_out_fwd_kernel<4><<<grid, 256, 0, st>>>(u16, w, bias, B, H, W, out_nchw); break;
+  for (int c0 = 0; c0 < Cs; c0 += kChunkC) {   // output planes in chunks of <= 4
+    const int cc = Cs - c0 < kChunkC ? Cs - c0 : kChunkC;
+    switch (cc) {
+      case 1: small_out_fwd_kernel<1><<<grid, 256, 0, st>>>(u16, w, bias, B, Cs, c0, H, W, out_nchw); break;
+      case 2: small_out_fwd_kernel<2><<<grid, 256, 0, st>>>(u16, w, bias, B, Cs, c0, H, W, out_nchw); break;
+      case 3: small_out_fwd_kernel<3><<<grid, 256, 0, st>>>(u16, w, bias, B, Cs, c0, H, W, out_nchw); break;
+      default: small_out_fwd_kernel<4><<<grid, 256, 0, st>>>(u16, w, bias, B, Cs, c0, H, W, out_nchw); break;
+    }
+    SRES_CHECK_LAUNCH("small_out: launch");
   }
-  SRES_CHECK_LAUNCH("small_out: launch");
   return SRES_OK;
 }
