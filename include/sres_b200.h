@@ -129,40 +129,6 @@ SRES_API size_t sres_conv_pair_flag_bytes(int B, int H, int W);
 SRES_API int sres_conv_pair_supported(const sres_conv_args* first, const sres_conv_args* second);
 SRES_API int sres_conv3x3_pair(const sres_conv_args* first, const sres_conv_args* second, void* flags, void* stream);
 
-/* A residual group's RCAB chain (forward) in ONE launch: n_blocks x [conv 3x3 + bias + ReLU -> conv 3x3 + bias ->
- * CALayer gate -> x += t2 * s, bf16 copy], replacing per block the fused pair launch + sres_ca_apply_fwd
- * (sres/model/rcan/network.py:50-64 RCAB, :31-47 CALayer, looped by ResidualGroup :66-77).  A cluster of two CTAs owns one
- * image for the whole chain (image-aligned M tiles; cluster barriers instead of grid-wide launch boundaries), so the grid
- * may have any size.  Buffers are arrays of bf16 PTL tensors of (B,H,W) geometry, `B*(H+1)*(W+1)*64` elements apart:
- *   block r reads XB[xi(r)] and writes XB[xi(r+1)], xi(r) = xb_ring ? (xb_first + r) % xb_ring : xb_first + r;
- *   its conv outputs go to T1[ti(r)], T2[ti(r)], ti(r) = t_fixed ? t_first : t_first + r  (training keeps every block's
- *   tensors for backward: xb_ring = 0, t_fixed = 0; inference ping-pongs: xb_ring = 2, t_fixed = 1).
- * wpack_bf16: forward-packed weights of conv1(0), conv2(0), conv1(1), ... (2 * n_blocks operands of 9*64*64 bf16);
- * params: fp32 parameters of block 0 in state_dict order (conv1 w, b, conv2 w, b, conv_du.0 w, b, conv_du.2 w, b), block r
- * at params + r * rcab_stride; x_in_f32: the group input (fp32 PTL); x_f32: running fp32 trunk (fp32 PTL, every block
- * writes it); save_mean / save_s: [B][64] per block, save_stride floats apart (0 = keep the last block's only);
- * scratch: sres_rcab_chain_scratch_bytes(B) bytes.                                                                    */
-typedef struct sres_rcab_chain_args {
-  void* xb_bf16;
-  void* t1_bf16;
-  void* t2_bf16;
-  const void* wpack_bf16;
-  const float* params;
-  const float* x_in_f32;
-  float* x_f32;
-  float* save_mean;
-  float* save_s;
-  void* scratch;
-  int64_t rcab_stride, save_stride;
-  int32_t B, H, W, n_blocks, hidden;
-  int32_t xb_first, xb_ring, xb_count;
-  int32_t t_first, t_fixed, t_count;
-  void* debug_timeline;    /* bring-up only: int64 [grid][16] per-CTA clock stamps, or NULL */
-} sres_rcab_chain_args;
-SRES_API int sres_rcab_chain_supported(int B, int H, int W);
-SRES_API size_t sres_rcab_chain_scratch_bytes(int B);
-SRES_API int sres_rcab_chain_fwd(const sres_rcab_chain_args* args, void* stream);
-
 /* Repack fp32 OIHW 3x3 weights (the checkpoint layout, state_dict of nn.Conv2d) to the bf16
  * tap-major operand the tensor-core kernels read.
  *   mode 0 (forward):   out[t][n][k] = w[oc(n)][k][ky][kx],              t = ky*3+kx
@@ -239,15 +205,6 @@ SRES_API int sres_ca_apply_fwd(const void* t2_bf16, const float* pool_part, cons
                                const float* b1, const float* w2, const float* b2, int hidden, const float* x_in,
                                float* x_out, void* xb_out_bf16, float* save_mean, float* save_s, int B, int H, int W,
                                void* stream);
-/* the same with the trunk value carried as a bf16 pair x = hi + lo (hi = bf16(x) is the copy the next convolution
- * reads, lo = bf16(x - hi)): 98 instead of 118 MB per call at B = 64.  Input: either x_in_f32 (a residual group's
- * first block, network.py:74-77) or xhi_in_bf16 + xlo_in_bf16; output xhi_out_bf16 (must not alias xhi_in) and
- * xlo_out_bf16 (may alias xlo_in).                                                                              */
-SRES_API int sres_ca_apply_fwd_split(const void* t2_bf16, const float* pool_part, const float* pool_sum, const float* w1,
-                                     const float* b1, const float* w2, const float* b2, int hidden, const float* x_in_f32,
-                                     const void* xhi_in_bf16, const void* xlo_in_bf16, void* xhi_out_bf16,
-                                     void* xlo_out_bf16, float* save_mean, float* save_s, int B, int H, int W,
-                                     void* stream);
 /* backward of the above w.r.t. t2: dt2 (bf16 PTL) from the fp32 trunk gradient; saves ds [B][64];
  * ds_part: scratch [B][sres_ca_blocks_per_image][64] floats                                       */
 SRES_API int sres_ca_bwd(const float* grad_f32, const void* t2_bf16, const float* w1, const float* b1,

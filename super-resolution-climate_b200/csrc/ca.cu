@@ -121,21 +121,11 @@ ca_pool_kernel(CaGeom g, const uint16_t* __restrict__ t2, float* __restrict__ po
 // x_out = x_in + t2 * s ;  xb_out = bf16(x_out) ; block 0 of each image stores mean and s.
 // Low register count on purpose: all blocks of the grid must be co-resident (one wave), otherwise every
 // wave pays the latency-bound pooled-mean + MLP prologue again.
-
-//
-// kSplit: the running trunk value travels as a bf16 pair, x = hi + lo, where hi = bf16(x) IS the bf16 copy the next
-// convolution reads (and backward keeps) and lo = bf16(x - hi) carries the next 8 mantissa bits (|x - hi - lo| <= 2^-18 |x|):
-// 19.7 (t2) + 2 x 19.7 read + 2 x 19.7 written = 98 MB instead of 118 MB at B = 64.  x_in (fp32) non-null = a group's
-// first block: the group input is still a plain fp32 tensor (written by the head / group-tail convolution); otherwise
-// hi/lo come in as xhi_in / xlo_in (xlo_in may alias xlo_out: every row is read and written by the same thread).
-// Opt-in (SRES_TRUNK_SPLIT=1, rcan_net.cu): measured no faster than the fp32 form on B200 -- see there.
-template <bool kSplit>
 __global__ void __launch_bounds__(kCaThreads)
 ca_apply_fwd_kernel(CaGeom g, const uint16_t* __restrict__ t2, const float* __restrict__ pool_part,
                     const float* __restrict__ pool_sum, const float* __restrict__ w1, const float* __restrict__ b1,
                     const float* __restrict__ w2, const float* __restrict__ b2, const float* x_in, float* x_out,
-                    uint16_t* __restrict__ xb_out, float* __restrict__ save_mean, float* __restrict__ save_s,
-                    const uint16_t* __restrict__ xhi_in, const uint16_t* xlo_in, uint16_t* xlo_out) {
+                    uint16_t* __restrict__ xb_out, float* __restrict__ save_mean, float* __restrict__ save_s) {
   __shared__ float sm_red[4][64];
   __shared__ float sm_m[64], sm_h[kCaMaxHidden], sm_s[64];
   CaWeights sw;
@@ -174,41 +164,6 @@ ca_apply_fwd_kernel(CaGeom g, const uint16_t* __restrict__ t2, const float* __re
     }
   }
   __syncthreads();
-  if constexpr (kSplit) {
-    // All-bf16 streams: a thread owns the 8 contiguous channels [8cg, 8cg+8) so that every access is one 16-byte vector
-    // and a warp instruction covers four whole contiguous rows (512 B) (8-byte accesses: 19.9 instead of 18.1 us).
-    float s8[8];
-#pragma unroll
-    for (int j = 0; j < 8; ++j) s8[j] = sm_s[cg * 8 + j];
-#pragma unroll 2
-    for (int r = r0; r < r1; r += kCaThreads / 8) {
-      const size_t q = (size_t)b * g.RP + r;
-      const uint4 tv = *reinterpret_cast<const uint4*>(t2 + q * 64 + cg * 8);
-      float x[8];
-      if (x_in) {
-        const float4 xa = *reinterpret_cast<const float4*>(x_in + q * 64 + cg * 8);
-        const float4 xb = *reinterpret_cast<const float4*>(x_in + q * 64 + cg * 8 + 4);
-        x[0] = xa.x; x[1] = xa.y; x[2] = xa.z; x[3] = xa.w; x[4] = xb.x; x[5] = xb.y; x[6] = xb.z; x[7] = xb.w;
-      } else {
-        const uint4 hv = *reinterpret_cast<const uint4*>(xhi_in + q * 64 + cg * 8);
-        const uint4 lv = *reinterpret_cast<const uint4*>(xlo_in + q * 64 + cg * 8);
-        x[0] = bf16_lo(hv.x) + bf16_lo(lv.x); x[1] = bf16_hi(hv.x) + bf16_hi(lv.x);
-        x[2] = bf16_lo(hv.y) + bf16_lo(lv.y); x[3] = bf16_hi(hv.y) + bf16_hi(lv.y);
-        x[4] = bf16_lo(hv.z) + bf16_lo(lv.z); x[5] = bf16_hi(hv.z) + bf16_hi(lv.z);
-        x[6] = bf16_lo(hv.w) + bf16_lo(lv.w); x[7] = bf16_hi(hv.w) + bf16_hi(lv.w);
-      }
-      float o[8];
-      o[0] = fmaf(bf16_lo(tv.x), s8[0], x[0]); o[1] = fmaf(bf16_hi(tv.x), s8[1], x[1]);
-      o[2] = fmaf(bf16_lo(tv.y), s8[2], x[2]); o[3] = fmaf(bf16_hi(tv.y), s8[3], x[3]);
-      o[4] = fmaf(bf16_lo(tv.z), s8[4], x[4]); o[5] = fmaf(bf16_hi(tv.z), s8[5], x[5]);
-      o[6] = fmaf(bf16_lo(tv.w), s8[6], x[6]); o[7] = fmaf(bf16_hi(tv.w), s8[7], x[7]);
-      const uint4 h = make_uint4(pack_bf16x2(o[0], o[1]), pack_bf16x2(o[2], o[3]), pack_bf16x2(o[4], o[5]), pack_bf16x2(o[6], o[7]));
-      *reinterpret_cast<uint4*>(xb_out + q * 64 + cg * 8) = h;
-      *reinterpret_cast<uint4*>(xlo_out + q * 64 + cg * 8) =
-          make_uint4(pack_bf16x2(o[0] - bf16_lo(h.x), o[1] - bf16_hi(h.x)), pack_bf16x2(o[2] - bf16_lo(h.y), o[3] - bf16_hi(h.y)),
-                     pack_bf16x2(o[4] - bf16_lo(h.z), o[5] - bf16_hi(h.z)), pack_bf16x2(o[6] - bf16_lo(h.w), o[7] - bf16_hi(h.w)));
-    }
-  } else {
   // A thread owns channels [4cg, 4cg+4) and [32+4cg, 32+4cg+4): every load/store instruction of a warp then
   // covers whole contiguous 128-byte (fp32) / 64-byte (bf16) row halves -- fully coalesced per instruction.
   float s8[8];
@@ -232,7 +187,6 @@ ca_apply_fwd_kernel(CaGeom g, const uint16_t* __restrict__ t2, const float* __re
       *reinterpret_cast<uint2*>(xb_out + q * 64 + cg * 4) = make_uint2(pack_bf16x2(o[0], o[1]), pack_bf16x2(o[2], o[3]));
       *reinterpret_cast<uint2*>(xb_out + q * 64 + 32 + cg * 4) = make_uint2(pack_bf16x2(o[4], o[5]), pack_bf16x2(o[6], o[7]));
     }
-  }
   }
 }
 
@@ -496,32 +450,9 @@ extern "C" int sres_ca_apply_fwd(const void* t2_bf16, const float* pool_part, co
   if (!t2_bf16 || (!pool_part && !pool_sum) || !w1 || !b1 || !w2 || !b2 || !x_in || !x_out || !save_mean || !save_s)
     return set_error(SRES_ERR_INVALID_ARG, "ca_apply_fwd: null pointer");
   dim3 grid(g.blocks_per_image, B);
-  cudaError_t e = launch_pdl_if(pdl_level() >= 2, ca_apply_fwd_kernel<false>, grid, dim3(kCaThreads), ca_weights_bytes(hidden), (cudaStream_t)stream, g, (const uint16_t*)t2_bf16,
-                             pool_part, pool_sum, w1, b1, w2, b2, x_in, x_out, (uint16_t*)xb_out_bf16, save_mean, save_s,
-                             (const uint16_t*)nullptr, (const uint16_t*)nullptr, (uint16_t*)nullptr);
+  cudaError_t e = launch_pdl_if(pdl_level() >= 2, ca_apply_fwd_kernel, grid, dim3(kCaThreads), ca_weights_bytes(hidden), (cudaStream_t)stream, g, (const uint16_t*)t2_bf16,
+                             pool_part, pool_sum, w1, b1, w2, b2, x_in, x_out, (uint16_t*)xb_out_bf16, save_mean, save_s);
   if (e != cudaSuccess) return set_cuda_error(e, "ca_apply_fwd: launch");
-  return SRES_OK;
-}
-
-extern "C" int sres_ca_apply_fwd_split(const void* t2_bf16, const float* pool_part, const float* pool_sum, const float* w1,
-                                       const float* b1, const float* w2, const float* b2, int hidden, const float* x_in_f32,
-                                       const void* xhi_in_bf16, const void* xlo_in_bf16, void* xhi_out_bf16,
-                                       void* xlo_out_bf16, float* save_mean, float* save_s, int B, int H, int W,
-                                       void* stream) {
-  CaGeom g;
-  int rc = ca_geom(&g, B, H, W, hidden);
-  if (rc) return rc;
-  if (!pool_sum && g.RP < 128) return set_error(SRES_ERR_UNSUPPORTED, "ca_apply_fwd_split: fused pool partials need (H+1)*(W+1) >= 128; pass pool_sum");
-  if (!t2_bf16 || (!pool_part && !pool_sum) || !w1 || !b1 || !w2 || !b2 || !xhi_out_bf16 || !xlo_out_bf16 || !save_mean || !save_s)
-    return set_error(SRES_ERR_INVALID_ARG, "ca_apply_fwd_split: null pointer");
-  if ((x_in_f32 != nullptr) == (xhi_in_bf16 != nullptr || xlo_in_bf16 != nullptr) || (!x_in_f32 && (!xhi_in_bf16 || !xlo_in_bf16)))
-    return set_error(SRES_ERR_INVALID_ARG, "ca_apply_fwd_split: pass either x_in_f32 or both xhi_in_bf16 and xlo_in_bf16");
-  if (xhi_in_bf16 == xhi_out_bf16) return set_error(SRES_ERR_INVALID_ARG, "ca_apply_fwd_split: xhi_out must not alias xhi_in");
-  dim3 grid(g.blocks_per_image, B);
-  cudaError_t e = launch_pdl_if(pdl_level() >= 2, ca_apply_fwd_kernel<true>, grid, dim3(kCaThreads), ca_weights_bytes(hidden), (cudaStream_t)stream, g, (const uint16_t*)t2_bf16,
-                             pool_part, pool_sum, w1, b1, w2, b2, x_in_f32, (float*)nullptr, (uint16_t*)xhi_out_bf16, save_mean, save_s,
-                             (const uint16_t*)xhi_in_bf16, (const uint16_t*)xlo_in_bf16, (uint16_t*)xlo_out_bf16);
-  if (e != cudaSuccess) return set_cuda_error(e, "ca_apply_fwd_split: launch");
   return SRES_OK;
 }
 

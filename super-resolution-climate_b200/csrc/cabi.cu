@@ -140,7 +140,7 @@ static std::atomic<long long> g_launches{0};
 void count_launch() { g_launches.fetch_add(1, std::memory_order_relaxed); }
 }  // namespace sres
 extern "C" long long sres_launch_count(void) { return sres::g_launches.load(std::memory_order_relaxed); }
-extern "C" int sres_abi_version(void) { return 3; }  // 3: device-side element count of the losses, sres_conv_tile_rows
+extern "C" int sres_abi_version(void) { return 4; }  // 4: image-resident RCAB chain and split-trunk channel-attention entry points removed
 extern "C" const char* sres_last_error(void) { return sres::t_err; }
 extern "C" int sres_device_sm_count(void) { return sres::device_sm_count(); }
 extern "C" int64_t sres_ptl_rows(int B, int H, int W) { return (int64_t)B * (H + 1) * (W + 1); }

@@ -22,9 +22,6 @@
 
 namespace sres {
 
-#ifndef SRES_RCAB_CHAIN_DEFAULT
-#define SRES_RCAB_CHAIN_DEFAULT 0
-#endif
 constexpr int kConvW = 64 * 64 * 9;  // floats of one 64->64 conv weight
 // bf16 gradient buffers rotate through a ring: a deferred weight-gradient job keeps reading its buffer until its
 // batch (8 jobs = 4 blocks by default, on the side stream) has been launched, so the ring holds one batch of blocks
@@ -41,23 +38,6 @@ static int ring_len() {   // buffers actually rotated through (<= kRing): fewer 
 }
 // SRES_JOIN_PER_SEG=1: the round-1 behaviour (join the side stream after every backward segment, squeeze-excite parameter
 // gradients on the main stream) for A/B runs.
-// SRES_TRUNK_SPLIT=1 (opt-in): inside a residual group the forward trunk value travels as a bf16 pair (hi = the bf16 copy
-// the next convolution reads anyway, lo = bf16(x - hi)) instead of an fp32 tensor next to that copy: the channel-attention
-// apply kernel moves 98 instead of 118 MB per RCAB (ca.cu).  Measured on B200 (round 2, tools/r2_split.sh): the kernel
-// alone is NOT faster (18.1 vs 17.1 us L2-warm, 24.4 vs 25.9 us cold: the extra unpack / subtract / convert instructions
-// cost what the bytes save) and the training step is slower (28.07 vs 27.47 ms): the fp32 trunk sits in the persisting
-// part of L2, the pair's hi half is an ordinary saved activation that competes with T1 / T2 for the rest.  Default off.
-static bool trunk_split() {
-  static const bool v = [] { const char* e = getenv("SRES_TRUNK_SPLIT"); return e && atoi(e) != 0; }();
-  return v;
-}
-// SRES_RCAB_CHAIN: 1 = a residual group's RCAB chain runs as ONE image-resident cluster launch (rcab_chain.cu) when the
-// geometry fits; 0 = per RCAB the fused pair launch + channel-attention kernel.  Read at every forward call (not cached)
-// so that a test can run both paths in one process.
-static bool rcab_chain_enabled() {
-  const char* e = getenv("SRES_RCAB_CHAIN");
-  return e ? atoi(e) != 0 : SRES_RCAB_CHAIN_DEFAULT != 0;
-}
 static bool join_per_segment() {
   static const bool v = [] { const char* e = getenv("SRES_JOIN_PER_SEG"); return e && atoi(e) != 0; }();
   return v;
@@ -382,8 +362,7 @@ static int forward(const Net& n, const float* P, const float* x, float* out, uin
   float* pool_sum = (float*)(ws + n.o_pool_sum);
   int xbi = 0;  // index of the bf16 copy of the current trunk value
   const bool l2hint = l2_hint_enabled();
-  const bool split = trunk_split() && !n.edsr;
-  if (l2hint) RC(sres_l2_persist_window(xf, (size_t)n.lvRows[0] * (split ? 128 : 256), st));
+  if (l2hint) RC(sres_l2_persist_window(xf, (size_t)n.lvRows[0] * 256, st));
   { PROF("head conv"); RC(sres_conv3x3_small_in(x, P + n.head_w, P + n.head_b, B, d.cin, H, W, 0, 0, hf, XB(0), st)); }
   const float* gin = hf;
   if (n.edsr) {
@@ -396,28 +375,9 @@ static int forward(const Net& n, const float* P, const float* x, float* out, uin
       ++xbi;
     }
   }
-  const bool chain = !n.edsr && rcab_chain_enabled() && fused_pool && sres_rcab_chain_supported(B, H, W);
   for (int g = 0; g < (n.edsr ? 0 : G); ++g) {
     float* gout = (float*)(ws + n.o_gf[g & 1]);
-    if (chain) {
-      PROF("rcab chain fwd (R blocks)");
-      sres_rcab_chain_args ca;
-      memset(&ca, 0, sizeof(ca));
-      ca.xb_bf16 = ws + n.o_xb; ca.t1_bf16 = ws + n.o_t1; ca.t2_bf16 = ws + n.o_t2;
-      ca.wpack_bf16 = WF(n.cidx(g, 0, 0));
-      ca.params = P + n.off_rcab(g, 0);
-      ca.x_in_f32 = gin; ca.x_f32 = xf;
-      ca.save_mean = (float*)(ws + n.o_mean) + (size_t)(training ? g * R : 0) * B * 64;
-      ca.save_s = (float*)(ws + n.o_s) + (size_t)(training ? g * R : 0) * B * 64;
-      ca.scratch = pool_part;   // per-tile partial sums are not used on this path: the buffer serves as the [B][2][64] scratch
-      ca.rcab_stride = n.rcab_sz; ca.save_stride = training ? (long long)B * 64 : 0;
-      ca.B = B; ca.H = H; ca.W = W; ca.n_blocks = R; ca.hidden = n.hid;
-      ca.xb_first = xbi; ca.xb_ring = training ? 0 : 2; ca.xb_count = n.n_xb;
-      ca.t_first = training ? g * R : 0; ca.t_fixed = training ? 0 : 1; ca.t_count = n.n_t;
-      RC(sres_rcab_chain_fwd(&ca, st));
-      xbi += R;
-    }
-    for (int r = 0; r < (chain ? 0 : R); ++r) {
+    for (int r = 0; r < R; ++r) {
       const int ti = g * R + r;
       const float* pr = P + n.off_rcab(g, r);
       const float* c1b = pr + kConvW;
@@ -434,11 +394,6 @@ static int forward(const Net& n, const float* P, const float* x, float* out, uin
       float* mean = (float*)(ws + n.o_mean) + (size_t)(training ? ti : 0) * B * 64;
       float* sv = (float*)(ws + n.o_s) + (size_t)(training ? ti : 0) * B * 64;
       { PROF("ca_apply_fwd");
-      if (split)   // xf's storage holds the bf16 low halves (first lvRows * 128 bytes)
-        RC(sres_ca_apply_fwd_split(T2(ti), fused_pool ? pool_part : nullptr, fused_pool ? nullptr : pool_sum, w1, b1, w2, b2,
-                                   n.hid, r == 0 ? gin : nullptr, r == 0 ? nullptr : XB(xbi), r == 0 ? nullptr : (const void*)xf,
-                                   XB(xbi + 1), xf, mean, sv, B, H, W, st));
-      else
         RC(sres_ca_apply_fwd(T2(ti), fused_pool ? pool_part : nullptr, fused_pool ? nullptr : pool_sum, w1, b1, w2, b2,
                              n.hid, r == 0 ? gin : xf, xf, XB(xbi + 1), mean, sv, B, H, W, st)); }
       ++xbi;

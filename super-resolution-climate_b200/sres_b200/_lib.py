@@ -42,20 +42,6 @@ class ConvArgs(C.Structure):
     ]
 
 
-class ChainArgs(C.Structure):
-    """sres_rcab_chain_args (include/sres_b200.h)."""
-    _fields_ = [
-        ("xb_bf16", C.c_void_p), ("t1_bf16", C.c_void_p), ("t2_bf16", C.c_void_p),
-        ("wpack_bf16", C.c_void_p), ("params", C.c_void_p), ("x_in_f32", C.c_void_p), ("x_f32", C.c_void_p),
-        ("save_mean", C.c_void_p), ("save_s", C.c_void_p), ("scratch", C.c_void_p),
-        ("rcab_stride", C.c_int64), ("save_stride", C.c_int64),
-        ("B", C.c_int32), ("H", C.c_int32), ("W", C.c_int32), ("n_blocks", C.c_int32), ("hidden", C.c_int32),
-        ("xb_first", C.c_int32), ("xb_ring", C.c_int32), ("xb_count", C.c_int32),
-        ("t_first", C.c_int32), ("t_fixed", C.c_int32), ("t_count", C.c_int32),
-        ("debug_timeline", C.c_void_p),
-    ]
-
-
 class WgradJob(C.Structure):
     """sres_wgrad_job (include/sres_b200.h)."""
     _fields_ = [
@@ -81,7 +67,6 @@ def lib():
         L.sres_last_error.restype = C.c_char_p
         L.sres_ptl_rows.restype = C.c_int64
         L.sres_launch_count.restype = C.c_longlong
-        L.sres_rcab_chain_scratch_bytes.restype = C.c_size_t
         _lib = L
     return _lib
 

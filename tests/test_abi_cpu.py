@@ -29,7 +29,7 @@ def test_library_exports_every_declared_symbol(lib):
     assert len(names) >= 30
     for n in names:
         assert hasattr(lib, n), f"{n} declared in include/sres_b200.h but not exported"
-    assert lib.sres_abi_version() == 3
+    assert lib.sres_abi_version() == 4
 
 
 def test_header_cites_reference_lines():

@@ -480,172 +480,6 @@ def test_channel_attention_forward_backward(env, B, H, W, red):
     assert rel_l2(gflat.cpu(), ref_flat) < 1e-4
 
 
-@pytest.mark.parametrize("B,H,W,red", [(3, 20, 24, 2), (2, 48, 48, 16)])
-def test_channel_attention_split_trunk_equals_fp32_trunk(env, B, H, W, red):
-    """sres_ca_apply_fwd_split (trunk as a bf16 pair hi + lo) against sres_ca_apply_fwd (fp32 trunk), two chained RCAB
-    residual updates (network.py:61-64): hi is bit-for-bit the fp32 kernel's bf16 copy of the same input, hi + lo is the
-    fp32 value to 2^-17, and both stay zero on the padding rows."""
-    L, lib, dev = env
-    hid = 64 // red
-    w1, b1 = (torch.randn(hid, 64) * 0.3).to(dev), torch.randn(hid).to(dev)
-    w2, b2 = (torch.randn(64, hid) * 0.3).to(dev), torch.randn(64).to(dev)
-    x0 = to_ptl((torch.randn(B, 64, H, W) * 3).to(dev), torch.float32)
-    rows = x0.shape[0]
-    mean, sv = torch.empty(B, 64, device=dev), torch.empty(B, 64, device=dev)
-    mean2, sv2 = torch.empty(B, 64, device=dev), torch.empty(B, 64, device=dev)
-    pool_sum = torch.empty(B, 64, device=dev)
-    st = L.cur_stream()
-    x_f32 = x0                      # fp32 trunk fed to the fp32 kernel
-    hi = lo = None
-    for step in range(2):
-        t2p = to_ptl(bf16_round(torch.randn(B, 64, H, W)).to(dev), torch.bfloat16)
-        L.check(lib.sres_ca_pool(ptr(t2p), ptr(pool_sum), B, H, W, st), "ca_pool")
-        xin = x_f32 if step == 0 else (hi.float() + lo.float())    # the value the pair represents (before lo is overwritten)
-        hi_out = torch.full((rows, 64), 7.0, device=dev, dtype=torch.bfloat16)
-        lo_out = lo if lo is not None else torch.full((rows, 64), 7.0, device=dev, dtype=torch.bfloat16)   # in place from step 1 on
-        L.check(lib.sres_ca_apply_fwd_split(ptr(t2p), None, ptr(pool_sum), ptr(w1), ptr(b1), ptr(w2), ptr(b2), hid,
-                                            ptr(x0) if step == 0 else None, None if step == 0 else ptr(hi), None if step == 0 else ptr(lo),
-                                            ptr(hi_out), ptr(lo_out), ptr(mean), ptr(sv), B, H, W, st), "ca_apply_fwd_split")
-        # the fp32 kernel on the same value
-        xo = torch.full((rows, 64), float("nan"), device=dev)
-        xb = torch.zeros(rows, 64, device=dev, dtype=torch.bfloat16)
-        L.check(lib.sres_ca_apply_fwd(ptr(t2p), None, ptr(pool_sum), ptr(w1), ptr(b1), ptr(w2), ptr(b2), hid, ptr(xin), ptr(xo), ptr(xb),
-                                      ptr(mean2), ptr(sv2), B, H, W, st), "ca_apply_fwd")
-        torch.cuda.synchronize()
-        assert torch.equal(hi_out.view(torch.int16), xb.view(torch.int16))
-        assert torch.equal(mean, mean2) and torch.equal(sv, sv2)
-        pair = hi_out.float() + lo_out.float()
-        err = (pair - xo).abs()
-        assert bool((err <= xo.abs() * 2.0 ** -17 + 1e-30).all()), float((err / (xo.abs() + 1e-30)).max())
-        assert pads_are_zero(hi_out, B, H, W) and pads_are_zero(lo_out, B, H, W)
-        hi, lo = hi_out, lo_out
-    # argument errors are reported, not guessed around
-    assert lib.sres_ca_apply_fwd_split(ptr(t2p), None, ptr(pool_sum), ptr(w1), ptr(b1), ptr(w2), ptr(b2), hid, ptr(x0), ptr(hi), ptr(lo),
-                                       ptr(hi_out), ptr(lo_out), ptr(mean), ptr(sv), B, H, W, st) != 0
-    assert lib.sres_ca_apply_fwd_split(ptr(t2p), None, ptr(pool_sum), ptr(w1), ptr(b1), ptr(w2), ptr(b2), hid, None, ptr(hi), None,
-                                       ptr(hi_out), ptr(lo_out), ptr(mean), ptr(sv), B, H, W, st) != 0
-
-
-@pytest.mark.parametrize("B,H,W,nb,red,training", [(3, 20, 24, 3, 4, True), (2, 48, 48, 2, 16, True), (5, 12, 12, 2, 16, False),
-                                                   (2, 48, 48, 3, 16, False), (1, 9, 9, 2, 2, True)])
-def test_rcab_chain_equals_kernel_by_kernel(env, B, H, W, nb, red, training):
-    """sres_rcab_chain_fwd (a residual group's RCABs in one image-resident cluster launch, network.py:50-77) against the same
-    blocks run kernel by kernel (two convolution launches, sres_ca_pool, sres_ca_apply_fwd): the first block's T1 / T2 are
-    bit-identical (same MMA order per output row); the pooled mean is summed in another order, so from the gate on the two
-    paths agree to fp32 round-off (plus a rare bf16 rounding flip downstream)."""
-    L, lib, dev = env
-    if not lib.sres_rcab_chain_supported(B, H, W):
-        pytest.skip("geometry not served by the chain kernel")
-    hid = 64 // red
-    RP = (H + 1) * (W + 1)
-    rows = B * RP
-    KW = 64 * 64 * 9
-    stride = 2 * (KW + 64) + hid * 64 + hid + 64 * hid + 64
-    g = torch.Generator().manual_seed(B * 1000 + H * 10 + nb)
-    params = torch.empty(nb, stride)
-    for r in range(nb):
-        params[r] = torch.cat([(torch.randn(KW, generator=g) * 0.04), torch.randn(64, generator=g) * 0.1,
-                               (torch.randn(KW, generator=g) * 0.04), torch.randn(64, generator=g) * 0.1,
-                               torch.randn(hid * 64, generator=g) * 0.3, torch.randn(hid, generator=g),
-                               torch.randn(64 * hid, generator=g) * 0.3, torch.randn(64, generator=g)])
-    params = params.to(dev).contiguous()
-    wpack = torch.empty(nb * 2, KW, device=dev, dtype=torch.bfloat16)
-    for r in range(nb):
-        for c in range(2):
-            w = params[r, c * (KW + 64): c * (KW + 64) + KW].reshape(64, 64, 3, 3).contiguous()
-            wpack[2 * r + c] = pack(lib, w, 0)
-    x0 = to_ptl(torch.randn(B, 64, H, W, generator=g).to(dev), torch.float32)
-    st = L.cur_stream()
-    n_xb, n_t = (nb + 2, nb) if training else (2, 1)
-    xb_first = 1 if training else 0
-
-    def fresh():
-        xb = torch.full((n_xb, rows, 64), 7.0, device=dev, dtype=torch.bfloat16)
-        xb[xb_first] = x0.bfloat16()
-        return (xb, torch.full((n_t, rows, 64), 7.0, device=dev, dtype=torch.bfloat16), torch.full((n_t, rows, 64), 7.0, device=dev, dtype=torch.bfloat16),
-                torch.full((rows, 64), float("nan"), device=dev), torch.zeros(nb if training else 1, B, 64, device=dev), torch.zeros(nb if training else 1, B, 64, device=dev))
-
-    # ---- kernel by kernel ----
-    xb_r, t1_r, t2_r, xf_r, mean_r, s_r = fresh()
-    pool_sum = torch.empty(B, 64, device=dev)
-    fused_pool = RP >= 128
-    pool_part = torch.zeros(lib.sres_conv_mtiles(B, H, W), 2, 4, 64, device=dev)
-    tol = 3e-4 * nb if fused_pool else 5e-3    # a 1-ulp difference of a gate flips a few bf16 roundings per block, and those spread
-    for r in range(nb):
-        xi, xo = ((xb_first + r) % 2, (xb_first + r + 1) % 2) if not training else (xb_first + r, xb_first + r + 1)
-        ti, si = (r, r) if training else (0, 0)
-        pr = params[r]
-        o = 0
-        c1b = pr[KW:KW + 64]; c2b = pr[2 * KW + 64: 2 * KW + 128]
-        o = 2 * (KW + 64)
-        w1 = pr[o:o + hid * 64]; b1 = pr[o + hid * 64: o + hid * 64 + hid]
-        o2 = o + hid * 64 + hid
-        w2 = pr[o2:o2 + 64 * hid]; b2 = pr[o2 + 64 * hid: o2 + 64 * hid + 64]
-        run_conv(lib, conv_args(in_bf16=xb_r[xi], wpack_bf16=wpack[2 * r], bias=c1b, out_bf16=t1_r[ti], B=B, H=H, W=W, n_out=64, epi_flags=L.EPI_RELU))
-        if fused_pool:   # the production path: channel sums of the fp32 accumulators in the conv2 epilogue, like the chain kernel
-            run_conv(lib, conv_args(in_bf16=t1_r[ti], wpack_bf16=wpack[2 * r + 1], bias=c2b, out_bf16=t2_r[ti], pool_part=pool_part, B=B, H=H, W=W,
-                                    n_out=64, epi_flags=L.EPI_POOL))
-        else:            # small images: sres_ca_pool sums the bf16-ROUNDED T2 (means differ by the mean rounding error, ~1e-3 relative)
-            run_conv(lib, conv_args(in_bf16=t1_r[ti], wpack_bf16=wpack[2 * r + 1], bias=c2b, out_bf16=t2_r[ti], B=B, H=H, W=W, n_out=64, epi_flags=0))
-            L.check(lib.sres_ca_pool(ptr(t2_r[ti]), ptr(pool_sum), B, H, W, st), "ca_pool")
-        L.check(lib.sres_ca_apply_fwd(ptr(t2_r[ti]), ptr(pool_part) if fused_pool else None, None if fused_pool else ptr(pool_sum), ptr(w1), ptr(b1), ptr(w2), ptr(b2), hid,
-                                      ptr(x0 if r == 0 else xf_r), ptr(xf_r), ptr(xb_r[xo]), ptr(mean_r[si]), ptr(s_r[si]), B, H, W, st), "ca_apply_fwd")
-    torch.cuda.synchronize()
-
-    # ---- one chain launch ----
-    xb_c, t1_c, t2_c, xf_c, mean_c, s_c = fresh()
-    scratch = torch.zeros(lib.sres_rcab_chain_scratch_bytes(B) // 4, device=dev)
-    a = L.ChainArgs()
-    a.xb_bf16, a.t1_bf16, a.t2_bf16 = xb_c.data_ptr(), t1_c.data_ptr(), t2_c.data_ptr()
-    a.wpack_bf16, a.params, a.x_in_f32, a.x_f32 = wpack.data_ptr(), params.data_ptr(), x0.data_ptr(), xf_c.data_ptr()
-    a.save_mean, a.save_s, a.scratch = mean_c.data_ptr(), s_c.data_ptr(), scratch.data_ptr()
-    a.rcab_stride, a.save_stride = stride, (B * 64 if training else 0)
-    a.B, a.H, a.W, a.n_blocks, a.hidden = B, H, W, nb, hid
-    a.xb_first, a.xb_ring, a.xb_count = xb_first, (0 if training else 2), n_xb
-    a.t_first, a.t_fixed, a.t_count = 0, (0 if training else 1), n_t
-    L.check(lib.sres_rcab_chain_fwd(C.byref(a), st), "sres_rcab_chain_fwd")
-    torch.cuda.synchronize()
-
-    if training:
-        assert torch.equal(t1_c[0].view(torch.int16), t1_r[0].view(torch.int16))
-        assert torch.equal(t2_c[0].view(torch.int16), t2_r[0].view(torch.int16))
-        for r in range(nb):
-            assert rel_l2(t1_c[r].float(), t1_r[r].float()) < tol and rel_l2(t2_c[r].float(), t2_r[r].float()) < tol, r
-            assert rel_l2(xb_c[xb_first + r + 1].float(), xb_r[xb_first + r + 1].float()) < tol, r
-            assert pads_are_zero(t1_c[r], B, H, W) and pads_are_zero(t2_c[r], B, H, W) and pads_are_zero(xb_c[xb_first + r + 1], B, H, W)
-        assert torch.equal(xb_c[0], xb_r[0]) and torch.equal(xb_c[xb_first], xb_r[xb_first])     # untouched buffers stay untouched
-    else:
-        last = (xb_first + nb) % 2
-        assert rel_l2(xb_c[last].float(), xb_r[last].float()) < tol and pads_are_zero(xb_c[last], B, H, W)
-    assert rel_l2(mean_c, mean_r) < tol and rel_l2(s_c, s_r) < tol
-    assert rel_l2(xf_c, xf_r) < tol and pads_are_zero(xf_c, B, H, W)
-    # run to run: bit-identical (fixed summation orders, no atomics)
-    xb_d, t1_d, t2_d, xf_d, mean_d, s_d = fresh()
-    a.xb_bf16, a.t1_bf16, a.t2_bf16, a.x_f32, a.save_mean, a.save_s = xb_d.data_ptr(), t1_d.data_ptr(), t2_d.data_ptr(), xf_d.data_ptr(), mean_d.data_ptr(), s_d.data_ptr()
-    L.check(lib.sres_rcab_chain_fwd(C.byref(a), st), "sres_rcab_chain_fwd")
-    torch.cuda.synchronize()
-    assert torch.equal(xf_d, xf_c) and torch.equal(s_d, s_c) and torch.equal(t2_d.view(torch.int16), t2_c.view(torch.int16))
-
-
-@pytest.mark.parametrize("setting", ["SRES_CHAIN_OVERLAP=1", "SRES_CHAIN_LEND=1", "SRES_CHAIN_BULK=1", "SRES_CHAIN_K=1", "SRES_CHAIN_LEND=1 SRES_CHAIN_BULK=1"])
-def test_rcab_chain_variants_keep_parity(setting):
-    """The chain kernel's measured variants (streaming under the next conv1 with six extra warps, 4-deep halo ring through the
-    idle weight region, bulk-copy streaming phase, one CTA per image) are selected by environment switches that the library
-    reads once per process: the same kernel-by-kernel parity test runs in a fresh interpreter for each of them."""
-    import os
-    import subprocess
-    import sys
-    env_ = dict(os.environ)
-    for kv in setting.split():
-        key, val = kv.split("=")
-        env_[key] = val
-    here = os.path.dirname(os.path.abspath(__file__))
-    r = subprocess.run([sys.executable, "-m", "pytest", os.path.join(here, "test_gpu_kernels.py"), "-q", "-x", "-m", "gpu", "-k",
-                        "test_rcab_chain_equals_kernel_by_kernel", "-p", "no:cacheprovider"], env=env_, capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-2000:]
-    assert "5 passed" in r.stdout, r.stdout[-1000:]
-
-
 def test_bicubic_matches_interpolate(env):
     L, lib, dev = env
     from sres_b200 import nn as snn

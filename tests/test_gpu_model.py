@@ -120,46 +120,6 @@ def test_train_step_matches_oracle_and_golden(name, dev, golden_dir):
     assert rel_l2(prd2.cpu(), prd_o) < TOL
 
 
-@pytest.mark.parametrize("B,S,nlayers,nblocks", [(3, 48, 2, 3), (2, 20, 1, 2), (64, 48, 1, 20)])
-def test_rcab_chain_path_equals_tile_parallel_path(dev, monkeypatch, B, S, nlayers, nblocks):
-    """The image-resident residual-group launch (SRES_RCAB_CHAIN=1, rcab_chain.cu) against the tile-parallel path (fused pair +
-    channel-attention kernel per RCAB) on the same weights and inputs: training-mode output, every gradient and the
-    inference-mode output agree to fp32 round-off (the pooled means are summed in another order)."""
-    from sres_b200 import nn as snn
-    cfg = O.model_cfg(nlayers=nlayers, nblocks=nblocks, cbottleneck=16)
-    sd = O.make_state_dict(cfg, 2, 2)
-    hr = synth_hr(B, 2, S * 4)
-    res = {}
-    for mode in ("0", "1"):
-        monkeypatch.setenv("SRES_RCAB_CHAIN", mode)
-        model = _build(cfg, 2, dev)
-        model.load_state_dict(sd)
-        hr_d = hr.to(dev)
-        lr_d = snn.bicubic_resize(hr_d, 0.25)
-        model.train()
-        prd = model(lr_d.clone().requires_grad_(True))
-        loss = snn.loss(prd, hr_d, "l2")
-        loss.backward()
-        grads = {k: p.grad.detach().clone() for k, p in model.named_parameters()}
-        model.eval()
-        with torch.no_grad():
-            inf = model(lr_d.clone())
-            inf2 = model(lr_d.clone())            # second call replays the captured graph
-        torch.cuda.synchronize()
-        assert torch.equal(inf, inf2)
-        res[mode] = (prd.detach().clone(), grads, inf.clone(), model.engine.launches_forward(S, S))
-    assert res["1"][3] < res["0"][3] - 2 * nlayers * (nblocks - 1)          # the chain really ran: one launch per group
-    tol = 2e-4 if nblocks * nlayers < 10 else 3e-3      # rare bf16 rounding flips of the saved activations add up with depth
-    d_train, d_inf = rel_l2(res["1"][0], res["0"][0]), rel_l2(res["1"][2], res["0"][2])
-    print(f"chain vs tile-parallel: train output {d_train:.2e}, inference output {d_inf:.2e}")
-    assert d_train < tol and d_inf < tol
-    num = sum((res["1"][1][k] - res["0"][1][k]).double().pow(2).sum().item() for k in res["0"][1])
-    den = sum(res["0"][1][k].double().pow(2).sum().item() for k in res["0"][1])
-    assert (num / den) ** 0.5 < 5 * tol
-    for k in res["0"][1]:
-        assert rel_l2(res["1"][1][k], res["0"][1][k]) < 2e-2, k
-
-
 @pytest.mark.parametrize("nblocks", [1, 20])
 def test_x8_wide_tiles_forward_and_backward_run(dev, nblocks):
     """BASELINE config 5 geometry (x8, 4 channels, 96x96 LR -> 768x768 HR) at batch 1, with one RCAB and with one FULL

@@ -20,10 +20,6 @@ dsp = torch.empty(B * bpi * 64, device=dev)
 st = L.cur_stream()
 def fwd(i): return lib.sres_ca_apply_fwd(L.ptr(t2[i]), L.ptr(pool), None, L.ptr(w1), L.ptr(b1), L.ptr(w2), L.ptr(b2), hid, L.ptr(x[i]), L.ptr(x[i]), L.ptr(xb[i]), L.ptr(mean), L.ptr(sv), B, H, W, st)
 def bwd(i): return lib.sres_ca_bwd(L.ptr(x[i]), L.ptr(t2[i]), L.ptr(w1), L.ptr(b1), L.ptr(w2), L.ptr(b2), hid, L.ptr(mean), L.ptr(dsp), L.ptr(xb[i]), L.ptr(ds), B, H, W, st)
-lo = [torch.zeros(rows, 64, device=dev, dtype=torch.bfloat16) for _ in range(NB)]
-xb2 = [torch.empty(rows, 64, device=dev, dtype=torch.bfloat16) for _ in range(NB)]
-def fwd_split(i): return lib.sres_ca_apply_fwd_split(L.ptr(t2[i]), L.ptr(pool), None, L.ptr(w1), L.ptr(b1), L.ptr(w2), L.ptr(b2), hid, None, L.ptr(xb[i]), L.ptr(lo[i]), L.ptr(xb2[i]), L.ptr(lo[i]), L.ptr(mean), L.ptr(sv), B, H, W, st)
-def fwd_split_first(i): return lib.sres_ca_apply_fwd_split(L.ptr(t2[i]), L.ptr(pool), None, L.ptr(w1), L.ptr(b1), L.ptr(w2), L.ptr(b2), hid, L.ptr(x[i]), None, None, L.ptr(xb2[i]), L.ptr(lo[i]), L.ptr(mean), L.ptr(sv), B, H, W, st)
 lib.sres_ca_bwd_apply.restype = C.c_int
 def bwd_apply(i): return lib.sres_ca_bwd_apply(L.ptr(x[i]), L.ptr(pool), L.ptr(w1), L.ptr(b1), L.ptr(w2), L.ptr(b2), hid, L.ptr(mean), L.ptr(xb[i]), L.ptr(ds), B, H, W, st)
 def timeit(fn, rot, n=48):
@@ -34,7 +30,5 @@ def timeit(fn, rot, n=48):
     b.record(); torch.cuda.synchronize()
     return a.elapsed_time(b) / n * 1e3
 print(f"bpi={bpi}  ca_apply_fwd: cold {timeit(fwd, True):.1f} us, hot {timeit(fwd, False):.1f} us   (118 MB at B=64); B={B}, {118e6*B/64/timeit(fwd, False)/1e6:.2f} TB/s hot")
-print(f"bpi={bpi}  ca_apply_fwd_split (hi/lo in, hi/lo out): cold {timeit(fwd_split, True):.1f} us, hot {timeit(fwd_split, False):.1f} us   (98 MB at B=64)")
-print(f"bpi={bpi}  ca_apply_fwd_split (fp32 in, hi/lo out: a group's first block): cold {timeit(fwd_split_first, True):.1f} us, hot {timeit(fwd_split_first, False):.1f} us   (98 MB at B=64)")
 print(f"bpi={bpi}  ca_bwd (2 kernels): cold {timeit(bwd, True):.1f} us, hot {timeit(bwd, False):.1f} us   (2 x 59 MB)")
 print(f"bpi={bpi}  ca_bwd_apply (fused-dot path, in-network kernel): cold {timeit(bwd_apply, True):.1f} us, hot {timeit(bwd_apply, False):.1f} us   (59 MB at B=64)")
