@@ -230,6 +230,25 @@ SRES_API int sres_bicubic_resize(const float* in, float* out, int planes, int Hi
                                  double scale_h, double scale_w, void* stream);
 
 /* ------------------------------------------------------------------------------------------ */
+/* Resize in any mode the reference's task.downsample_mode / upsample_mode can name            */
+/*   sres/base/util/array.py:37-41 (torch_interp_mode: linear -> bilinear, cubic -> bicubic,    */
+/*   every other name passed through), :72-76 (downsample) and :84-87 (upsample):              */
+/*   F.interpolate(t, scale_factor=..., mode=...) on 4-D fp32 NCHW, align_corners=False, no     */
+/*   antialias.  planes = N*C; (Ho,Wo) = floor((Hi,Wi) * scale_factor) as F.interpolate sizes   */
+/*   it; scale_h / scale_w = 1 / scale_factor (positive, finite; SRES_RESIZE_AREA ignores them:  */
+/*   adaptive_avg_pool2d to (Ho,Wo), output o averages input [floor(o*in/out), ceil((o+1)*in/out))). */
+/*   SRES_RESIZE_BICUBIC runs the sres_bicubic_resize kernel.  Null pointers, sizes <= 0, an    */
+/*   unknown mode or a bad scale return SRES_ERR_INVALID_ARG before anything is enqueued.       */
+/* ------------------------------------------------------------------------------------------ */
+#define SRES_RESIZE_NEAREST 0        /* "nearest":       src = min(floor(dst*scale), in-1) (1:1 copy, 2x shift) */
+#define SRES_RESIZE_NEAREST_EXACT 1  /* "nearest-exact": src = min(floor((dst+0.5)*scale), in-1)              */
+#define SRES_RESIZE_BILINEAR 2       /* "bilinear" ("linear"): src = max(scale*(dst+0.5)-0.5, 0), two taps    */
+#define SRES_RESIZE_BICUBIC 3        /* "bicubic" ("cubic"): the kernel above                                 */
+#define SRES_RESIZE_AREA 4           /* "area": block mean (adaptive average pool)                            */
+SRES_API int sres_resize(const float* in, float* out, int planes, int Hi, int Wi, int Ho, int Wo, double scale_h,
+                         double scale_w, int mode, void* stream);
+
+/* ------------------------------------------------------------------------------------------ */
 /* Losses: kind 0 = l2 / RMSE (sres/controller/stats.py:5-8), 1 = charbonnier                  */
 /* (sres/controller/dual_trainer.py:196-198), 2 = l1 (BASELINE north_star variant).            */
 /* The target plane (tH,tW) may exceed the product's (H,W): conform_to_product,                */

@@ -62,6 +62,100 @@ __global__ void bicubic_resize_kernel(const float* __restrict__ in, float* __res
 }
 
 // ---------------------------------------------------------------------------------------------
+// Nearest, nearest-exact, bilinear and area resize: F.interpolate(mode=..., align_corners=False,
+// antialias=False) on 4-D input, the other settings of task.downsample_mode / upsample_mode
+// (sres/base/util/array.py:37-41 passes them to F.interpolate unchanged).  Index arithmetic as in
+// ATen (UpSample.h, AdaptiveAveragePooling), so nearest / nearest-exact pick the same source
+// pixels as torch's CPU and CUDA kernels and area sums in the same order.
+// ---------------------------------------------------------------------------------------------
+// upsample_nearest2d on the CPU: a plain copy for equal sizes and a shift for exactly 2x, else
+// floor(dst * scale) with the float scale 1/scale_factor.
+__device__ __forceinline__ int nearest_src(int dst, int in, int out, float scale) {
+  if (out == in) return dst;
+  if (out == 2 * in) return dst >> 1;
+  return min(int(floorf(__fmul_rn((float)dst, scale))), in - 1);
+}
+__device__ __forceinline__ int nearest_exact_src(int dst, int in, float scale) {
+  return min(int(floorf(__fmul_rn(__fadd_rn((float)dst, 0.5f), scale))), in - 1);
+}
+// linear source index (area_pixel_compute_source_index, clamped at 0 unlike cubic) and lambdas
+// (guard_index_and_lambda).  ATen's float build contracts scale * (dst + 0.5) - 0.5 into one FMA.
+__device__ __forceinline__ void linear_src(int dst, int in, int out, float scale, int& i0, int& i1, float& l0, float& l1) {
+  if (out == in) {
+    i0 = i1 = dst;
+    l0 = 1.f;
+    l1 = 0.f;
+    return;
+  }
+  const float r = fmaxf(__fmaf_rn(scale, __fadd_rn((float)dst, 0.5f), -0.5f), 0.f);
+  i0 = min(int(floorf(r)), in - 1);
+  l1 = fminf(fmaxf(r - (float)i0, 0.f), 1.f);
+  l0 = 1.f - l1;
+  i1 = i0 + (i0 < in - 1 ? 1 : 0);
+}
+
+__device__ __forceinline__ float add_in_order(float s, float q) { return s + q; }
+__device__ __forceinline__ float add_in_order(float s, float4 q) { return (((s + q.x) + q.y) + q.z) + q.w; }
+// Sum of rows [y0, y1) x columns [x0, x0 + kw) in fp32, row by row and left to right (ATen's order), read as pieces of
+// sizeof(V) bytes (kw a multiple of the piece) four at a time, so that four loads are in flight before the adds.
+template <typename V>
+__device__ __forceinline__ float window_sum(const float* ip, int Wi, int y0, int y1, int x0, int kw) {
+  constexpr int P = sizeof(V) / sizeof(float);
+  const int per_row = kw / P, n = (y1 - y0) * per_row;
+  float sum = 0.f;
+  for (int p = 0; p < n; p += 4) {
+    V q[4];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      if (p + k < n) {
+        const int r = (p + k) / per_row, c = p + k - r * per_row;
+        q[k] = __ldg(reinterpret_cast<const V*>(ip + (size_t)(y0 + r) * Wi + x0) + c);
+      }
+    }
+#pragma unroll
+    for (int k = 0; k < 4; ++k)
+      if (p + k < n) sum = add_in_order(sum, q[k]);
+  }
+  return sum;
+}
+
+template <int MODE>
+__global__ void __launch_bounds__(256)
+resize_kernel(const float* __restrict__ in, float* __restrict__ out, int planes, int Hi, int Wi, int Ho, int Wo,
+              float scale_h, float scale_w, int rows16) {
+  const long long total = (long long)planes * Ho * Wo;
+  for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total;
+       idx += (long long)gridDim.x * blockDim.x) {
+    const int ox = int(idx % Wo), oy = int((idx / Wo) % Ho);
+    const int pl = int(idx / ((long long)Wo * Ho));
+    const float* ip = in + (size_t)pl * Hi * Wi;
+    float v;
+    if (MODE == SRES_RESIZE_NEAREST) {
+      v = __ldg(ip + (size_t)nearest_src(oy, Hi, Ho, scale_h) * Wi + nearest_src(ox, Wi, Wo, scale_w));
+    } else if (MODE == SRES_RESIZE_NEAREST_EXACT) {
+      v = __ldg(ip + (size_t)nearest_exact_src(oy, Hi, scale_h) * Wi + nearest_exact_src(ox, Wi, scale_w));
+    } else if (MODE == SRES_RESIZE_BILINEAR) {
+      int y0, y1, x0, x1;
+      float a0, a1, b0, b1;
+      linear_src(oy, Hi, Ho, scale_h, y0, y1, a0, a1);
+      linear_src(ox, Wi, Wo, scale_w, x0, x1, b0, b1);
+      const float* r0 = ip + (size_t)y0 * Wi;
+      const float* r1 = ip + (size_t)y1 * Wi;
+      v = a0 * (b0 * __ldg(r0 + x0) + b1 * __ldg(r0 + x1)) + a1 * (b0 * __ldg(r1 + x0) + b1 * __ldg(r1 + x1));
+    } else {  // SRES_RESIZE_AREA: adaptive_avg_pool2d, rows [floor(o*in/out), ceil((o+1)*in/out))
+      const int y0 = (int)(((long long)oy * Hi) / Ho), y1 = (int)(((long long)(oy + 1) * Hi + Ho - 1) / Ho);
+      const int x0 = (int)(((long long)ox * Wi) / Wo), x1 = (int)(((long long)(ox + 1) * Wi + Wo - 1) / Wo);
+      const int kw = x1 - x0;
+      const float sum = (rows16 && ((x0 | kw) & 3) == 0)   // whole 16-byte row pieces (a x4 / x8 block mean)
+                            ? window_sum<float4>(ip, Wi, y0, y1, x0, kw)
+                            : window_sum<float>(ip, Wi, y0, y1, x0, kw);
+      v = sum / (float)(y1 - y0) / (float)kw;
+    }
+    out[idx] = v;
+  }
+}
+
+// ---------------------------------------------------------------------------------------------
 // Losses.  kind 0 = l2 (RMSE, sres/controller/stats.py:5-8), 1 = charbonnier
 // (sres/controller/dual_trainer.py:196-198), 2 = l1 (north_star variant, not in the reference).
 // Forward stage 1: per-block sums of f(d); stage 2: one block sums the partials in order and
@@ -182,6 +276,38 @@ extern "C" int sres_bicubic_resize(const float* in, float* out, int planes, int 
   bicubic_resize_kernel<<<ew_grid(total), 256, 0, (cudaStream_t)stream>>>(in, out, planes, Hi, Wi, Ho, Wo,
                                                                           (float)scale_h, (float)scale_w);
   SRES_CHECK_LAUNCH("bicubic: launch");
+  return SRES_OK;
+}
+
+extern "C" int sres_resize(const float* in, float* out, int planes, int Hi, int Wi, int Ho, int Wo, double scale_h,
+                           double scale_w, int mode, void* stream) {
+  if (!in || !out) return set_error(SRES_ERR_INVALID_ARG, "resize: null pointer");
+  if (planes <= 0 || Hi <= 0 || Wi <= 0 || Ho <= 0 || Wo <= 0) return set_error(SRES_ERR_INVALID_ARG, "resize: bad shape");
+  if (mode < SRES_RESIZE_NEAREST || mode > SRES_RESIZE_AREA)
+    return set_error(SRES_ERR_INVALID_ARG, "resize: unknown mode (SRES_RESIZE_NEAREST .. SRES_RESIZE_AREA)");
+  if (mode != SRES_RESIZE_AREA && !(scale_h > 0.0 && scale_w > 0.0 && scale_h < INFINITY && scale_w < INFINITY))
+    return set_error(SRES_ERR_INVALID_ARG, "resize: scales must be positive and finite");
+  if (mode == SRES_RESIZE_BICUBIC) return sres_bicubic_resize(in, out, planes, Hi, Wi, Ho, Wo, scale_h, scale_w, stream);
+  const long long total = (long long)planes * Ho * Wo;
+  const int grid = ew_grid(total);
+  const float sh = (float)scale_h, sw = (float)scale_w;
+  const cudaStream_t st = (cudaStream_t)stream;
+  const int rows16 = (Wi % 4 == 0) && ((uintptr_t)in % 16 == 0);
+  switch (mode) {
+    case SRES_RESIZE_NEAREST:
+      resize_kernel<SRES_RESIZE_NEAREST><<<grid, 256, 0, st>>>(in, out, planes, Hi, Wi, Ho, Wo, sh, sw, rows16);
+      break;
+    case SRES_RESIZE_NEAREST_EXACT:
+      resize_kernel<SRES_RESIZE_NEAREST_EXACT><<<grid, 256, 0, st>>>(in, out, planes, Hi, Wi, Ho, Wo, sh, sw, rows16);
+      break;
+    case SRES_RESIZE_BILINEAR:
+      resize_kernel<SRES_RESIZE_BILINEAR><<<grid, 256, 0, st>>>(in, out, planes, Hi, Wi, Ho, Wo, sh, sw, rows16);
+      break;
+    default:
+      resize_kernel<SRES_RESIZE_AREA><<<grid, 256, 0, st>>>(in, out, planes, Hi, Wi, Ho, Wo, sh, sw, rows16);
+      break;
+  }
+  SRES_CHECK_LAUNCH("resize: launch");
   return SRES_OK;
 }
 

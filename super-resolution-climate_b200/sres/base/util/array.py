@@ -8,6 +8,7 @@ import torch
 from sres.base.gpu import get_device
 from sres.base.util.config import cfg
 from sres_b200 import nn as _snn
+from sres_b200._lib import RESIZE_MODES
 
 Tensor = torch.Tensor
 
@@ -35,9 +36,12 @@ def array2tensor(darray) -> Tensor:
 
 def _resize(t: Tensor, factor: float, down: bool) -> Tensor:
     mode = torch_interp_mode(down)
-    if mode != "bicubic":
-        raise NotImplementedError(f"sres (B200 build): interpolation mode '{mode}' has no CUDA kernel (bicubic only)")
-    return _snn.bicubic_resize(t, factor)
+    if mode == "bicubic":
+        return _snn.bicubic_resize(t, factor)
+    if mode not in RESIZE_MODES:
+        raise ValueError(f"sres (B200 build): interpolation mode '{mode}' is not supported; task.downsample_mode / "
+                         "upsample_mode accepts cubic, linear, nearest, nearest-exact, area (or bicubic, bilinear)")
+    return _snn.resize(t, factor, mode)
 
 
 def downsample(target_data, **kwargs) -> Tensor:

@@ -14,6 +14,8 @@ EPI_RELU = 1
 EPI_POOL = 2
 EPI_DOT = 4
 MAP_IDENT, MAP_SHUFFLE, MAP_UNSHUFFLE = 0, 1, 2
+# SRES_RESIZE_* of include/sres_b200.h, keyed by F.interpolate's mode names
+RESIZE_MODES = {"nearest": 0, "nearest-exact": 1, "bilinear": 2, "bicubic": 3, "area": 4}
 
 
 class SresError(RuntimeError):
@@ -67,6 +69,9 @@ def lib():
         L.sres_last_error.restype = C.c_char_p
         L.sres_ptl_rows.restype = C.c_int64
         L.sres_launch_count.restype = C.c_longlong
+        L.sres_resize.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_double,
+                                  C.c_double, C.c_int, C.c_void_p]
+        L.sres_resize.restype = C.c_int
         _lib = L
     return _lib
 

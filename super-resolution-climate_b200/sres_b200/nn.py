@@ -1,5 +1,6 @@
 """torch.nn surface of the CUDA engine: an nn.Module with the reference RCAN's parameter names whose
-forward/backward are single C-ABI calls, CUDA losses, bicubic resize and a fused flat Adam.
+forward/backward are single C-ABI calls, CUDA losses, resize (bicubic and the other interpolation modes) and a fused
+flat Adam.
 
 Reference interface mirrored here:
   RCAN / get_model            sres/model/rcan/network.py:5-27
@@ -303,6 +304,23 @@ def bicubic_resize(t: torch.Tensor, scale_factor: float) -> torch.Tensor:
     with torch.cuda.device(x.device):
         L.check(L.lib().sres_bicubic_resize(L.ptr(x), L.ptr(out), B * Cc, Hi, Wi, Ho, Wo, C.c_double(1.0 / scale_factor),
                                             C.c_double(1.0 / scale_factor), L.cur_stream()), "sres_bicubic_resize")
+    return out
+
+
+def resize(t: torch.Tensor, scale_factor: float, mode: str) -> torch.Tensor:
+    """F.interpolate(t, scale_factor=scale_factor, mode=mode) for 4-D input on the CUDA kernels (no autograd).
+    mode: 'nearest', 'nearest-exact', 'bilinear', 'bicubic' or 'area' (align_corners=False, no antialias)."""
+    if mode not in L.RESIZE_MODES:
+        raise ValueError(f"sres_b200.resize: mode '{mode}' is not one of {', '.join(L.RESIZE_MODES)}")
+    if t.device.type != "cuda":
+        raise L.SresError("sres_b200.resize needs a CUDA tensor")
+    x = t.detach().contiguous().float()
+    B, Cc, Hi, Wi = x.shape
+    Ho, Wo = int(math.floor(Hi * scale_factor)), int(math.floor(Wi * scale_factor))
+    out = torch.empty(B, Cc, Ho, Wo, device=x.device, dtype=torch.float32)
+    with torch.cuda.device(x.device):
+        L.check(L.lib().sres_resize(L.ptr(x), L.ptr(out), B * Cc, Hi, Wi, Ho, Wo, 1.0 / scale_factor, 1.0 / scale_factor,
+                                    L.RESIZE_MODES[mode], L.cur_stream()), "sres_resize")
     return out
 
 
