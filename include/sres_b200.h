@@ -104,14 +104,13 @@ typedef struct sres_conv_args {
   int32_t sub_i, sub_j;    /* sub-pixel of SRES_MAP_SHUFFLE                                     */
   int32_t shuffle_factor;  /* PixelShuffle factor of SRES_MAP_(UN)SHUFFLE; 0 means 2             */
   int32_t debug_flags;     /* bring-up only: bit1 (2) forces the direct (non-TMA) epilogue, bit4 (16) the runtime-flag
-                              instance, bit6 (64) the tap-per-MMA kernel (partial sums per 128-row tile), bit7 (128) the
-                              three-taps-per-MMA kernel (partial sums per 126-row tile) whatever SRES_CONV_N192 says */
+                              instance, bit6 (64) the tap-per-MMA kernel for the n_out == 16 tail conv (bit1 does too)
+                              instead of the three-taps-per-MMA one                                                     */
   void* debug_timeline;    /* bring-up only: int64 [grid][16] per-CTA clock stamps, or NULL          */
 } sres_conv_args;
 
-/* Output rows per M tile of the convolutions that emit per-tile partial sums for (H,W) images: 126 when the
- * three-taps-per-MMA kernel serves them (SRES_CONV_N192=2; tiles of 128 MMA rows overlap by two), else 128.  pool_part is indexed
- * [tile][segment][lane quarter][64] with tile = first output row / sres_conv_tile_rows.                      */
+/* Output rows per M tile of the convolutions that emit per-tile partial sums for (H,W) images: 128 for every geometry.
+ * pool_part is indexed [tile][segment][lane quarter][64] with tile = first output row / sres_conv_tile_rows.    */
 SRES_API int sres_conv_tile_rows(int H, int W);
 /* Number of M tiles of a (B,H,W) batch (size of pool_part's leading dim). */
 SRES_API int sres_conv_mtiles(int B, int H, int W);

@@ -47,18 +47,11 @@ int device_sm_count() {
   return cached_sms;
 }
 
-// Grid of a persistent kernel that walks n_tiles equal tiles.  SRES_MIN_GRID=1 picks the FEWEST CTAs that still finish in the
-// minimal number of waves: 1201 tiles on 148 SMs take 9 waves whether 148 or 134 CTAs share them (134 x 9 >= 1201), which
-// leaves 14 SMs to the NCCL all-reduce kernels of the data-parallel backward.  Off by default: on one GPU it is 1.3 % SLOWER
-// (28.49 vs 28.11 ms per step) -- with 148 CTAs the 131 that own only 8 tiles free their SMs a tile early, and the next
-// kernel's prologue (barriers, TMEM, 72 KB of weights) runs there under programmatic dependent launch.
-int persistent_grid(int n_tiles, int sms) {
-  if (n_tiles <= sms) return n_tiles;
-  static const int on = [] { const char* e = getenv("SRES_MIN_GRID"); return e ? atoi(e) : 0; }();
-  if (!on) return sms;
-  const int waves = (n_tiles + sms - 1) / sms;
-  return (n_tiles + waves - 1) / waves;
-}
+// Grid of a persistent kernel that walks n_tiles equal tiles: every SM, even when fewer CTAs would finish in the same number
+// of waves (1201 tiles take 9 waves on 148 or on 134 CTAs).  With 148 CTAs the 131 that own only 8 tiles free their SMs a
+// tile early, and the next kernel's prologue (barriers, TMEM, 72 KB of weights) runs there under programmatic dependent
+// launch: the smallest grid measured 1.3 % slower per training step on one B200 (28.49 vs 28.11 ms).
+int persistent_grid(int n_tiles, int sms) { return n_tiles < sms ? n_tiles : sms; }
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                   const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,

@@ -56,16 +56,13 @@ struct ConvKParams {
   long long* timeline;  // bring-up only: per-CTA clock stamps [grid][16]
 };
 
-// PAIR = true: launched as clusters of two CTAs that run every UMMA together (cta_group::2, M = 256): tile
-// 2k goes to the pair's rank 0, tile 2k+1 to rank 1, and each CTA keeps only HALF of the packed weights
-// (output features [32*rank, 32*rank+32) of every tap) -- a third less B-operand traffic out of shared
-// memory, which is what bounds this kernel, and 36 KB more room for the halo ring.
 // FL >= 0: an instance specialised at compile time for one epilogue flavour of the TMA-staged path (bit set below);
 // the RCAB loop's four convolutions each get one, which keeps the epilogue's code and instruction count small --
-// it shares the SM's issue ports and instruction cache with the single MMA-issuing thread.  FL = -1 is the generic
-// kernel (runtime flags, all mappings).  kFlFrag selects the fragment-layout epilogue for the column reductions.
-constexpr int kFlO16 = 1, kFlO32 = 2, kFlR32 = 4, kFlMsk = 8, kFlRelu = 16, kFlPool = 32, kFlDot = 64, kFlFrag = 128;
-template <int N_OUT, bool PAIR, int FL>
+// it shares the SM's issue ports and instruction cache with the single MMA-issuing thread.  The specialised pooled /
+// dot-product instances reduce their columns in the fragment layout; FL = -1 is the generic kernel (runtime flags, all
+// mappings, column sums in the row layout).
+constexpr int kFlO16 = 1, kFlO32 = 2, kFlR32 = 4, kFlMsk = 8, kFlRelu = 16, kFlPool = 32, kFlDot = 64;
+template <int N_OUT, int FL>
 __global__ void __launch_bounds__(kConvThreads, 1)
 conv3x3_igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmW,
                      const __grid_constant__ CUtensorMap tmO16, const __grid_constant__ CUtensorMap tmMsk,
@@ -75,10 +72,7 @@ conv3x3_igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
   // 1024-B aligned carve-up (128B swizzle atoms are 1024 B).
   // offset arithmetic (not an integer round trip) keeps the pointer in the shared address space: LDS/STS, not generic LD/ST
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-  constexpr int kWRows = PAIR ? N_OUT / 2 : N_OUT;  // weight rows (output features) per tap held by this CTA
-  constexpr int kWBytes = 9 * kWRows * 128;
-  const uint32_t rank = PAIR ? cluster_ctarank() : 0u;
-  const bool lead_cta = rank == 0;
+  constexpr int kWBytes = 9 * N_OUT * 128;
   uint8_t* smem_w = smem;
   uint8_t* smem_a = smem + kWBytes;
   const int stage_bytes = p.stage_rows * 128;
@@ -118,24 +112,18 @@ conv3x3_igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
     mbar_init(bar_w, 1);
     for (int i = 0; i < kAccStages; ++i) {
       mbar_init(&bar_tfull[i], 1);
-      mbar_init(&bar_tempty[i], PAIR ? 16 : 8);  // one arrive per epilogue warp (of both CTAs of a pair)
+      mbar_init(&bar_tempty[i], 8);  // one arrive per epilogue warp
     }
     for (int i = 0; i < 8; ++i) mbar_init(&bar_in[i], 1);
     mbar_fence_init();
   }
   if (warp == 2) {
-    if constexpr (PAIR) {
-      tmem_alloc2(tmem_holder, tmem_cols);
-      tmem_relinquish2();
-    } else {
-      tmem_alloc(tmem_holder, tmem_cols);
-      tmem_relinquish();
-    }
+    tmem_alloc(tmem_holder, tmem_cols);
+    tmem_relinquish();
   }
   if (threadIdx.x < N_OUT) s_bias[threadIdx.x] = p.bias ? p.bias[threadIdx.x] : 0.f;
   tc_fence_before();
-  if constexpr (PAIR) cluster_sync_all();  // the peer's barriers must be initialised before anything signals them
-  else __syncthreads();
+  __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = __shfl_sync(0xffffffffu, *tmem_holder, 0);
   if (warp == 0) SRES_STAMP(1);
@@ -145,39 +133,27 @@ conv3x3_igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
     // ===================== TMA producer (whole warp runs the loop, one elected lane issues) ==========
     const bool leader = elect_one();
     if (leader) {
-      if constexpr (PAIR) {
-        const uint32_t lbar_w = mapa_u32(smem_u32(bar_w), 0);
-        if (lead_cta) mbar_expect_tx(bar_w, 2 * kWBytes);
-        for (int t = 0; t < 9; ++t) tma_load_2d_pair(smem_w + t * kWRows * 128, &tmW, lbar_w, 0, t * N_OUT + int(rank) * kWRows);
-      } else {
-        mbar_expect_tx(bar_w, kWBytes);
-        for (int t = 0; t < 9; ++t) tma_load_2d(smem_w + t * N_OUT * 128, &tmW, bar_w, 0, t * N_OUT);
-      }
+      mbar_expect_tx(bar_w, kWBytes);
+      for (int t = 0; t < 9; ++t) tma_load_2d(smem_w + t * N_OUT * 128, &tmW, bar_w, 0, t * N_OUT);
     }
     pdl_wait();  // the packed weights are old; the activations come from the previous kernel
     int it = 0;
-    for (int tile = blockIdx.x; (PAIR ? (tile & ~1) : tile) < p.n_tiles; tile += gridDim.x, ++it) {
+    for (int tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x, ++it) {
       const int slot = it % p.nstage;
       const uint32_t ph = (it / p.nstage) & 1;
       mbar_wait(&bar_empty[slot], ph ^ 1, 1);
       const int row0 = tile * 128 - (p.P + 1);
       uint8_t* dst = smem_a + slot * stage_bytes;
       if (leader) {
-        if constexpr (PAIR) {  // both CTAs' bytes complete on the leader CTA's barrier
-          const uint32_t lbar = mapa_u32(smem_u32(&bar_full[slot]), 0);
-          if (lead_cta) mbar_expect_tx(&bar_full[slot], 2 * stage_bytes);
-          for (int r = 0; r < p.stage_rows; r += p.box_rows) tma_load_2d_pair(dst + r * 128, &tmA, lbar, 0, row0 + r);
-        } else {
-          mbar_expect_tx(&bar_full[slot], stage_bytes);
-          for (int r = 0; r < p.stage_rows; r += p.box_rows) tma_load_2d(dst + r * 128, &tmA, &bar_full[slot], 0, row0 + r);
-        }
+        mbar_expect_tx(&bar_full[slot], stage_bytes);
+        for (int r = 0; r < p.stage_rows; r += p.box_rows) tma_load_2d(dst + r * 128, &tmA, &bar_full[slot], 0, row0 + r);
       }
       __syncwarp();
     }
-  } else if (warp == 1 && lead_cta) {
+  } else if (warp == 1) {
     // ===================== MMA issuer (whole warp runs the loop, one elected lane issues) ==========
     const bool leader = elect_one();
-    constexpr uint32_t idesc = make_idesc_bf16(PAIR ? 256 : 128, N_OUT, 0, 0);
+    constexpr uint32_t idesc = make_idesc_bf16(128, N_OUT, 0, 0);
     constexpr uint32_t dhi = sdesc_hi_sw128(1024);
     const uint32_t w_lo = sdesc_lo(smem_u32(smem_w), 16);
     const uint32_t a_lo0 = sdesc_lo(smem_u32(smem_a), 16);
@@ -185,7 +161,7 @@ conv3x3_igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
     mbar_wait(bar_w, 0, 2);
     SRES_STAMP(3);
     int it = 0;
-    for (int tile = blockIdx.x; (PAIR ? (tile & ~1) : tile) < p.n_tiles; tile += gridDim.x, ++it) {
+    for (int tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x, ++it) {
       const int slot = it % p.nstage;
       const uint32_t ph = (it / p.nstage) & 1;
       const int acc = it % kAccStages;
@@ -204,25 +180,15 @@ conv3x3_igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
 #pragma unroll
         for (int t = 0; t < 9; ++t) {
           const uint32_t a_tap = a_tile + uint32_t(t / 3) * row_step + uint32_t(t % 3) * 8;
-          const uint32_t b_tap = w_lo + uint32_t(t * kWRows * 8);
+          const uint32_t b_tap = w_lo + uint32_t(t * N_OUT * 8);
 #pragma unroll
           for (int k = 0; k < 4; ++k) {
-            if constexpr (PAIR) {
-              if (t == 0 && k == 0) umma2_bf16_lohi<false>(d_tmem, a_tap, dhi, b_tap, dhi, idesc);
-              else umma2_bf16_lohi<true>(d_tmem, a_tap + k * 2, dhi, b_tap + k * 2, dhi, idesc);
-            } else {
-              if (t == 0 && k == 0) umma_bf16_lohi<false>(d_tmem, a_tap, dhi, b_tap, dhi, idesc);
-              else umma_bf16_lohi<true>(d_tmem, a_tap + k * 2, dhi, b_tap + k * 2, dhi, idesc);
-            }
+            if (t == 0 && k == 0) umma_bf16_lohi<false>(d_tmem, a_tap, dhi, b_tap, dhi, idesc);
+            else umma_bf16_lohi<true>(d_tmem, a_tap + k * 2, dhi, b_tap + k * 2, dhi, idesc);
           }
         }
-        if constexpr (PAIR) {
-          umma_commit2(&bar_empty[slot]);  // both CTAs' ring slots / accumulators
-          umma_commit2(&bar_tfull[acc]);
-        } else {
-          umma_commit(&bar_empty[slot]);  // smem slot free once these MMAs retire
-          umma_commit(&bar_tfull[acc]);   // accumulator ready
-        }
+        umma_commit(&bar_empty[slot]);  // smem slot free once these MMAs retire
+        umma_commit(&bar_tfull[acc]);   // accumulator ready
       }
       __syncwarp();
     }
@@ -240,7 +206,7 @@ conv3x3_igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
     uint8_t* s32 = smem + p.off_s32 + ew * 4096;   // 32 rows x 128 B (fp32 half rows, 128B swizzle)
     uint64_t* bin = &bar_in[ew];
     constexpr bool kSpec = FL >= 0;
-    constexpr bool FRAG = kSpec && (FL & kFlFrag);
+    constexpr bool FRAG = kSpec && (FL & (kFlPool | kFlDot));
     const bool f_tma = kSpec ? true : bool(p.tma_epi);
     const bool f_o16 = kSpec ? bool(FL & kFlO16) : bool(p.use_o16);
     const bool f_o32 = kSpec ? bool(FL & kFlO32) : bool(p.use_o32);
@@ -261,11 +227,10 @@ conv3x3_igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
     }
     pdl_wait();
     int it = 0;
-    for (int tile = blockIdx.x; (PAIR ? (tile & ~1) : tile) < p.n_tiles; tile += gridDim.x, ++it) {
+    for (int tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x, ++it) {
       const int acc = it % kAccStages;
       const uint32_t aph = (it / kAccStages) & 1;
       const int row0 = tile * 128 + wq * 32;
-      const bool tile_ok = !PAIR || tile < p.n_tiles;  // an odd tile count leaves rank 1's last tile empty
       if (f_tma) {
         // the slab must have been read out by the previous tile's TMA stores; then prefetch this tile's
         // fp32 addend / mask while the tensor core is still working on it
@@ -347,12 +312,10 @@ conv3x3_igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
           // one column total per lane; an unmixed warp belongs to exactly one image segment
           const float t0 = frag_colsum(cs0, lane);
           const float t1 = mixed ? frag_colsum(cs1, lane) : 0.f;
-          if (tile_ok) {
-            float* dst = p.pool_part + ((long long)tile * 2 * 4 + wq) * 64 + half * 32 + fcol;
-            const bool all1 = seg1 == 0xffffffffu;
-            dst[0] = all1 ? 0.f : t0;
-            dst[4 * 64] = all1 ? t0 : t1;
-          }
+          float* dst = p.pool_part + ((long long)tile * 2 * 4 + wq) * 64 + half * 32 + fcol;
+          const bool all1 = seg1 == 0xffffffffu;
+          dst[0] = all1 ? 0.f : t0;
+          dst[4 * 64] = all1 ? t0 : t1;
         } else {
         uint32_t raw[16 * NCH];
         if constexpr (N_OUT == 64) {
@@ -428,7 +391,7 @@ conv3x3_igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
                   t[8 * j + 2 * e + 1] = v[8 * j + 2 * e + 1] * bf16_hi(w4[e]);
                 }
               }
-              if (tile_ok) pool_partials(t, seg, lane, p.pool_part + ((long long)tile * 2 * 4 + wq) * 64 + c0);
+              pool_partials(t, seg, lane, p.pool_part + ((long long)tile * 2 * 4 + wq) * 64 + c0);
             }
             if (f_o32) {
 #pragma unroll
@@ -443,8 +406,7 @@ conv3x3_igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
                     make_uint4(pack_bf16x2(v[8 * j], v[8 * j + 1]), pack_bf16x2(v[8 * j + 2], v[8 * j + 3]),
                                pack_bf16x2(v[8 * j + 4], v[8 * j + 5]), pack_bf16x2(v[8 * j + 6], v[8 * j + 7]));
             }
-            if (f_pool && tile_ok)
-              pool_partials(v, seg, lane, p.pool_part + ((long long)tile * 2 * 4 + wq) * 64 + c0);
+            if (f_pool) pool_partials(v, seg, lane, p.pool_part + ((long long)tile * 2 * 4 + wq) * 64 + c0);
           }
         } else {
           // ---------------- direct epilogue (PixelShuffle scatter / planar output / narrow conv) ----------------
@@ -528,8 +490,7 @@ conv3x3_igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
                   if (c0 + c < p.c_real) p.out_nchw[(((long long)b * p.c_real + c0 + c) * p.H + y) * p.W + x] = v[c];
               }
             }
-            if (f_pool && tile_ok)
-              pool_partials(v, seg, lane, p.pool_part + ((long long)tile * 2 * 4 + wq) * 64 + c0);
+            if (f_pool) pool_partials(v, seg, lane, p.pool_part + ((long long)tile * 2 * 4 + wq) * 64 + c0);
           }
         }
         }
@@ -537,10 +498,7 @@ conv3x3_igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
       // accumulator stage drained (all tcgen05.ld of this warp have completed)
       tc_fence_before();
       __syncwarp();
-      if (lane == 0) {
-        if constexpr (PAIR) mbar_arrive_cluster(mapa_u32(smem_u32(&bar_tempty[acc]), 0));
-        else mbar_arrive(&bar_tempty[acc]);
-      }
+      if (lane == 0) mbar_arrive(&bar_tempty[acc]);
       if (f_tma) {
         fence_proxy_async_smem();
         __syncwarp();
@@ -557,58 +515,14 @@ conv3x3_igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
   }
 
   tc_fence_before();
-  if constexpr (PAIR) cluster_sync_all();  // neither CTA may leave while the other still signals it / its MMAs run
-  else __syncthreads();
+  __syncthreads();
   if (tl && threadIdx.x == 0) {
     unsigned long long gt;
     asm volatile("mov.u64 %0, %globaltimer;" : "=l"(gt));
     tl[11] = (long long)gt;
     tl[12] = clock64();
   }
-  if (warp == 2) {
-    if constexpr (PAIR) tmem_dealloc2(tmem_base, tmem_cols);
-    else tmem_dealloc(tmem_base, tmem_cols);
-  }
-}
-
-// launch with programmatic dependent launch and, for the CTA-pair kernel, a cluster dimension of 2
-template <typename... KArgs, typename... Args>
-static cudaError_t launch_conv_kernel(bool pair, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
-                                      Args... args) {
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
-  cudaLaunchAttribute at[2];
-  int n = 0;
-  if (pdl_enabled()) {
-    at[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[n].val.programmaticStreamSerializationAllowed = 1;
-    ++n;
-  }
-  if (pair) {
-    at[n].id = cudaLaunchAttributeClusterDimension;
-    at[n].val.clusterDim.x = 2; at[n].val.clusterDim.y = 1; at[n].val.clusterDim.z = 1;
-    ++n;
-  }
-  cfg.attrs = at;
-  cfg.numAttrs = n;
-  count_launch();
-  return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
-}
-
-static bool conv_frag_enabled() {
-  static const int on = [] {
-    const char* e = getenv("SRES_CONV_FRAG");
-    return e ? atoi(e) : 1;
-  }();
-  return on != 0;
-}
-
-static bool conv_pair_enabled() {
-  static const int on = [] {
-    const char* e = getenv("SRES_CONV_PAIR");
-    return e ? atoi(e) : 0;  // measured slower than the single-CTA kernel for N = 64 (see DESIGN.md)
-  }();
-  return on != 0;
+  if (warp == 2) tmem_dealloc(tmem_base, tmem_cols);
 }
 
 // ---------------------------------------------------------------------------
@@ -626,20 +540,11 @@ static int launch_conv(const sres_conv_args* a, cudaStream_t stream) {
                                          a->out_nchw || (a->debug_flags & 2)))
     return set_error(SRES_ERR_INVALID_ARG, "conv: SRES_EPI_DOT needs mask_bf16 (the other factor), identity mapping, 64 outputs and no SRES_EPI_POOL");
 
-  // The RCAB loop's convolutions (identity mapping, TMA-staged epilogue, one fp32 addend at most) run on the
-  // three-taps-per-MMA kernel; debug_flags bit 6 (64) keeps them on this one for A/B runs and tests.
-  {
-    const bool ident_tma = a->map_mode == SRES_MAP_IDENT && a->n_out == 64 && !a->out_nchw && !a->resid2_f32 &&
-                           !(a->debug_flags & (2 | 4 | 8 | 32 | 64));
-    if (ident_tma && conv_n192_fits(a)) return launch_conv_n192(a, stream);
-    if ((a->epi_flags & (SRES_EPI_POOL | SRES_EPI_DOT)) && conv_n192_available(a->H, a->W) && !(a->debug_flags & (2 | 4 | 8 | 32 | 64)))
-      return set_error(SRES_ERR_UNSUPPORTED, "conv: with SRES_CONV_N192=2 per-tile partial sums need the identity-mapped TMA epilogue with one output and no second addend");
-  }
-  // tail convolution (16 packed output rows, planar output): the three-taps-per-MMA kernel's narrow variant; its halo
-  // staging does not grow with the image width (debug_flags bit 6 keeps the tap-per-MMA kernel)
+  // tail convolution (16 packed output rows, planar output): the three-taps-per-MMA kernel of conv_n192.cu, whose halo
+  // staging does not grow with the image width (debug_flags bits 1 and 6 keep the tap-per-MMA kernel)
   if (a->n_out == 16 && a->out_nchw && a->map_mode == SRES_MAP_IDENT && !a->out_f32 && !a->out_bf16 && !a->resid_f32 &&
       !a->resid2_f32 && !a->mask_bf16 && !(a->epi_flags & (SRES_EPI_POOL | SRES_EPI_DOT)) && a->c_real >= 1 && a->c_real <= 16 &&
-      !(a->debug_flags & (2 | 4 | 8 | 32 | 64)) && conv_n48_available(a->H, a->W))
+      !(a->debug_flags & (2 | 64)) && conv_n48_available(a->H, a->W))
     return launch_conv_n48(a, stream);
   ConvKParams p{};
   p.B = a->B; p.H = a->H; p.W = a->W; p.P = a->W + 1; p.R = a->H + 1;
@@ -658,16 +563,14 @@ static int launch_conv(const sres_conv_args* a, cudaStream_t stream) {
     p.use_o16 = a->out_bf16 != nullptr; p.use_msk = a->mask_bf16 != nullptr;
     p.use_r32 = a->resid_f32 != nullptr; p.use_o32 = a->out_f32 != nullptr;
   }
-  // CTA pairs for the 64-output convolutions (debug_flags bit 2 forces the single-CTA kernel)
-  const bool pair = a->n_out == 64 && p.n_tiles >= 2 && (conv_pair_enabled() || (a->debug_flags & 8)) && !(a->debug_flags & 4);
-  const int wbytes = 9 * (pair ? a->n_out / 2 : a->n_out) * 128;
+  const int wbytes = 9 * a->n_out * 128;
   const int smem_max = 232448;  // 227 KB
   const int tail_bytes = 1024;
   int slab_bytes = (p.use_o16 ? 16384 : 0) + (p.use_msk ? 16384 : 0) + ((p.use_r32 | p.use_o32) ? 32768 : 0);
   const int rows = 128 + 2 * (p.P + 1);
   // one TMA box of the exact window (rounded to the 8-row swizzle atom) when it fits the 256-row box limit: fewer bytes
   // into shared memory (232 instead of 256 rows at 48x48) and one TMA instruction per tile instead of four
-  const bool one_box = (rows + 7) / 8 * 8 <= 256 && !getenv("SRES_CONV_BOX64");
+  const bool one_box = (rows + 7) / 8 * 8 <= 256;
   p.box_rows = one_box ? (rows + 7) / 8 * 8 : kBoxRows;
   p.stage_rows = (rows + p.box_rows - 1) / p.box_rows * p.box_rows;
   int ns = (smem_max - 1024 - wbytes - tail_bytes - slab_bytes) / (p.stage_rows * 128);
@@ -689,7 +592,7 @@ static int launch_conv(const sres_conv_args* a, cudaStream_t stream) {
   CUtensorMap tmA, tmW, tmO16, tmMsk, tmR32, tmO32;
   int rc = make_tmap_rows64(&tmA, a->in_bf16, (uint64_t)p.npos, p.box_rows);
   if (rc) return rc;
-  rc = make_tmap_rows64(&tmW, a->wpack_bf16, (uint64_t)(9 * a->n_out), pair ? a->n_out / 2 : a->n_out);
+  rc = make_tmap_rows64(&tmW, a->wpack_bf16, (uint64_t)(9 * a->n_out), a->n_out);
   if (rc) return rc;
   tmO16 = tmA; tmMsk = tmA; tmR32 = tmA; tmO32 = tmA;
   if (p.tma_epi) {
@@ -701,46 +604,39 @@ static int launch_conv(const sres_conv_args* a, cudaStream_t stream) {
 
   int sms = device_sm_count();
   if (sms <= 0) return set_error(SRES_ERR_NO_DEVICE, "conv: no CUDA device");
-  int grid = persistent_grid(p.n_tiles, sms);
+  const int grid = persistent_grid(p.n_tiles, sms);
   cudaError_t e = cudaSuccess;
   int dev = 0;
   cudaGetDevice(&dev);
   // compile-time flavour of the TMA-staged epilogue, if this call is one of the specialised ones
   int fl = -1;
-  if (p.tma_epi && !pair && !a->resid2_f32 && !(a->debug_flags & 16)) {
+  if (p.tma_epi && !a->resid2_f32 && !(a->debug_flags & 16)) {
     fl = (p.use_o16 ? kFlO16 : 0) | (p.use_o32 ? kFlO32 : 0) | (p.use_r32 ? kFlR32 : 0) | (p.use_msk ? kFlMsk : 0) |
          ((a->epi_flags & SRES_EPI_RELU) ? kFlRelu : 0) | ((a->epi_flags & SRES_EPI_POOL) ? kFlPool : 0) |
          ((a->epi_flags & SRES_EPI_DOT) ? kFlDot : 0);
-    if ((fl & (kFlPool | kFlDot)) && conv_frag_enabled() && !(a->debug_flags & 32)) fl |= kFlFrag;
   }
-#define SRES_CONV_CASE(NOUT, PAIRED, FLV)                                                                                  \
+#define SRES_CONV_CASE(NOUT, FLV)                                                                                        \
   {                                                                                                                      \
     static thread_local int attr_dev = -1;                                                                               \
     if (attr_dev != dev) {                                                                                               \
-      e = cudaFuncSetAttribute(conv3x3_igemm_kernel<NOUT, PAIRED, FLV>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max); \
+      e = cudaFuncSetAttribute(conv3x3_igemm_kernel<NOUT, FLV>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);  \
       if (e != cudaSuccess) return set_cuda_error(e, "conv: smem attribute");                                           \
       attr_dev = dev;                                                                                                    \
     }                                                                                                                    \
-    e = launch_conv_kernel(PAIRED, conv3x3_igemm_kernel<NOUT, PAIRED, FLV>, dim3(grid), dim3(kConvThreads), smem, stream, tmA, \
-                           tmW, tmO16, tmMsk, tmR32, tmO32, p);                                                         \
+    e = launch_pdl(conv3x3_igemm_kernel<NOUT, FLV>, dim3(grid), dim3(kConvThreads), smem, stream, tmA, tmW, tmO16, tmMsk, \
+                   tmR32, tmO32, p);                                                                                     \
   }
-  if (pair) {
-    grid = ((p.n_tiles + 1) / 2 < sms / 2 ? (p.n_tiles + 1) / 2 : sms / 2) * 2;
-    SRES_CONV_CASE(64, true, -1)
-  } else if (a->n_out == 16) {
-    SRES_CONV_CASE(16, false, -1)
+  if (a->n_out == 16) {
+    SRES_CONV_CASE(16, -1)
   } else {
     switch (fl) {
-      case kFlRelu | kFlO16: SRES_CONV_CASE(64, false, kFlRelu | kFlO16) break;                                          // RCAB conv1
-      case kFlPool | kFlO16: SRES_CONV_CASE(64, false, kFlPool | kFlO16) break;                                          // RCAB conv2
-      case kFlPool | kFlO16 | kFlFrag: SRES_CONV_CASE(64, false, kFlPool | kFlO16 | kFlFrag) break;
-      case kFlMsk | kFlO16: SRES_CONV_CASE(64, false, kFlMsk | kFlO16) break;                                            // dgrad of conv2
-      case kFlR32 | kFlO32 | kFlMsk | kFlDot: SRES_CONV_CASE(64, false, kFlR32 | kFlO32 | kFlMsk | kFlDot) break;        // dgrad of conv1
-      case kFlR32 | kFlO32 | kFlMsk | kFlDot | kFlFrag: SRES_CONV_CASE(64, false, kFlR32 | kFlO32 | kFlMsk | kFlDot | kFlFrag) break;
-      case kFlR32 | kFlO32 | kFlO16: SRES_CONV_CASE(64, false, kFlR32 | kFlO32 | kFlO16) break;                          // EDSR conv2 / conv1 dgrad
-      case kFlO32 | kFlMsk | kFlDot: SRES_CONV_CASE(64, false, kFlO32 | kFlMsk | kFlDot) break;                          // dgrad of a group tail
-      case kFlO32 | kFlMsk | kFlDot | kFlFrag: SRES_CONV_CASE(64, false, kFlO32 | kFlMsk | kFlDot | kFlFrag) break;
-      default: SRES_CONV_CASE(64, false, -1) break;
+      case kFlRelu | kFlO16: SRES_CONV_CASE(64, kFlRelu | kFlO16) break;                                  // RCAB conv1
+      case kFlPool | kFlO16: SRES_CONV_CASE(64, kFlPool | kFlO16) break;                                  // RCAB conv2
+      case kFlMsk | kFlO16: SRES_CONV_CASE(64, kFlMsk | kFlO16) break;                                    // dgrad of conv2
+      case kFlR32 | kFlO32 | kFlMsk | kFlDot: SRES_CONV_CASE(64, kFlR32 | kFlO32 | kFlMsk | kFlDot) break;    // dgrad of conv1
+      case kFlR32 | kFlO32 | kFlO16: SRES_CONV_CASE(64, kFlR32 | kFlO32 | kFlO16) break;                  // EDSR conv2 / conv1 dgrad
+      case kFlO32 | kFlMsk | kFlDot: SRES_CONV_CASE(64, kFlO32 | kFlMsk | kFlDot) break;                  // dgrad of a group tail
+      default: SRES_CONV_CASE(64, -1) break;
     }
   }
 #undef SRES_CONV_CASE
@@ -752,7 +648,10 @@ static int launch_conv(const sres_conv_args* a, cudaStream_t stream) {
 
 }  // namespace sres
 
-extern "C" int sres_conv_tile_rows(int H, int W) { return sres::conv_n192_available(H, W) ? 126 : 128; }
+extern "C" int sres_conv_tile_rows(int H, int W) {
+  (void)H; (void)W;
+  return 128;
+}
 
 extern "C" int sres_conv_mtiles(int B, int H, int W) {
   const long long npos = (long long)B * (H + 1) * (W + 1);

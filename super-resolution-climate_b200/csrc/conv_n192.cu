@@ -1,28 +1,26 @@
-// 3x3 convolution 64 -> 64 over the padded tile layout with the three horizontal taps stacked on the UMMA N
-// dimension (sm_100a).
+// Tail convolution 64 -> Cout <= 16 over the padded tile layout with the three horizontal taps stacked on the UMMA N
+// dimension (sm_100a), planar fp32 output.
 //
-// The tap-per-MMA kernel (conv_igemm.cu) issues 36 tcgen05.mma of M128 x N64 x K16 per tile; each reads 4 KB of A and
-// 2 KB of B from shared memory per 32 tensor-pipe cycles = 192 B/clk against the 128 B/clk shared memory delivers, so
-// it can never pass 2/3 of the tensor peak (measured: 49 clk per instruction, tools/ubench_umma.cu).  Here one
-// instruction covers the three taps (ky, 0..2) of a kernel row:
+// The weights are packed with 16 output rows per tap.  One instruction covers the three taps (ky, 0..2) of a kernel row:
 //
-//     D_kx[i] = sum_ky  X[m_i + (ky-1) P] . W(ky, kx)          N = 192 = 3 x 64 output features, 12 MMAs per tile
+//     D_kx[i] = sum_ky  X[m_i + (ky-1) P] . W(ky, kx)          N = 48 = 3 x 16 output features, 12 MMAs per tile
 //     out[m_i] = D_0[i-1] + D_1[i] + D_2[i+1]                   (P = W+1: one image row of the padded tile layout)
 //
-// B for kernel row ky is simply taps 3ky..3ky+2 of the packed weights, which are contiguous (192 rows).  An MMA
-// reads 4 KB + 6 KB per 96 cycles = 107 B/clk: the tensor pipe, not shared memory, paces it (measured: 97 clk).
-// The price is paid in the epilogue: the three 64-column accumulators of a tile have to be added with a shift of
-// one TMEM lane (= one PTL row).  A warp owns 32 lanes, so the shift is a lane rotation by warp shuffle; the two
-// rows that cross a warp's lane quarter travel through a 4 KB shared-memory exchange, and because the first and last
-// MMA row of a tile have no neighbour the tiles overlap by two rows: a tile is 128 MMA rows = 126 output rows.
+// B for kernel row ky is simply taps 3ky..3ky+2 of the packed weights, which are contiguous (48 rows).  The three
+// 16-column accumulators of a tile are added with a shift of one TMEM lane (= one PTL row) in the epilogue.  A warp owns
+// 32 lanes, so the shift is a lane rotation by warp shuffle; the two rows that cross a warp's lane quarter travel
+// through a small shared-memory exchange, and because the first and last MMA row of a tile have no neighbour the tiles
+// overlap by two rows: a tile is 128 MMA rows = 126 output rows.
 //
 // The A operand of kernel row ky is the 128-row block starting (ky-1) P rows from the tile, so the halo window is
 // 128 + 2P rows (one TMA box when it fits 256 rows), or -- for wide images, where that window would not fit --
-// three independent 128-row boxes: the shared-memory footprint no longer grows with the image width (x8 upscaling
-// of 96 x 96 tiles, BASELINE config 5).
+// three independent 128-row boxes: the shared-memory footprint does not grow with the image width (x8 upscaling
+// of 96 x 96 tiles, BASELINE config 5's 768-pixel rows).
 //
-// Replaces nn.Conv2d(64, 64, 3, padding=1) forward / input-gradient of the reference
-// (sres/model/common/cnn.py:8-9 used at sres/model/rcan/network.py:55,71, sres/model/common/residual.py:30-54).
+// (The 64 -> 64 form of this kernel, N = 192, lost to the tap-per-MMA kernel of conv_igemm.cu and was removed: DESIGN.md
+// section 3.1a.)
+//
+// Replaces nn.Conv2d(64, Cout, 3, padding=1) forward of the reference's tail conv (sres/model/rcan/network.py:16).
 #include "ptx.cuh"
 #include "internal.h"
 
@@ -32,9 +30,10 @@ constexpr int kNStages = 6;
 constexpr int kNWarps = 18;             // 0 = TMA producer (+ TMEM allocation), 1 = MMA issuer, 2..17 = two epilogue groups
 constexpr int kNThreads = kNWarps * 32;
 constexpr int kNTileOut = 126;          // output rows per tile (128 MMA rows, one halo row on each side)
-constexpr int kNWBytes = 9 * 64 * 128;  // packed weights, all taps
+constexpr int kNB = 16;                 // output features per horizontal tap
+constexpr int kNWBytes = 9 * kNB * 128; // packed weights, all taps
 
-struct ConvN192Params {
+struct ConvN48Params {
   int H, W, P, R;
   int npos, n_tiles;
   int nstage, stage_bytes;
@@ -43,12 +42,9 @@ struct ConvN192Params {
   int ky_step16;       // distance between the A blocks of consecutive kernel rows, in 16-byte units
   unsigned flags;
   const float* bias;
-  const uint16_t* mask;  // bf16 PTL: ReLU mask, or the second factor of SRES_EPI_DOT (read straight from global memory)
-  float* part;           // [n_tiles][2][4][64] per-tile, per-image-segment channel sums (SRES_EPI_POOL / SRES_EPI_DOT)
-  float* out_nchw;       // narrow variant: planar fp32 output (B, c_real, H, W)
+  float* out_nchw;     // planar fp32 output (B, c_real, H, W)
   int c_real;
-  int use_o16, use_msk, use_r32, use_o32;
-  int off_s16, off_s32, off_xch, off_tail;
+  int off_xch, off_tail;
   long long* timeline;
 };
 
@@ -56,88 +52,16 @@ __device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
   asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
 }
 
-// 16-value butterfly (see conv_igemm.cu): lane l (even) ends with the sum over the 32 lanes of column l >> 1
-__device__ __forceinline__ float n192_butterfly16(float (&v)[16], int lane) {
-  {
-    const bool up = lane & 16;
-#pragma unroll
-    for (int j = 0; j < 8; ++j) {
-      const float send = up ? v[j] : v[j + 8];
-      const float keep = up ? v[j + 8] : v[j];
-      v[j] = keep + __shfl_xor_sync(0xffffffffu, send, 16);
-    }
-  }
-  {
-    const bool up = lane & 8;
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const float send = up ? v[j] : v[j + 4];
-      const float keep = up ? v[j + 4] : v[j];
-      v[j] = keep + __shfl_xor_sync(0xffffffffu, send, 8);
-    }
-  }
-  {
-    const bool up = lane & 4;
-#pragma unroll
-    for (int j = 0; j < 2; ++j) {
-      const float send = up ? v[j] : v[j + 2];
-      const float keep = up ? v[j + 2] : v[j];
-      v[j] = keep + __shfl_xor_sync(0xffffffffu, send, 4);
-    }
-  }
-  {
-    const bool up = lane & 2;
-    const float send = up ? v[0] : v[1];
-    const float keep = up ? v[1] : v[0];
-    v[0] = keep + __shfl_xor_sync(0xffffffffu, send, 2);
-  }
-  v[0] += __shfl_xor_sync(0xffffffffu, v[0], 1);
-  return v[0];
-}
-
-// per-image-segment channel sums of 16 columns -> part[tile][seg][quarter][64]
-__device__ __forceinline__ void n192_partials(const float (&v)[16], int seg, int lane, float* dst) {
-  const bool any1 = __any_sync(0xffffffffu, seg == 1);
-  const bool any0 = __any_sync(0xffffffffu, seg == 0);
-  float s0 = 0.f, s1 = 0.f;
-  if (any0) {
-    float t[16];
-#pragma unroll
-    for (int j = 0; j < 16; ++j) t[j] = seg == 0 ? v[j] : 0.f;
-    s0 = n192_butterfly16(t, lane);
-  }
-  if (any1) {
-    float t[16];
-#pragma unroll
-    for (int j = 0; j < 16; ++j) t[j] = seg == 1 ? v[j] : 0.f;
-    s1 = n192_butterfly16(t, lane);
-  }
-  if ((lane & 1) == 0) {
-    dst[lane >> 1] = s0;
-    dst[4 * 64 + (lane >> 1)] = s1;
-  }
-}
-
-// FL >= 0: epilogue flavour fixed at compile time (bits below); FL = -1: runtime flags.
-constexpr int kNO16 = 1, kNO32 = 2, kNR32 = 4, kNMsk = 8, kNRelu = 16, kNPool = 32, kNDot = 64;
-
 // Warp roles (576 threads): 0 = TMA producer, 1 = MMA issuer, 2..9 = epilogue group 0, 10..17 = epilogue group 1.
-// Group g drains accumulator stage g, i.e. every second tile of the CTA: the shifted sum costs 512 warp shuffles per
-// tile and the SM shuffles one warp per clock, so one group alone (drain, exchange, shuffle, store in sequence) needs
-// about 1700 cycles per tile against the 1164 the tensor pipe takes; two groups have two tile times each.
-// NB = output features per horizontal tap: 64 (N = 192, the trunk convolutions) or 16 (N = 48: the tail convolution
-// 64 -> Cout <= 16, planar fp32 output straight from registers, any image width -- BASELINE config 5's 768-pixel rows).
-template <int NB, int FL>
+// Group g drains accumulator stage g, i.e. every second tile of the CTA; in each group one warp per TMEM lane quarter
+// has work.
 __global__ void __launch_bounds__(kNThreads, 1)
-conv3x3_n192_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmW,
-                    const __grid_constant__ CUtensorMap tmO16a, const __grid_constant__ CUtensorMap tmO16b,
-                    const __grid_constant__ CUtensorMap tmMsk, const __grid_constant__ CUtensorMap tmR32,
-                    const __grid_constant__ CUtensorMap tmO32a, const __grid_constant__ CUtensorMap tmO32b,
-                    const ConvN192Params p) {
+conv3x3_n48_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmW,
+                   const __grid_constant__ ConvN48Params p) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);  // offset arithmetic keeps LDS/STS
   uint8_t* smem_w = smem;
-  constexpr int kWRow = 3 * NB * 128;   // bytes of one kernel row of the packed weights (three taps)
+  constexpr int kWRow = 3 * kNB * 128;  // bytes of one kernel row of the packed weights (three taps)
   uint8_t* smem_a = smem + 3 * kWRow;
   uint8_t* tail = smem + p.off_tail;
   uint64_t* bar_full = reinterpret_cast<uint64_t*>(tail);  // [kNStages]
@@ -145,14 +69,14 @@ conv3x3_n192_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
   uint64_t* bar_w = bar_empty + kNStages;                   // [3] one per kernel row of the weights
   uint64_t* bar_tfull = bar_w + 3;                          // [2]
   uint64_t* bar_tempty = bar_tfull + 2;                     // [2]
-  uint64_t* bar_in = bar_tempty + 2;                        // [16] epilogue operand loads, one per warp
+  uint64_t* bar_in = bar_tempty + 2;                        // [16]
   uint32_t* tmem_holder = reinterpret_cast<uint32_t*>(bar_in + 16);
   float* s_bias = reinterpret_cast<float*>(tmem_holder + 2);  // [64]
 
   const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0);
   const int lane = threadIdx.x & 31;
   long long* tl = p.timeline ? p.timeline + (size_t)blockIdx.x * 16 : nullptr;
-#define N192_STAMP(i)                          \
+#define N48_STAMP(i)                           \
   do {                                         \
     if (tl && lane == 0) tl[i] = clock64();    \
   } while (0)
@@ -171,21 +95,21 @@ conv3x3_n192_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
     for (int i = 0; i < 3; ++i) mbar_init(&bar_w[i], 1);
     for (int i = 0; i < 2; ++i) {
       mbar_init(&bar_tfull[i], 1);
-      mbar_init(&bar_tempty[i], NB == 64 ? 8 : 4);  // one arrive per warp of the group that drains the stage
+      mbar_init(&bar_tempty[i], 4);  // one arrive per warp of the group that drains the stage
     }
     for (int i = 0; i < 16; ++i) mbar_init(&bar_in[i], 1);
     mbar_fence_init();
   }
   if (warp == 0) {
-    tmem_alloc(tmem_holder, 512);  // two accumulator stages of 192 columns, 256 apart
+    tmem_alloc(tmem_holder, 512);  // two accumulator stages, 256 columns apart
     tmem_relinquish();
   }
-  if (threadIdx.x >= 64 && threadIdx.x < 64 + NB) s_bias[threadIdx.x - 64] = p.bias ? p.bias[threadIdx.x - 64] : 0.f;
+  if (threadIdx.x >= 64 && threadIdx.x < 64 + kNB) s_bias[threadIdx.x - 64] = p.bias ? p.bias[threadIdx.x - 64] : 0.f;
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = __shfl_sync(0xffffffffu, *tmem_holder, 0);
-  if (warp == 0) N192_STAMP(1);
+  if (warp == 0) N48_STAMP(1);
   pdl_launch_dependents();
 
   if (warp == 0) {
@@ -194,11 +118,11 @@ conv3x3_n192_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
     if (leader) {
       for (int ky = 0; ky < 3; ++ky) {   // one barrier per kernel row: the first MMAs start after a third of the weights
         mbar_expect_tx(&bar_w[ky], kWRow);
-        tma_load_2d(smem_w + ky * kWRow, &tmW, &bar_w[ky], 0, ky * 3 * NB);
+        tma_load_2d(smem_w + ky * kWRow, &tmW, &bar_w[ky], 0, ky * 3 * kNB);
       }
     }
     pdl_wait();  // the packed weights are old; the activations come from the previous kernel
-    if (warp == 0) N192_STAMP(2);
+    if (warp == 0) N48_STAMP(2);
     int it = 0;
     for (int tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x, ++it) {
       const int slot = it % p.nstage;
@@ -215,7 +139,7 @@ conv3x3_n192_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
   } else if (warp == 1) {
     // ===================== MMA issuer =====================
     const bool leader = elect_one();
-    constexpr uint32_t idesc = make_idesc_bf16(128, 3 * NB, 0, 0);
+    constexpr uint32_t idesc = make_idesc_bf16(128, 3 * kNB, 0, 0);
     constexpr uint32_t dhi = sdesc_hi_sw128(1024);
     const uint32_t w_lo = sdesc_lo(smem_u32(smem_w), 16);
     const uint32_t a_lo0 = sdesc_lo(smem_u32(smem_a), 16);
@@ -232,7 +156,7 @@ conv3x3_n192_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
       if (tl) w1 = clock64();
       mbar_wait(&bar_full[slot], ph, 4);
       if (tl && lane == 0 && it > 0) { tl[14] += w1 - w0; tl[15] += clock64() - w1; }
-      if (it == 0) N192_STAMP(4);
+      if (it == 0) N48_STAMP(4);
       tc_fence_after();
       const uint32_t a_tile = a_lo0 + uint32_t(slot * p.stage_bytes) / 16;
       const uint32_t d_tmem = tmem_base + uint32_t(acc * 256);
@@ -241,11 +165,11 @@ conv3x3_n192_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
         if (it == 0) {
           mbar_wait(&bar_w[ky], 0, 2);
           tc_fence_after();
-          if (ky == 0) N192_STAMP(3);
+          if (ky == 0) N48_STAMP(3);
         }
         if (leader) {
           const uint32_t a_row = a_tile + uint32_t(ky) * ky_step;
-          const uint32_t b_row = w_lo + uint32_t(ky * 3 * NB * 8);
+          const uint32_t b_row = w_lo + uint32_t(ky * 3 * kNB * 8);
 #pragma unroll
           for (int k = 0; k < 4; ++k) {
             if (ky == 0 && k == 0) umma_bf16_lohi<false>(d_tmem, a_row, dhi, b_row, dhi, idesc);
@@ -260,9 +184,9 @@ conv3x3_n192_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
       }
       __syncwarp();
     }
-    N192_STAMP(5);
-  } else if constexpr (NB == 16) {
-    // ===================== epilogue, narrow variant: 16 columns per tap, planar fp32 output =====================
+    N48_STAMP(5);
+  } else {
+    // ===================== epilogue: 16 columns per tap, planar fp32 output =====================
     const int ew = warp - 2;
     const int grp = ew >> 3;
     const int wq = warp & 3;
@@ -343,244 +267,22 @@ conv3x3_n192_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
         }
       }
     }
-  } else {
-    // ===================== epilogue =====================
-    const int ew = warp - 2;          // 0..15
-    const int grp = ew >> 3;          // accumulator stage / tile parity this warp serves
-    const int half = (ew >> 2) & 1;   // which 32 of the 64 output features
-    const int wq = warp & 3;          // TMEM lane quarter
-    const int RP = p.R * p.P;
-    uint8_t* s16 = smem + p.off_s16 + ew * 2048;  // 32 rows x 64 B (bf16, 64B swizzle)
-    uint8_t* s32 = smem + p.off_s32 + ew * 4096;  // 32 rows x 128 B (fp32 half rows, 128B swizzle)
-    float* xch = reinterpret_cast<float*>(smem + p.off_xch) + grp * 512;  // [2 chunks][2 directions][4 quarters][2 halves][16]
-    uint64_t* bin = &bar_in[ew];
-    constexpr bool kSpec = FL >= 0;
-    const bool f_o16 = kSpec ? bool(FL & kNO16) : bool(p.use_o16);
-    const bool f_o32 = kSpec ? bool(FL & kNO32) : bool(p.use_o32);
-    const bool f_r32 = kSpec ? bool(FL & kNR32) : bool(p.use_r32);
-    const bool f_msk = kSpec ? bool(FL & kNMsk) : bool(p.use_msk);
-    const bool f_relu = kSpec ? bool(FL & kNRelu) : bool(p.flags & SRES_EPI_RELU);
-    const bool f_pool = kSpec ? bool(FL & kNPool) : bool(p.flags & SRES_EPI_POOL);
-    const bool f_dot = kSpec ? bool(FL & kNDot) : bool(p.flags & SRES_EPI_DOT);
-    // A ReLU mask next to a bf16 output is TMA-loaded into the output slab and replaced in place; next to an fp32
-    // output (no bf16 slab) the mask / second factor comes straight from global memory, 64 bytes per row.
-    const bool msk_slab = f_msk && f_o16;
-    const bool use_in = f_r32 | msk_slab;
-    // The first quarter's lane 0 (MMA row 0) and the last quarter's lane 31 (MMA row 127) are halo rows of the
-    // neighbouring tiles: those two warps store 31-row boxes, and the first quarter keeps its rows one slab row up.
-    const int srow = wq == 0 ? ((lane + 31) & 31) : lane;
-    const int src_up = (lane + 31) & 31, src_dn = (lane + 1) & 31;
-    const int sw7 = srow & 7, sw3 = (srow >> 1) & 3;
-    uint8_t* r16 = s16 + srow * 64;
-    uint8_t* r32 = s32 + srow * 128;
-    const int bar_id = 1 + grp * 2 + half;
-    const bool tstamp = tl && ew == 0;
-    pdl_wait();
-    for (int tile = blockIdx.x + grp * gridDim.x, it = grp; tile < p.n_tiles; tile += 2 * gridDim.x, it += 2) {
-      const uint32_t aph = (it >> 1) & 1;
-      const int tile_base = tile * kNTileOut;
-      const int box_q0 = wq == 0 ? tile_base : tile_base - 1 + 32 * wq;
-      // ---- row geometry ----
-      const int i = wq * 32 + lane;           // MMA row
-      const int q = tile_base - 1 + i;        // PTL row
-      const bool own = i >= 1 && i <= kNTileOut && q < p.npos;
-      const int qc = own ? q : tile_base;
-      const int b = qc / RP;
-      const int rem = qc - b * RP;
-      const int y = rem / p.P;
-      const int x = rem - y * p.P;
-      const bool pad = !own || x == p.W || y == p.H;
-      const int seg = (b != tile_base / RP) ? 1 : 0;
-      if (lane == 0) {
-        bulk_wait_read<0>();  // the slabs have been read out by this warp's previous TMA stores
-        if (use_in) {
-          mbar_expect_tx(bin, (f_r32 ? 4096u : 0u) + (msk_slab ? 2048u : 0u));
-          if (f_r32) tma_load_2d(s32, &tmR32, bin, half * 32, box_q0);
-          if (msk_slab) tma_load_2d(s16, &tmMsk, bin, half * 32, box_q0);
-        }
-      }
-      uint4 mk[4];
-      if (f_msk && !msk_slab) {
-        const uint4* mp = reinterpret_cast<const uint4*>(p.mask + (long long)qc * 64 + half * 32);
-#pragma unroll
-        for (int j = 0; j < 4; ++j) mk[j] = __ldg(mp + j);
-      }
-      __syncwarp();
-      long long e0 = 0;
-      if (tstamp) e0 = clock64();
-      mbar_wait(&bar_tfull[grp], aph, 5);
-      if (tstamp && lane == 0 && it >= 2) tl[13] += clock64() - e0;
-      if (ew == 0) { if (it == 0) N192_STAMP(6); N192_STAMP(7); }
-      tc_fence_after();
-      if (use_in) mbar_wait(bin, (it >> 1) & 1, 6);
-      const uint32_t trow = tmem_base + (uint32_t(wq * 32) << 16) + uint32_t(grp * 256 + half * 32);
-#pragma unroll
-      for (int ch = 0; ch < 2; ++ch) {
-        const int c0 = half * 32 + ch * 16;
-        uint32_t d0[16], d1[16], d2[16];
-        tmem_ld16(trow + ch * 16, d0);
-        tmem_ld16(trow + ch * 16 + NB, d1);
-        tmem_ld16(trow + ch * 16 + 2 * NB, d2);
-        tmem_ld_wait();
-        if (ch == 1) {  // accumulator stage drained: the tensor core may reuse it
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&bar_tempty[grp]);
-        }
-        // ---- rows that cross the lane quarter: D_0 of lane 31 goes up to the next quarter, D_2 of lane 0 down ----
-        float* xs = xch + ch * 256;
-        if (lane == 31) {
-          float4* d = reinterpret_cast<float4*>(xs + ((0 * 4 + wq) * 2 + half) * 16);
-#pragma unroll
-          for (int j = 0; j < 4; ++j)
-            d[j] = make_float4(__uint_as_float(d0[4 * j]), __uint_as_float(d0[4 * j + 1]), __uint_as_float(d0[4 * j + 2]),
-                               __uint_as_float(d0[4 * j + 3]));
-        }
-        if (lane == 0) {
-          float4* d = reinterpret_cast<float4*>(xs + ((1 * 4 + wq) * 2 + half) * 16);
-#pragma unroll
-          for (int j = 0; j < 4; ++j)
-            d[j] = make_float4(__uint_as_float(d2[4 * j]), __uint_as_float(d2[4 * j + 1]), __uint_as_float(d2[4 * j + 2]),
-                               __uint_as_float(d2[4 * j + 3]));
-        }
-        named_bar_sync(bar_id, 128);  // the four quarter warps of this group and column half
-        // lane 31 now carries what lane 0 needs from the quarter below (and vice versa), so that ONE lane rotation
-        // delivers every row's neighbour
-        if (lane == 31 && wq > 0) {
-          const float4* s = reinterpret_cast<const float4*>(xs + ((0 * 4 + wq - 1) * 2 + half) * 16);
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            const float4 t = s[j];
-            d0[4 * j] = __float_as_uint(t.x); d0[4 * j + 1] = __float_as_uint(t.y);
-            d0[4 * j + 2] = __float_as_uint(t.z); d0[4 * j + 3] = __float_as_uint(t.w);
-          }
-        }
-        if (lane == 0 && wq < 3) {
-          const float4* s = reinterpret_cast<const float4*>(xs + ((1 * 4 + wq + 1) * 2 + half) * 16);
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            const float4 t = s[j];
-            d2[4 * j] = __float_as_uint(t.x); d2[4 * j + 1] = __float_as_uint(t.y);
-            d2[4 * j + 2] = __float_as_uint(t.z); d2[4 * j + 3] = __float_as_uint(t.w);
-          }
-        }
-        __syncwarp();
-        float v[16];
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          const float4 b4 = *reinterpret_cast<const float4*>(s_bias + c0 + 4 * j);
-          const float bb[4] = {b4.x, b4.y, b4.z, b4.w};
-#pragma unroll
-          for (int e = 0; e < 4; ++e) {
-            const int c = 4 * j + e;
-            float up, dn;
-            if (!kSpec && (p.flags & 0x100u)) {   // timing experiment only (wrong results): no lane rotation
-              up = __uint_as_float(d0[c]); dn = __uint_as_float(d2[c]);
-            } else {
-              up = __uint_as_float(__shfl_sync(0xffffffffu, d0[c], src_up));   // D_0 of the row above
-              dn = __uint_as_float(__shfl_sync(0xffffffffu, d2[c], src_dn));   // D_2 of the row below
-            }
-            v[c] = ((__uint_as_float(d1[c]) + bb[e]) + up) + dn;
-          }
-        }
-        if (f_r32) {
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            const float4 r = *reinterpret_cast<const float4*>(r32 + (((ch * 4 + j) ^ sw7) << 4));
-            v[4 * j + 0] += r.x; v[4 * j + 1] += r.y; v[4 * j + 2] += r.z; v[4 * j + 3] += r.w;
-          }
-        }
-        if (f_relu) {
-#pragma unroll
-          for (int j = 0; j < 16; ++j) v[j] = fmaxf(v[j], 0.f);
-        }
-        if (f_msk && !f_dot) {
-#pragma unroll
-          for (int j = 0; j < 2; ++j) {
-            const uint4 m4 = msk_slab ? *reinterpret_cast<const uint4*>(r16 + (((ch * 2 + j) ^ sw3) << 4)) : mk[ch * 2 + j];
-            const uint32_t w4[4] = {m4.x, m4.y, m4.z, m4.w};
-#pragma unroll
-            for (int e = 0; e < 4; ++e) {
-              if (!(bf16_lo(w4[e]) > 0.f)) v[8 * j + 2 * e] = 0.f;
-              if (!(bf16_hi(w4[e]) > 0.f)) v[8 * j + 2 * e + 1] = 0.f;
-            }
-          }
-        }
-        if (pad) {
-#pragma unroll
-          for (int j = 0; j < 16; ++j) v[j] = 0.f;
-        }
-        if (f_dot) {
-          float t[16];
-#pragma unroll
-          for (int j = 0; j < 2; ++j) {
-            const uint4 m4 = mk[ch * 2 + j];
-            const uint32_t w4[4] = {m4.x, m4.y, m4.z, m4.w};
-#pragma unroll
-            for (int e = 0; e < 4; ++e) {
-              t[8 * j + 2 * e] = v[8 * j + 2 * e] * bf16_lo(w4[e]);
-              t[8 * j + 2 * e + 1] = v[8 * j + 2 * e + 1] * bf16_hi(w4[e]);
-            }
-          }
-          n192_partials(t, seg, lane, p.part + ((long long)tile * 2 * 4 + wq) * 64 + c0);
-        }
-        if (f_o32) {
-#pragma unroll
-          for (int j = 0; j < 4; ++j)
-            *reinterpret_cast<float4*>(r32 + (((ch * 4 + j) ^ sw7) << 4)) =
-                make_float4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
-        }
-        if (f_o16) {
-#pragma unroll
-          for (int j = 0; j < 2; ++j)
-            *reinterpret_cast<uint4*>(r16 + (((ch * 2 + j) ^ sw3) << 4)) =
-                make_uint4(pack_bf16x2(v[8 * j], v[8 * j + 1]), pack_bf16x2(v[8 * j + 2], v[8 * j + 3]),
-                           pack_bf16x2(v[8 * j + 4], v[8 * j + 5]), pack_bf16x2(v[8 * j + 6], v[8 * j + 7]));
-        }
-        if (f_pool) n192_partials(v, seg, lane, p.part + ((long long)tile * 2 * 4 + wq) * 64 + c0);
-      }
-      fence_proxy_async_smem();
-      __syncwarp();
-      if (lane == 0) {
-        const bool short_box = wq == 0 || wq == 3;
-        if (f_o16) tma_store_2d(short_box ? &tmO16b : &tmO16a, s16, half * 32, box_q0);
-        if (f_o32) tma_store_2d(short_box ? &tmO32b : &tmO32a, s32, half * 32, box_q0);
-        bulk_commit();
-      }
-      if (ew == 0 || ew == 8) N192_STAMP(8 + grp);
-    }
-    if (lane == 0) bulk_wait_all<0>();
-    if (ew == 0) N192_STAMP(10);
   }
 
   tc_fence_before();
   __syncthreads();
   if (tl && threadIdx.x == 0) tl[12] = clock64();
   if (warp == 0) tmem_dealloc(tmem_base, 512);
-#undef N192_STAMP
+#undef N48_STAMP
 }
 
-// SRES_CONV_N192: 0 = never (default), 1 = the flavours without mask and per-tile partial sums (RCAB conv1, plain bf16 /
-// fp32 outputs), 2 = every identity-mapped flavour that fits (the per-tile partial sums of SRES_EPI_POOL / SRES_EPI_DOT
-// are then laid out per 126-row tile).  Measured on B200 (profiles/README.md, round 2): alone the kernel matches or beats
-// the tap-per-MMA kernel by 0-7 % for the light flavours (13.4 vs 13.8 us) and loses for the heavy ones; the 64-tile
-// training step is 28.32 / 28.46 / 30.45 ms in modes 0 / 1 / 2 -- the warp shuffles of the shifted sum travel through the
-// same 128 B/clk shared-memory crossbar as the UMMA operands they were meant to relieve.
-static int conv_n192_mode() {
-  static const int mode = [] {
-    const char* e = getenv("SRES_CONV_N192");
-    return e ? atoi(e) : 0;
-  }();
-  return mode;
-}
-
-// shared-memory plan: weights | ring | slabs | exchange | barriers
-struct N192Plan {
+// shared-memory plan: weights | ring | exchange | barriers
+struct N48Plan {
   int nbox, box_rows, box_step, ky_step16, stage_bytes, nstage;
-  int off_s16, off_s32, off_xch, off_tail;
+  int off_xch, off_tail;
   size_t smem;
 };
-static bool n192_plan(N192Plan* pl, int W, bool o16, bool f32slab, int wbytes = kNWBytes) {
+static bool n48_plan(N48Plan* pl, int W) {
   const int smem_max = 232448;  // 227 KB
   const int P = W + 1;
   const int window = 128 + 2 * P;   // union of the three kernel rows' 128-row blocks
@@ -593,131 +295,27 @@ static bool n192_plan(N192Plan* pl, int W, bool o16, bool f32slab, int wbytes = 
     pl->nbox = 3; pl->box_rows = 128; pl->box_step = P; pl->ky_step16 = 128 * 8;
   }
   pl->stage_bytes = pl->nbox * pl->box_rows * 128;
-  const int slab = (o16 ? 32768 : 0) + (f32slab ? 65536 : 0);   // one slab per epilogue warp, two groups of eight
-  int ns = (smem_max - 1024 - wbytes - slab - 4096 - 1024) / pl->stage_bytes;
+  int ns = (smem_max - 1024 - kNWBytes - 4096 - 1024) / pl->stage_bytes;
   if (ns > kNStages) ns = kNStages;
   if (ns < 2) return false;
   pl->nstage = ns;
-  int off = wbytes + ns * pl->stage_bytes;
-  pl->off_s16 = off; off += o16 ? 32768 : 0;
-  pl->off_s32 = off; off += f32slab ? 65536 : 0;
+  int off = kNWBytes + ns * pl->stage_bytes;
   pl->off_xch = off; off += 4096;
   pl->off_tail = off; off += 1024;
   pl->smem = (size_t)off + 1024;
   return true;
 }
 
-// true when the flavours of the RCAB loop (a bf16 output slab, or an fp32 read-modify-write slab, per epilogue warp)
-// fit next to a ring of >= 2 halo windows; the per-tile partial sums (SRES_EPI_POOL / SRES_EPI_DOT) are then laid
-// out per 126-row tile
-bool conv_n192_available(int H, int W) {
-  (void)H;
-  N192Plan pl;
-  return conv_n192_mode() >= 2 && n192_plan(&pl, W, false, true);
-}
-// this call's epilogue: bf16 output OR fp32 addend/output (both together would need 96 KB of slabs)
-bool conv_n192_fits(const sres_conv_args* a) {
-  N192Plan pl;
-  const bool o16 = a->out_bf16 != nullptr, f32 = a->resid_f32 != nullptr || a->out_f32 != nullptr;
-  const bool forced = (a->debug_flags & 128) != 0;   // tests / A-B runs: this kernel whatever the mode
-  const bool heavy = a->mask_bf16 != nullptr || (a->epi_flags & (SRES_EPI_POOL | SRES_EPI_DOT)) != 0;
-  if (!forced && (conv_n192_mode() <= 0 || (conv_n192_mode() == 1 && heavy))) return false;
-  return !(o16 && f32) && n192_plan(&pl, a->W, o16, f32);
-}
-
-template <typename... KArgs, typename... Args>
-static cudaError_t launch_n192(void (*kernel)(KArgs...), dim3 grid, size_t smem, cudaStream_t st, Args... args) {
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = grid; cfg.blockDim = dim3(kNThreads); cfg.dynamicSmemBytes = smem; cfg.stream = st;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
-  count_launch();
-  return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
-}
-
-// identity-mapped 64 -> 64 convolution with TMA-staged epilogue operands (the caller has checked the arguments)
-int launch_conv_n192(const sres_conv_args* a, cudaStream_t stream) {
-  ConvN192Params p{};
-  p.H = a->H; p.W = a->W; p.P = a->W + 1; p.R = a->H + 1;
-  const long long npos = (long long)a->B * p.R * p.P;
-  if (npos > 0x7fff0000LL) return set_error(SRES_ERR_UNSUPPORTED, "conv: batch too large for 32-bit rows");
-  p.npos = (int)npos;
-  p.n_tiles = (p.npos + kNTileOut - 1) / kNTileOut;
-  p.flags = a->epi_flags | ((a->debug_flags & 256) ? 0x100u : 0u); p.bias = a->bias; p.part = a->pool_part;
-  p.timeline = (long long*)a->debug_timeline;
-  p.use_o16 = a->out_bf16 != nullptr; p.use_msk = a->mask_bf16 != nullptr;
-  p.use_r32 = a->resid_f32 != nullptr; p.use_o32 = a->out_f32 != nullptr;
-  p.mask = (const uint16_t*)a->mask_bf16;
-  N192Plan pl;
-  if (!n192_plan(&pl, a->W, p.use_o16, p.use_r32 | p.use_o32))
-    return set_error(SRES_ERR_UNSUPPORTED, "conv: no room for the halo ring");
-  p.nstage = pl.nstage; p.stage_bytes = pl.stage_bytes; p.nbox = pl.nbox; p.box_rows = pl.box_rows; p.box_step = pl.box_step;
-  p.ky_step16 = pl.ky_step16;
-  p.off_s16 = pl.off_s16; p.off_s32 = pl.off_s32; p.off_xch = pl.off_xch; p.off_tail = pl.off_tail;
-
-  CUtensorMap tmA, tmW, tmO16a, tmO16b, tmMsk, tmR32, tmO32a, tmO32b;
-  int rc = make_tmap_rows64(&tmA, a->in_bf16, (uint64_t)p.npos, pl.box_rows);
-  if (rc) return rc;
-  rc = make_tmap_rows64(&tmW, a->wpack_bf16, 9 * 64, 192);
-  if (rc) return rc;
-  tmO16a = tmA; tmO16b = tmA; tmMsk = tmA; tmR32 = tmA; tmO32a = tmA; tmO32b = tmA;
-  if (p.use_msk && p.use_o16 && (rc = make_tmap_rows64_half(&tmMsk, a->mask_bf16, (uint64_t)p.npos, 32))) return rc;
-  if (p.use_o16 && ((rc = make_tmap_rows64_half(&tmO16a, a->out_bf16, (uint64_t)p.npos, 32)) ||
-                    (rc = make_tmap_rows64_half(&tmO16b, a->out_bf16, (uint64_t)p.npos, 31)))) return rc;
-  if (p.use_r32 && (rc = make_tmap_rows64_f32(&tmR32, a->resid_f32, (uint64_t)p.npos, 32))) return rc;
-  if (p.use_o32 && ((rc = make_tmap_rows64_f32(&tmO32a, a->out_f32, (uint64_t)p.npos, 32)) ||
-                    (rc = make_tmap_rows64_f32(&tmO32b, a->out_f32, (uint64_t)p.npos, 31)))) return rc;
-
-  const int sms = device_sm_count();
-  if (sms <= 0) return set_error(SRES_ERR_NO_DEVICE, "conv: no CUDA device");
-  const int grid = persistent_grid(p.n_tiles, sms);
-  int dev = 0;
-  cudaGetDevice(&dev);
-  int fl = (p.use_o16 ? kNO16 : 0) | (p.use_o32 ? kNO32 : 0) | (p.use_r32 ? kNR32 : 0) | (p.use_msk ? kNMsk : 0) |
-           ((a->epi_flags & SRES_EPI_RELU) ? kNRelu : 0) | ((a->epi_flags & SRES_EPI_POOL) ? kNPool : 0) |
-           ((a->epi_flags & SRES_EPI_DOT) ? kNDot : 0);
-  if (a->debug_flags & 16) fl = -1;  // force the runtime-flag instance
-  cudaError_t e = cudaSuccess;
-#define N192_CASE(FLV)                                                                                                   \
-  {                                                                                                                      \
-    static thread_local int attr_dev = -1;                                                                               \
-    if (attr_dev != dev) {                                                                                               \
-      e = cudaFuncSetAttribute(conv3x3_n192_kernel<64, FLV>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);           \
-      if (e != cudaSuccess) return set_cuda_error(e, "conv: smem attribute");                                           \
-      attr_dev = dev;                                                                                                    \
-    }                                                                                                                    \
-    e = launch_n192(conv3x3_n192_kernel<64, FLV>, dim3(grid), pl.smem, stream, tmA, tmW, tmO16a, tmO16b, tmMsk, tmR32,       \
-                    tmO32a, tmO32b, p);                                                                                  \
-  }
-  switch (fl) {
-    case kNRelu | kNO16: N192_CASE(kNRelu | kNO16) break;                                  // RCAB conv1
-    case kNPool | kNO16: N192_CASE(kNPool | kNO16) break;                                  // RCAB conv2
-    case kNMsk | kNO16: N192_CASE(kNMsk | kNO16) break;                                    // dgrad of conv2
-    case kNR32 | kNO32 | kNMsk | kNDot: N192_CASE(kNR32 | kNO32 | kNMsk | kNDot) break;    // dgrad of conv1
-    case kNO32 | kNMsk | kNDot: N192_CASE(kNO32 | kNMsk | kNDot) break;                    // dgrad of a group tail
-    case kNO16: N192_CASE(kNO16) break;
-    default: N192_CASE(-1) break;
-  }
-#undef N192_CASE
-  if (e != cudaSuccess) return set_cuda_error(e, "conv: launch");
-  e = cudaGetLastError();
-  if (e != cudaSuccess) return set_cuda_error(e, "conv: launch");
-  return SRES_OK;
-}
-
 // tail convolution 64 -> c_real <= 16 (weights packed with 16 rows per tap), planar fp32 output, any image width
 bool conv_n48_available(int H, int W) {
   (void)H;
-  N192Plan pl;
+  N48Plan pl;
   static const int on = [] { const char* e = getenv("SRES_CONV_N48"); return e ? atoi(e) : 1; }();
-  return on != 0 && n192_plan(&pl, W, false, false, 9 * 16 * 128);
+  return on != 0 && n48_plan(&pl, W);
 }
 
 int launch_conv_n48(const sres_conv_args* a, cudaStream_t stream) {
-  ConvN192Params p{};
+  ConvN48Params p{};
   p.H = a->H; p.W = a->W; p.P = a->W + 1; p.R = a->H + 1;
   const long long npos = (long long)a->B * p.R * p.P;
   if (npos > 0x7fff0000LL) return set_error(SRES_ERR_UNSUPPORTED, "conv: batch too large for 32-bit rows");
@@ -725,15 +323,15 @@ int launch_conv_n48(const sres_conv_args* a, cudaStream_t stream) {
   p.n_tiles = (p.npos + kNTileOut - 1) / kNTileOut;
   p.flags = a->epi_flags; p.bias = a->bias; p.out_nchw = a->out_nchw; p.c_real = a->c_real;
   p.timeline = (long long*)a->debug_timeline;
-  N192Plan pl;
-  if (!n192_plan(&pl, a->W, false, false, 9 * 16 * 128)) return set_error(SRES_ERR_UNSUPPORTED, "conv: no room for the halo ring");
+  N48Plan pl;
+  if (!n48_plan(&pl, a->W)) return set_error(SRES_ERR_UNSUPPORTED, "conv: no room for the halo ring");
   p.nstage = pl.nstage; p.stage_bytes = pl.stage_bytes; p.nbox = pl.nbox; p.box_rows = pl.box_rows; p.box_step = pl.box_step;
   p.ky_step16 = pl.ky_step16;
-  p.off_s16 = pl.off_s16; p.off_s32 = pl.off_s32; p.off_xch = pl.off_xch; p.off_tail = pl.off_tail;
+  p.off_xch = pl.off_xch; p.off_tail = pl.off_tail;
   CUtensorMap tmA, tmW;
   int rc = make_tmap_rows64(&tmA, a->in_bf16, (uint64_t)p.npos, pl.box_rows);
   if (rc) return rc;
-  rc = make_tmap_rows64(&tmW, a->wpack_bf16, 9 * 16, 48);
+  rc = make_tmap_rows64(&tmW, a->wpack_bf16, 9 * kNB, 3 * kNB);
   if (rc) return rc;
   const int sms = device_sm_count();
   if (sms <= 0) return set_error(SRES_ERR_NO_DEVICE, "conv: no CUDA device");
@@ -743,11 +341,11 @@ int launch_conv_n48(const sres_conv_args* a, cudaStream_t stream) {
   static thread_local int attr_dev = -1;
   cudaError_t e;
   if (attr_dev != dev) {
-    e = cudaFuncSetAttribute(conv3x3_n192_kernel<16, -1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
+    e = cudaFuncSetAttribute(conv3x3_n48_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
     if (e != cudaSuccess) return set_cuda_error(e, "conv: smem attribute");
     attr_dev = dev;
   }
-  e = launch_n192(conv3x3_n192_kernel<16, -1>, dim3(grid), pl.smem, stream, tmA, tmW, tmA, tmA, tmA, tmA, tmA, tmA, p);
+  e = launch_pdl(conv3x3_n48_kernel, dim3(grid), dim3(kNThreads), pl.smem, stream, tmA, tmW, p);
   if (e != cudaSuccess) return set_cuda_error(e, "conv: launch");
   e = cudaGetLastError();
   if (e != cudaSuccess) return set_cuda_error(e, "conv: launch");

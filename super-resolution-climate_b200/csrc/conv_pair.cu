@@ -46,10 +46,9 @@ struct PairParams {
   unsigned* ready;         // [n_tiles] phase-1 tiles stored (counts epilogue warps), self-cleaning
   unsigned* consumed;      // [n_tiles] phase-2 tiles that have seen ready[t]
   long long* timeline;     // bring-up only: per-CTA clock stamps [grid][16]
-  int fence_mode;          // proxy fence around the global hand-over (see fence_proxy_async_mode)
-  int dual_w;              // 0: one 72 KB weight region, swapped between the phases; 1: both weight sets resident from the
-                           // start; 2: two regions, and the one a phase does not need lends its space to the halo ring
-                           // (see pair_slot)
+  int strict;              // hand-over protocol: 1 acquire / release with proxy fences, 0 light (see fence_handover)
+  int dual_w;              // 0: one 72 KB weight region, swapped between the phases; 1: two regions, and the one a phase does
+                           // not need lends its space to the halo ring (see pair_slot)
 };
 
 constexpr int kPO16 = 1, kPO32 = 2, kPR32 = 4, kPMsk = 8, kPRelu = 16, kPPool = 32, kPDot = 64;
@@ -70,21 +69,16 @@ __device__ __forceinline__ unsigned ld_relaxed_gpu(const unsigned* p) {
   asm volatile("ld.relaxed.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
   return v;
 }
-// Hand-over protocol, SRES_PAIR_FENCE:
-//   8 (default) "light": the tile counter is bumped with red.relaxed.gpu after cp.async.bulk.wait_group has reported the slab
+// Hand-over protocol (SRES_PAIR_FENCE=1 selects the strict one):
+//   light (default): the tile counter is bumped with red.relaxed.gpu after cp.async.bulk.wait_group has reported the slab
 //       store COMPLETE, and read with ld.relaxed.gpu; no gpu-scope fences.  Both the slab (TMA store) and its consumer (TMA
 //       load) go straight to L2, the point of coherence at gpu scope, and the counter is bumped strictly after the completion
 //       of the store it covers, so a consumer that has seen the count cannot read older data.
-//   1 "strict": red.release.gpu / ld.acquire.gpu plus fence.proxy.async.global on both sides -- the by-the-book pattern; the
+//   strict: red.release.gpu / ld.acquire.gpu plus fence.proxy.async.global on both sides -- the by-the-book pattern; the
 //       per-tile MEMBAR.GPU of the release costs 0.7 ms per training step (27.87 vs 27.0-27.2 ms; unfused 28.20).
-//   0 / 2: strict without the proxy fence / with the full fence.proxy.async (bring-up).  +16 / +32 / +64 / +128: timing-only
-//   bring-up bits (no publication, no phase 2, relaxed bump, no completion wait).
 // Both protocols are bit-exact against two separate launches in tests/test_gpu_kernels.py::test_conv_pair_equals_two_launches.
-__device__ __forceinline__ void fence_proxy_async_mode(int mode) {
-  if (mode & 8) return;
-  mode &= 3;
-  if (mode == 1) asm volatile("fence.proxy.async.global;" ::: "memory");
-  else if (mode == 2) asm volatile("fence.proxy.async;" ::: "memory");
+__device__ __forceinline__ void fence_handover(int strict) {
+  if (strict) asm volatile("fence.proxy.async.global;" ::: "memory");
 }
 
 // per-warp epilogue state shared by both phases
@@ -231,9 +225,9 @@ __device__ __forceinline__ void epi_frag(const PairParams& p, EpiWarp& w, const 
 
 // Which halo-ring slot the i-th tile of a phase uses, and how often that slot has been used before (mbarrier parity).
 //
-// Plain modes (dual_w 0 / 1): slot = it % nstage over the whole launch.
+// One weight region (dual_w 0): slot = it % nstage over the whole launch.
 //
-// Lending mode (dual_w 2, the forward pair): with both 72 KB weight regions the ring has only two slots of its own (B0, B1) --
+// Lending mode (dual_w 1, the forward pair): with both 72 KB weight regions the ring has only two slots of its own (B0, B1) --
 // one tile of prefetch, and the MMA warp waited for TMA 10 % of the time.  But phase 1 does not need the phase-2 weights'
 // region and phase 2 does not need phase 1's, and a region holds two slots: phase 1 cycles through X0 X1 B0 B1 (X in the
 // phase-2 weight region) for all but its last two tiles, which use B0 B1 only; once X0 / X1 are released for the last time
@@ -242,8 +236,8 @@ __device__ __forceinline__ void epi_frag(const PairParams& p, EpiWarp& w, const 
 // producer has seen by then: it waited for B1's release by the last phase-1 tile).  Physical slots: 0 1 = B, 2 3 = X, 4 5 = Y.
 // (The sequence and the use counts below were checked on the host against a running count for every n1, n2 < 60.)
 struct SlotUse { int slot; uint32_t use; };
-__device__ __forceinline__ SlotUse pair_slot(int mode, int nstage, int phase, int i, int it, int n1) {
-  if (mode != 2) return SlotUse{it % nstage, uint32_t(it / nstage)};
+__device__ __forceinline__ SlotUse pair_slot(int lend, int nstage, int phase, int i, int it, int n1) {
+  if (!lend) return SlotUse{it % nstage, uint32_t(it / nstage)};
   if (phase == 0) {
     if (i >= n1 - 2) {
       const int sl = i - (n1 - 2);                                        // B0 (if n1 >= 2), then B1
@@ -273,7 +267,7 @@ conv3x3_pair_kernel(const __grid_constant__ CUtensorMap tmA1, const __grid_const
   const int stage_bytes = p.stage_rows * 128;
   // byte offset of a physical ring slot from smem_a (slots 2..5 exist in lending mode only and lie in the weight regions)
   auto slot_off = [&](int slot) -> int {
-    if (slot < 2 || p.dual_w != 2) return slot * stage_bytes;
+    if (slot < 2 || !p.dual_w) return slot * stage_bytes;
     return (slot < 4 ? kPWBytes + (slot - 2) * stage_bytes : (slot - 4) * stage_bytes) - 2 * kPWBytes;
   };
   uint8_t* tail = smem + p.off_tail;
@@ -290,8 +284,7 @@ conv3x3_pair_kernel(const __grid_constant__ CUtensorMap tmA1, const __grid_const
   const int lane = threadIdx.x & 31;
   const int G = gridDim.x;
   const int c1 = blockIdx.x;             // phase-1 tiles: c1 + kG
-  const int c2 = (p.fence_mode & 48) ? p.n_tiles : G - 1 - blockIdx.x;   // phase-2 tiles: c2 + kG (reversed ownership balances
-                                                                         // the ninth tiles); bring-up bits 16 / 32: no phase 2
+  const int c2 = G - 1 - blockIdx.x;     // phase-2 tiles: c2 + kG (reversed ownership balances the ninth tiles)
   const int n1 = c1 < p.n_tiles ? (p.n_tiles - 1 - c1) / G + 1 : 0;
   long long* tl = p.timeline ? p.timeline + (size_t)blockIdx.x * 16 : nullptr;
 #define PSTAMP(i)                              \
@@ -337,10 +330,6 @@ conv3x3_pair_kernel(const __grid_constant__ CUtensorMap tmA1, const __grid_const
     if (leader) {
       mbar_expect_tx(&bar_w[0], kPWBytes);
       for (int t = 0; t < 9; ++t) tma_load_2d(smem_w + t * 64 * 128, &tmW1, &bar_w[0], 0, t * 64);
-      if (p.dual_w == 1) {   // room for both weight sets: no swap between the phases
-        mbar_expect_tx(&bar_w[1], kPWBytes);
-        for (int t = 0; t < 9; ++t) tma_load_2d(smem_w2 + t * 64 * 128, &tmW2, &bar_w[1], 0, t * 64);
-      }
     }
     pdl_wait();
     int it = 0;
@@ -357,7 +346,7 @@ conv3x3_pair_kernel(const __grid_constant__ CUtensorMap tmA1, const __grid_const
       }
       __syncwarp();
     }
-    if (p.dual_w == 2) {
+    if (p.dual_w) {
       // lending mode: the phase-2 weights go where the lent slots X0 / X1 were, once phase 1 has released them for the last
       // time (X0 was used n1 / 4 times, X1 (n1 + 1) / 4 times) -- its last two tiles are still running on B0 / B1
       const int ux0 = n1 / 4, ux1 = (n1 + 1) / 4;
@@ -369,9 +358,8 @@ conv3x3_pair_kernel(const __grid_constant__ CUtensorMap tmA1, const __grid_const
         for (int t = 0; t < 9; ++t) tma_load_2d(smem_w2 + t * 64 * 128, &tmW2, &bar_w[1], 0, t * 64);
       }
       __syncwarp();
-    }
-    // phase-2 weights replace phase 1's once every phase-1 MMA of this CTA has retired (its last ring slot was released)
-    if (!p.dual_w) {
+    } else {
+      // phase-2 weights replace phase 1's once every phase-1 MMA of this CTA has retired (its last ring slot was released)
       if (n1 > 0) mbar_wait(&bar_empty[(n1 - 1) % p.nstage], ((n1 - 1) / p.nstage) & 1, 7);
       PSTAMP(2);   // every phase-1 MMA retired
       if (leader) {
@@ -397,7 +385,7 @@ conv3x3_pair_kernel(const __grid_constant__ CUtensorMap tmA1, const __grid_const
       if (prev_t >= 0) seen = atomicAdd(p.consumed + prev_t, 1u) + 1u;
       if (watch) {
         long long t0 = clock64();
-        while (((p.fence_mode & 8) ? ld_relaxed_gpu(p.ready + t) : ld_acquire_gpu(p.ready + t)) < 8u) {
+        while ((p.strict ? ld_acquire_gpu(p.ready + t) : ld_relaxed_gpu(p.ready + t)) < 8u) {
           __nanosleep(32);
           if (clock64() - t0 > 8000000000LL) { atomicExch(&g_sres_dev_error, 0xDEAD0008u); __threadfence_system(); __trap(); }
         }
@@ -407,7 +395,7 @@ conv3x3_pair_kernel(const __grid_constant__ CUtensorMap tmA1, const __grid_const
         if (seen == users) { p.ready[prev_t] = 0u; p.consumed[prev_t] = 0u; }
       }
       prev_t = watch ? t : -1;
-      if (watch) fence_proxy_async_mode(p.fence_mode);   // generic acquire -> async-proxy reads, on a lane without TMA ops in flight
+      if (watch) fence_handover(p.strict);   // generic acquire -> async-proxy reads, on a lane without TMA ops in flight
       __syncwarp();
       if (tl && lane == 4) tl[12] += clock64() - f0;   // producer: flag bookkeeping + spinning, phase 2
       // (the watchers' acquires and proxy fences are ordered before the elected lane's TMA load by the warp barrier above;
@@ -456,7 +444,7 @@ conv3x3_pair_kernel(const __grid_constant__ CUtensorMap tmA1, const __grid_const
         mbar_wait(&bar_full[slot], ph, 4);
         if (tl && lane == 0) { tl[14] += w1 - w0; tl[15] += clock64() - w1; }   // MMA warp waiting for the epilogue / for TMA
         tc_fence_after();
-        const uint32_t a_tile = p.dual_w == 2 ? sdesc_lo(smem_u32(smem_a) + slot_off(slot), 16) : a_lo0 + uint32_t(slot * stage_bytes) / 16;
+        const uint32_t a_tile = p.dual_w ? sdesc_lo(smem_u32(smem_a) + slot_off(slot), 16) : a_lo0 + uint32_t(slot * stage_bytes) / 16;
         const uint32_t d_tmem = tmem_base + uint32_t(acc * 64);
         if (leader) {
 #pragma unroll
@@ -505,11 +493,11 @@ conv3x3_pair_kernel(const __grid_constant__ CUtensorMap tmA1, const __grid_const
       const int row0 = tile * 128 + w.wq * 32;
       if (lane == 0) {
         bulk_wait_read<0>();                        // the slab may be overwritten
-        if (pend[0] >= 0 && !(p.fence_mode & 16)) {
-          if (!(p.fence_mode & 128)) bulk_wait_all<kLag - 1>();   // the oldest pending store has reached global memory ...
-          fence_proxy_async_mode(p.fence_mode);      // (async-proxy writes ordered before the generic release)
-          if (p.fence_mode & (64 | 8)) red_relaxed_gpu_add(p.ready + pend[0], 1u);
-          else red_release_gpu_add(p.ready + pend[0], 1u);   // ... publish it to the phase-2 producers of other CTAs
+        if (pend[0] >= 0) {
+          bulk_wait_all<kLag - 1>();                 // the oldest pending store has reached global memory ...
+          fence_handover(p.strict);                  // (async-proxy writes ordered before the generic release)
+          if (p.strict) red_release_gpu_add(p.ready + pend[0], 1u);
+          else red_relaxed_gpu_add(p.ready + pend[0], 1u);   // ... publish it to the phase-2 producers of other CTAs
         }
         if (in1) {
           mbar_expect_tx(w.bin, 2048u);
@@ -535,14 +523,14 @@ conv3x3_pair_kernel(const __grid_constant__ CUtensorMap tmA1, const __grid_const
       for (int i = 0; i + 1 < kLag; ++i) pend[i] = pend[i + 1];
       pend[kLag - 1] = tile;
     }
-    if (lane == 0 && !(p.fence_mode & 48)) {
+    if (lane == 0) {
       bulk_wait_all<0>();
-      fence_proxy_async_mode(p.fence_mode);
+      fence_handover(p.strict);
 #pragma unroll
       for (int i = 0; i < kLag; ++i)
         if (pend[i] >= 0) {
-          if (p.fence_mode & 8) red_relaxed_gpu_add(p.ready + pend[i], 1u);
-          else red_release_gpu_add(p.ready + pend[i], 1u);
+          if (p.strict) red_release_gpu_add(p.ready + pend[i], 1u);
+          else red_relaxed_gpu_add(p.ready + pend[i], 1u);
         }
     }
     __syncwarp();
@@ -599,21 +587,14 @@ static bool pair_plan(int W, bool fwd, PairParams* p, size_t* smem_bytes) {
   const int rows = 128 + 2 * (W + 2);
   const int box = (rows + 7) / 8 * 8 <= 256 ? (rows + 7) / 8 * 8 : 64;   // the whole window as one TMA box when it fits
   const int stage_rows = (rows + box - 1) / box * box;
-  static const int dual_env = [] { const char* e = getenv("SRES_PAIR_DUALW"); return e ? atoi(e) : 2; }();
-  int dual = 0;
-  int ns = (smem_max - 1024 - kPWBytes - 1024 - slab) / (stage_rows * 128);
-  if (dual_env) {   // two weight regions when that still leaves a ring of two slots or more
-    const int ns2 = (smem_max - 1024 - 2 * kPWBytes - 1024 - slab) / (stage_rows * 128);
-    if (ns2 >= 2) {
-      // 2 (default): the region a phase does not need lends two slots to the ring (pair_slot); 1: both weight sets resident
-      dual = (dual_env >= 2 && 2 * stage_rows * 128 <= kPWBytes) ? 2 : 1;
-      ns = dual == 2 ? 2 : ns2;
-    }
-  }
+  // Two weight regions when that still leaves a ring of two slots or more (stages of <= 260 rows for the forward pair).  The
+  // region a phase does not need then lends the ring two more slots (pair_slot): a 72 KB region holds two stages of <= 288 rows.
+  const bool dual = (smem_max - 1024 - 2 * kPWBytes - 1024 - slab) / (stage_rows * 128) >= 2;
+  int ns = dual ? 2 : (smem_max - 1024 - kPWBytes - 1024 - slab) / (stage_rows * 128);
   if (ns > kPStages) ns = kPStages;
   if (ns < 2) return false;
   if (p) {
-    p->box_rows = box; p->stage_rows = stage_rows; p->nstage = ns; p->dual_w = dual;
+    p->box_rows = box; p->stage_rows = stage_rows; p->nstage = ns; p->dual_w = dual ? 1 : 0;
     int off = kPWBytes * (dual ? 2 : 1) + ns * stage_rows * 128;   // (lending mode: 2 ring slots of its own, 4 more inside the weight regions)
     p->off_s16 = off; off += 16384;
     p->off_msk = off; off += fwd ? 0 : 16384;
@@ -670,8 +651,8 @@ extern "C" int sres_conv3x3_pair(const sres_conv_args* a1, const sres_conv_args*
   p.ready = (unsigned*)flags; p.consumed = p.ready + p.n_tiles;
   p.timeline = (long long*)a1->debug_timeline;
   {
-    static const int fm = [] { const char* e = getenv("SRES_PAIR_FENCE"); return e ? atoi(e) : 8; }();
-    p.fence_mode = fm;
+    static const int strict = [] { const char* e = getenv("SRES_PAIR_FENCE"); return e && atoi(e) == 1 ? 1 : 0; }();
+    p.strict = strict;
   }
   const int smem_max = 232448;
   size_t smem = 0;

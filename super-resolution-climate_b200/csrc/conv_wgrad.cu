@@ -8,14 +8,6 @@
 // (off_b - off_a) rows, expressed through the descriptor's leading-dimension byte offset.  9 taps
 // -> 5 accumulators of 128 x 64 fp32 in TMEM (the last one carries one junk half).
 //
-// N128 variant (opt-in, see wgrad_n128_enabled): the SAME stacking trick on the N side.  The MMA's K index k pairs X[k + alpha] with
-// dY[k + beta], which is the tap of offset alpha - beta; two dY windows (beta = -P and 0, second 64-column group
-// reached through the B descriptor's leading-dimension offset) times two X windows give FOUR taps per
-// M128 x N128 MMA:  {-P-1,-P} x {-P,0} -> taps (1,0)(1,1)(0,0)(0,1);  {-P+1,+1} x {-P,0} -> (1,2)(2,2)(0,2)(dup);
-// {P-1,P} x {0} -> (2,0)(2,1) (N = 64).  3 MMA groups instead of 5 per K step, 22 KB instead of 30 KB of operand
-// reads from shared memory -- the resource that bounds this kernel.  (dY's padding rows are zero, so the rows the
-// shifted window drops at the very end of the buffer contribute nothing.)
-//
 // Up to SRES_WGRAD_MAX_JOBS (8) independent weight gradients ("jobs": different layers of the backward pass) share one
 // launch: CTA c works on job c % njobs and reduces every nsplit-th 128-position chunk of it.  Fewer
 // split-K partials per job means less partial traffic and the per-launch cost (prologue, accumulator
@@ -48,14 +40,12 @@ struct WgradKParams {
   float* part_bias;    // [njobs][max_split][64]
 };
 
-template <bool N128>
 __global__ void __launch_bounds__(256, 1)
 conv3x3_wgrad_kernel(const __grid_constant__ WgMaps maps, const __grid_constant__ CUtensorMap tmPart, const WgradKParams p) {
   extern __shared__ uint8_t smem_raw[];
   // offset arithmetic (not an integer round trip) keeps the pointer in the shared address space: LDS/STS, not generic LD/ST
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
   const int stage_bytes = (p.dyrows + p.xrows) * 128;
-  const int dy_row0 = N128 ? p.P : 0;   // window row of PTL row q0 (the window starts P rows earlier for the beta = -P group)
   uint8_t* tail = smem + p.nstage * stage_bytes;
   uint64_t* bar_full = reinterpret_cast<uint64_t*>(tail);
   uint64_t* bar_empty = bar_full + kWgMaxStages;
@@ -104,7 +94,7 @@ conv3x3_wgrad_kernel(const __grid_constant__ WgMaps maps, const __grid_constant_
       const int q0 = c * 128;
       if (leader) {
         mbar_expect_tx(&bar_full[slot], stage_bytes);
-        for (int r = 0; r < p.dyrows; r += p.dybox) tma_load_2d(dst + r * 128, tmDY, &bar_full[slot], 0, q0 - dy_row0 + r);
+        for (int r = 0; r < p.dyrows; r += p.dybox) tma_load_2d(dst + r * 128, tmDY, &bar_full[slot], 0, q0 + r);
         uint8_t* xdst = dst + p.dyrows * 128;
         const int x0 = q0 - (p.P + 1);
         for (int r = 0; r < p.xrows; r += p.xbox) tma_load_2d(xdst + r * 128, tmX, &bar_full[slot], 0, x0 + r);
@@ -114,7 +104,6 @@ conv3x3_wgrad_kernel(const __grid_constant__ WgMaps maps, const __grid_constant_
   } else if (warp == 1) {
     const bool leader = elect_one();
     constexpr uint32_t idesc = make_idesc_bf16(128, 64, 1, 1);
-    constexpr uint32_t idesc128 = make_idesc_bf16(128, 128, 1, 1);
     constexpr uint32_t dhi = sdesc_hi_sw128(1024);
     const uint32_t s_addr = smem_u32(smem);
     uint32_t xoff[kWgAcc];
@@ -128,35 +117,14 @@ conv3x3_wgrad_kernel(const __grid_constant__ WgMaps maps, const __grid_constant_
       tc_fence_after();
       const uint32_t x_lo = sdesc_lo(s_addr + slot * stage_bytes + p.dyrows * 128, 0);
       if (leader) {
-        if constexpr (N128) {
-          // B: dY window rows [q0 - P, ...): column group 0 = beta -P (window row k), group 1 = beta 0 (row k + P)
-          const uint32_t dy2_lo = sdesc_lo(s_addr + slot * stage_bytes, uint32_t(p.P) * 128);
-          const uint32_t dy1_lo = sdesc_lo(s_addr + slot * stage_bytes + p.P * 128, 1024);
+        const uint32_t dy_lo = sdesc_lo(s_addr + slot * stage_bytes, 1024);
 #pragma unroll
-          for (int g = 0; g < 3; ++g) {
-            const uint32_t xa = x_lo + xoff[g];
-            const uint32_t dcol = tmem_base + g * 128;
+        for (int a = 0; a < kWgAcc; ++a) {
+          const uint32_t xa = x_lo + xoff[a];
 #pragma unroll
-            for (int kk = 0; kk < 8; ++kk) {
-              if (g < 2) {
-                if (kk == 0) umma_bf16_lohi_p(dcol, xa, dhi, dy2_lo, dhi, idesc128, it ? 1u : 0u);
-                else umma_bf16_lohi<true>(dcol, xa + kk * 128, dhi, dy2_lo + kk * 128, dhi, idesc128);
-              } else {
-                if (kk == 0) umma_bf16_lohi_p(dcol, xa, dhi, dy1_lo, dhi, idesc, it ? 1u : 0u);
-                else umma_bf16_lohi<true>(dcol, xa + kk * 128, dhi, dy1_lo + kk * 128, dhi, idesc);
-              }
-            }
-          }
-        } else {
-          const uint32_t dy_lo = sdesc_lo(s_addr + slot * stage_bytes, 1024);
-#pragma unroll
-          for (int a = 0; a < kWgAcc; ++a) {
-            const uint32_t xa = x_lo + xoff[a];
-#pragma unroll
-            for (int kk = 0; kk < 8; ++kk) {
-              if (kk == 0) umma_bf16_lohi_p(tmem_base + a * 64, xa, dhi, dy_lo, dhi, idesc, it ? 1u : 0u);
-              else umma_bf16_lohi<true>(tmem_base + a * 64, xa + kk * 128, dhi, dy_lo + kk * 128, dhi, idesc);
-            }
+          for (int kk = 0; kk < 8; ++kk) {
+            if (kk == 0) umma_bf16_lohi_p(tmem_base + a * 64, xa, dhi, dy_lo, dhi, idesc, it ? 1u : 0u);
+            else umma_bf16_lohi<true>(tmem_base + a * 64, xa + kk * 128, dhi, dy_lo + kk * 128, dhi, idesc);
           }
         }
         umma_commit(&bar_empty[slot]);
@@ -180,7 +148,7 @@ conv3x3_wgrad_kernel(const __grid_constant__ WgMaps maps, const __grid_constant_
       const uint8_t* dy = smem + slot * stage_bytes;
 #pragma unroll
       for (int r = 0; r < 32; r += 4) {
-        const int row = dy_row0 + wq * 32 + r + rg;
+        const int row = wq * 32 + r + rg;
         const uint4 v = *reinterpret_cast<const uint4*>(dy + row * 128 + ((ck ^ (row & 7)) << 4));
         acc[0] += bf16_lo(v.x); acc[1] += bf16_hi(v.x); acc[2] += bf16_lo(v.y); acc[3] += bf16_hi(v.y);
         acc[4] += bf16_lo(v.z); acc[5] += bf16_hi(v.z); acc[6] += bf16_lo(v.w); acc[7] += bf16_hi(v.w);
@@ -253,7 +221,7 @@ struct WgReduceJob {
 };
 struct WgReduceJobs {
   WgReduceJob j[kWgMaxJobs];
-  signed char tap[2 * kWgAcc];  // tap held by (64-column block a, row half h) of the partial, -1 = junk / duplicate
+  signed char tap[2 * kWgAcc];  // tap held by (64-column block a, row half h) of the partial, -1 = junk
 };
 
 // Every thread sums FOUR consecutive output features of one (accumulator block, row) over the split-K partials with 16-byte
@@ -317,14 +285,6 @@ wgrad_reduce_kernel(const float* __restrict__ part, const float* __restrict__ pa
   }
 }
 
-// Opt-in (SRES_WGRAD_N128=1, read per call so tests can flip it): measured on B200 the four-taps-per-MMA scheme is
-// NOT faster than the plain one (33.6 vs 31.1 us per job alone, 29.1 vs 29.0 ms per step) although it reads 27 % fewer
-// operand bytes -- the N = 128 MN-major B operand does not stream out of shared memory as well as two N = 64 ones.
-static bool wgrad_n128_enabled() {
-  const char* e = getenv("SRES_WGRAD_N128");
-  return e && atoi(e) != 0;
-}
-
 static int wg_grid() {
   int sms = device_sm_count();
   return sms > 0 ? sms : 148;
@@ -362,18 +322,13 @@ extern "C" int sres_conv3x3_wgrad_batch(const sres_wgrad_job* jobs, int njobs, i
   p.n_chunks = (p.npos + 127) / 128;
   // X window: 128 positions + the halo of 2(P+1)+1 rows.  When it fits one TMA box (<= 256 rows) it is loaded exactly
   // (rounded to the 8-row swizzle period) in ONE copy; wider windows go in 64-row boxes.  The kernel's slope per job is set
-  // by this feed, not by its MMAs (see wgrad_n128_enabled), so the 24 rows the 64-row rounding added at 48 x 48 were 6 % of it.
+  // by this feed, not by its MMAs (DESIGN.md section 3.2), so the 24 rows the 64-row rounding added at 48 x 48 were 6 % of it.
   const int xneed = 128 + 2 * (p.P + 1) + 1;
-  bool n128 = wgrad_n128_enabled();
-  const bool exact = !n128 && (xneed + 7) / 8 * 8 <= 256 && !getenv("SRES_WGRAD_BOX64");
+  const bool exact = (xneed + 7) / 8 * 8 <= 256;
   p.xrows = exact ? (xneed + 7) / 8 * 8 : (xneed + 63) / 64 * 64;
   p.xbox = exact ? p.xrows : 64;
   p.dybox = exact ? 128 : 64;
-  p.dyrows = n128 ? (128 + p.P + 63) / 64 * 64 : 128;
-  if (n128 && ((232448 - 1024 - 2048) / ((p.dyrows + p.xrows) * 128) < 1 || p.P * 128 >= (1 << 18))) {
-    n128 = false;  // very wide images: the plain scheme needs less shared memory
-    p.dyrows = 128;
-  }
+  p.dyrows = 128;
   const int stage_bytes = (p.dyrows + p.xrows) * 128;
   int nstage = (232448 - 1024 - 2048) / stage_bytes;
   if (nstage > kWgMaxStages) nstage = kWgMaxStages;
@@ -381,23 +336,14 @@ extern "C" int sres_conv3x3_wgrad_batch(const sres_wgrad_job* jobs, int njobs, i
   if (nstage * stage_bytes < 32768) return set_error(SRES_ERR_UNSUPPORTED, "wgrad: operand ring smaller than the drain slabs");
   p.nstage = nstage;
   WgReduceJobs rj;
-  if (n128) {
-    // X-window row offsets (window starts at q0 - P - 1) and second-half distances of the three MMA groups
-    const int offs[3] = {0, 2, 2 * p.P}, lbos[3] = {128, p.P * 128, 128};
-    for (int g = 0; g < kWgAcc; ++g) { p.off_a[g] = g < 3 ? offs[g] : 0; p.lbo[g] = g < 3 ? lbos[g] : 128; }
-    // partial column block a = (group, dY shift): tap offset = alpha - beta (see the header comment)
-    const signed char taps[2 * kWgAcc] = {3, 4, 0, 1, 5, 8, 2, -1, 6, 7};
-    for (int i = 0; i < 2 * kWgAcc; ++i) rj.tap[i] = taps[i];
-  } else {
-    for (int a = 0; a < kWgAcc; ++a) {
-      const int ta = 2 * a, tb = (2 * a + 1 <= 8) ? 2 * a + 1 : -1;
-      const int offa = (ta / 3) * p.P + (ta % 3);
-      p.off_a[a] = offa;
-      p.lbo[a] = tb >= 0 ? (((tb / 3) * p.P + (tb % 3)) - offa) * 128 : 128;
-      if (p.lbo[a] >= (1 << 18)) return set_error(SRES_ERR_UNSUPPORTED, "wgrad: tap distance exceeds descriptor range");
-      rj.tap[2 * a] = (signed char)ta;
-      rj.tap[2 * a + 1] = (signed char)tb;
-    }
+  for (int a = 0; a < kWgAcc; ++a) {
+    const int ta = 2 * a, tb = (2 * a + 1 <= 8) ? 2 * a + 1 : -1;
+    const int offa = (ta / 3) * p.P + (ta % 3);
+    p.off_a[a] = offa;
+    p.lbo[a] = tb >= 0 ? (((tb / 3) * p.P + (tb % 3)) - offa) * 128 : 128;
+    if (p.lbo[a] >= (1 << 18)) return set_error(SRES_ERR_UNSUPPORTED, "wgrad: tap distance exceeds descriptor range");
+    rj.tap[2 * a] = (signed char)ta;
+    rj.tap[2 * a + 1] = (signed char)tb;
   }
   const int sms = device_sm_count();
   if (sms <= 0) return set_error(SRES_ERR_NO_DEVICE, "wgrad: no CUDA device");
@@ -428,11 +374,9 @@ extern "C" int sres_conv3x3_wgrad_batch(const sres_wgrad_job* jobs, int njobs, i
   int rc = make_tmap_rows64_f32(&tmPart, part, (uint64_t)njobs * p.max_split * kWgAcc * 128, 32);
   if (rc) return rc;
   const size_t smem = (size_t)nstage * stage_bytes + 1024 + 2048;
-  cudaError_t e = cudaFuncSetAttribute(n128 ? conv3x3_wgrad_kernel<true> : conv3x3_wgrad_kernel<false>,
-                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  cudaError_t e = cudaFuncSetAttribute(conv3x3_wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return set_cuda_error(e, "wgrad: smem attribute");
-  e = n128 ? launch_pdl(conv3x3_wgrad_kernel<true>, dim3(grid), dim3(256), smem, stream, maps, tmPart, p)
-           : launch_pdl(conv3x3_wgrad_kernel<false>, dim3(grid), dim3(256), smem, stream, maps, tmPart, p);
+  e = launch_pdl(conv3x3_wgrad_kernel, dim3(grid), dim3(256), smem, stream, maps, tmPart, p);
   if (e != cudaSuccess) return set_cuda_error(e, "wgrad: launch");
   const int total = kWgPartFloats / 4 + 16;   // groups of four floats + 16 bias groups
   e = launch_pdl(wgrad_reduce_kernel, dim3((total + 255) / 256, njobs), dim3(256), 0, stream, (const float*)part,

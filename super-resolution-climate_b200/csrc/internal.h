@@ -13,7 +13,7 @@ int set_cuda_error(cudaError_t e, const char* where);
 
 // cached SM count of the current device (<=0 when there is none)
 int device_sm_count();
-// fewest CTAs of a persistent kernel that still finish n_tiles equal tiles in the minimal number of waves
+// grid of a persistent kernel that walks n_tiles equal tiles: one CTA per SM, or per tile when there are fewer
 int persistent_grid(int n_tiles, int sms);
 
 // 2-D TMA descriptor over a row-major [nrows][64] bf16 matrix (128-byte rows), box = 64 x box_rows,
@@ -61,11 +61,7 @@ cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t s
   return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
 }
 
-// N = 192 convolution kernel (conv_n192.cu): identity-mapped 64 -> 64 convolutions with TMA-staged epilogue operands
-bool conv_n192_available(int H, int W);
-bool conv_n192_fits(const sres_conv_args* a);
-int launch_conv_n192(const sres_conv_args* a, cudaStream_t stream);
-// narrow variant (N = 48): tail convolution 64 -> c_real <= 16 with planar fp32 output, any image width
+// three-taps-per-MMA tail convolution (conv_n192.cu, N = 48): 64 -> c_real <= 16 with planar fp32 output, any image width
 bool conv_n48_available(int H, int W);
 int launch_conv_n48(const sres_conv_args* a, cudaStream_t stream);
 

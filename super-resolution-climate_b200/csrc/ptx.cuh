@@ -304,80 +304,6 @@ __device__ __forceinline__ void tmem_ld_wait() {
 }
 
 // ---------------------------------------------------------------------------
-// CTA pairs (cta_group::2): two CTAs of a 2-cluster run one UMMA of M = 256; each holds its own 128 rows of A
-// and half of B's N rows in shared memory and its own 128 accumulator lanes in TMEM.  Only rank 0 issues MMAs;
-// its shared-memory "full" barriers collect the TMA bytes of BOTH CTAs, and its commits are multicast.
-// ---------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-// shared::cluster address of the same shared-memory location in CTA `rank` of the cluster
-__device__ __forceinline__ uint32_t mapa_u32(uint32_t saddr, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(saddr), "r"(rank));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-// TMA load into this CTA's shared memory whose bytes complete on a barrier of the pair's leader CTA
-__device__ __forceinline__ void tma_load_2d_pair(void* smem_dst, const CUtensorMap* m, uint32_t leader_bar, int32_t c0,
-                                                 int32_t c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes"
-      " [%0], [%1, {%3, %4}], [%2];"
-      :
-      : "r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(leader_bar), "r"(c0), "r"(c1)
-      : "memory");
-}
-__device__ __forceinline__ void tmem_alloc2(uint32_t* smem_holder, uint32_t ncols) {
-  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_holder)), "r"(ncols)
-               : "memory");
-}
-__device__ __forceinline__ void tmem_relinquish2() {
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc2(uint32_t taddr, uint32_t ncols) {
-  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-}
-template <bool kAccumulate>
-__device__ __forceinline__ void umma2_bf16_lohi(uint32_t tmem_d, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo,
-                                                uint32_t b_hi, uint32_t idesc) {
-  if constexpr (kAccumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\t"
-        "mov.b64 da, {%1, %2};\n\tmov.b64 db, {%3, %4};\n\t"
-        "setp.eq.b32 p, 0, 0;\n\t"
-        "tcgen05.mma.cta_group::2.kind::f16 [%0], da, db, %5, p;\n\t}\n"
-        :
-        : "r"(tmem_d), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc)
-        : "memory");
-  } else {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\t"
-        "mov.b64 da, {%1, %2};\n\tmov.b64 db, {%3, %4};\n\t"
-        "setp.ne.b32 p, 0, 0;\n\t"
-        "tcgen05.mma.cta_group::2.kind::f16 [%0], da, db, %5, p;\n\t}\n"
-        :
-        : "r"(tmem_d), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc)
-        : "memory");
-  }
-}
-// arrive on the barrier at this shared-memory offset in BOTH CTAs of the pair once the issued MMAs retire
-__device__ __forceinline__ void umma_commit2(uint64_t* bar) {
-  asm volatile(
-      "{\n\t.reg .b16 m;\n\tmov.b16 m, 3;\n\t"
-      "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], m;\n\t}\n" ::"r"(
-          smem_u32(bar))
-      : "memory");
-}
-
-// ---------------------------------------------------------------------------
 // small helpers
 // ---------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {

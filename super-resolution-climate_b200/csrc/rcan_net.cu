@@ -36,12 +36,6 @@ static int ring_len() {   // buffers actually rotated through (<= kRing): fewer 
   }();
   return v;
 }
-// SRES_JOIN_PER_SEG=1: the round-1 behaviour (join the side stream after every backward segment, squeeze-excite parameter
-// gradients on the main stream) for A/B runs.
-static bool join_per_segment() {
-  static const bool v = [] { const char* e = getenv("SRES_JOIN_PER_SEG"); return e && atoi(e) != 0; }();
-  return v;
-}
 static int wgrad_batch_jobs() {
   static const int v = [] {
     const char* e = getenv("SRES_WGRAD_BATCH");
@@ -496,7 +490,7 @@ struct WgQueue {
   // parameter gradients of a finished group) behind the weight-gradient batches on the side stream.
   template <class F>
   int run_side(F fn) {
-    if (!ax || join_per_segment()) return fn(st);
+    if (!ax) return fn(st);
     const int i = ax->next;
     ax->next = (i + 1) % AsyncCtx::kEvents;
     RC(wait_slot(i));
@@ -590,7 +584,6 @@ static int backward(const Net& n, const float* P, const float* x, const float* d
       RC(wq.before_write(gb16));
       RC(conv64(dres16, WD(n.cidx_bt()), nullptr, B, H, W, st, ga, gb16));
       RC(wq.flush());
-      if (join_per_segment()) RC(wq.join_all());
     } else if (seg <= G && n.edsr) {
       // ResBlocks R-1..0.  ga = fp32 gradient trunk; its bf16 copy for block r lives in gb16 (r = R-1, written by
       // segment 0) or dt2[r % ring_len()] (written by block r+1's conv1 input-gradient).
@@ -662,7 +655,6 @@ static int backward(const Net& n, const float* P, const float* x, const float* d
       // the next group's input-gradient chain.
       const long long first = n.off_rcab(g, 0) + 2 * (kConvW + 64);
       PROF("ca_param_grads");
-      if (join_per_segment()) RC(wq.join_all());
       RC(wq.run_side([&](void* s) {
         return sres_ca_param_grads(P + first, Gr + first, n.rcab_sz, R, (const float*)(ws + n.o_mean) + (size_t)g * R * B * 64,
                                    (const float*)(ws + n.o_ds) + (size_t)g * R * B * 64, B, n.hid, accumulate,

@@ -43,7 +43,7 @@ def test_geometry_helpers(lib):
     lib.sres_ptl_rows.restype = C.c_int64
     assert lib.sres_ptl_rows(64, 48, 48) == 64 * 49 * 49
     tr = lib.sres_conv_tile_rows(48, 48)
-    assert tr in (126, 128)   # 126: three-taps-per-MMA kernel (tiles overlap by two rows)
+    assert tr == 128
     assert lib.sres_conv_mtiles(64, 48, 48) == (64 * 49 * 49 + tr - 1) // tr
 
 

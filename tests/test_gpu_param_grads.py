@@ -273,21 +273,6 @@ def test_wgrad_batches_back_to_back(env):
             check_job(f"batch {k} {geom} job {i}", j, wg_bound(env, *geom, len(jobs)))
 
 
-def test_wgrad_batch_n128_tap_table(env, monkeypatch):
-    """The opt-in four-taps-per-MMA scheme (SRES_WGRAD_N128=1, read per call) scatters through its own tap table: 8 plain
-    jobs and the x2 PixelShuffle batch at 48 x 48 against fp64 (same bounds as the default scheme).
-    Measured on a B200: x2 PixelShuffle rel-L2 dw 4.3e-6, db 1.2e-7."""
-    monkeypatch.setenv("SRES_WGRAD_N128", "1")
-    B, H, W = 64, 48, 48
-    ws = workspace(env)
-    jobs = plain_jobs(env, B, H, W, 8, seed=4)
-    run_batch(env, jobs, B, H, W, ws)
-    print(f"\n  wgrad batch {(B, H, W)} x 8 jobs, SRES_WGRAD_N128=1")
-    for i, j in enumerate(jobs):
-        check_job(f"job {i}", j, wg_bound(env, B, H, W, 8))
-    _x2_shuffle(env, B, H, W, "SRES_WGRAD_N128=1")
-
-
 # ---------------------------------------------------------------------------------------------------------------------
 # B. head and tail weight gradients (CUDA cores, fp32)
 # ---------------------------------------------------------------------------------------------------------------------

@@ -6,7 +6,7 @@ sys.path.insert(0, os.path.join(ROOT, "super-resolution-climate_b200"))
 from sres_b200 import _lib as L
 lib = L.lib(); dev = torch.device("cuda:0")
 B, H, W = 64, 48, 48
-rows = lib.sres_ptl_rows(B, H, W); nt = (rows + 125) // 126
+rows = lib.sres_ptl_rows(B, H, W); nt = lib.sres_conv_mtiles(B, H, W)
 xin = (torch.randn(rows, 64, device=dev)).bfloat16()
 msk = (torch.randn(rows, 64, device=dev)).bfloat16()
 o16 = torch.zeros(rows, 64, device=dev, dtype=torch.bfloat16)
@@ -27,12 +27,7 @@ base = {
   "dgrad1    (fp32 rmw + dot)      ": dict(out_f32=f32.data_ptr(), resid_f32=f32.data_ptr(), mask_bf16=msk.data_ptr(), epi_flags=4, pool_part=pool.data_ptr()),
   "bf16 out only                   ": dict(bias=bias.data_ptr(), out_bf16=o16.data_ptr()),
 }
-flav = {}
-for k, v in base.items():
-    flav[k + " N192 (forced)         "] = mk(debug_flags=128, **v)
-    flav[k + " N192 runtime flags    "] = mk(debug_flags=128 | 16, **v)
-    flav[k + " tap-per-MMA specialised"] = mk(debug_flags=64, **v)
-    flav[k + " N192 rt flags, NO shuffles (timing only)"] = mk(debug_flags=128 | 16 | 256, **v)
+flav = {k + " specialised": mk(**v) for k, v in base.items()}
 st_ = L.cur_stream()
 for name, a in flav.items():
     for _ in range(5): L.check(lib.sres_conv3x3_igemm(C.byref(a), st_), name)

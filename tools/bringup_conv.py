@@ -169,7 +169,7 @@ def main():
                  7: "last accumulator ready", 8: "last store issued", 9: "stores drained", 12: "exit"}
         print("per-CTA timeline, cycles since CTA entry (min / median / max over CTAs):")
         for i in (1, 3, 4, 6, 5, 7, 8, 9, 12):
-            sel = t[:, i] != 0   # the CTA-pair kernel stamps MMA events on leader CTAs only
+            sel = t[:, i] != 0   # CTAs without a tile stamp nothing
             d = (t[:, i] - t[:, 0])[sel]
             print(f"  {names[i]:26s} {d.min():9.0f} {d.median():9.0f} {d.max():9.0f}")
         for i, nm in ((13, "epilogue warp idle (waits for MMA)"), (14, "MMA warp waits for epilogue"), (15, "MMA warp waits for TMA")):
