@@ -345,6 +345,26 @@ SRES_API int sres_tiles_lnorm(const float* in, int nplanes, int T, int flip_inde
 SRES_API int sres_tiles_stitch(const float* tiles, int C, int ivar, int t, int gy, int gx, const int32_t* cell_to_tile,
                                const float* mean, const float* std_, float* out, void* stream);
 
+/* Rectangular tiles (task.tile_size {x, y} with x != y; sres/data/tiles.py:110-127 and raw.py:216-233 treat the two
+ * axes separately).  Same contracts as the square entry points above, which are these with Th = Tw = T.        */
+/* candidate tile (c, ty, tx) starts at (y0 + ty*Th, x0 + tx*Tw); the grid must fit the region on each axis      */
+SRES_API int sres_tiles_finite_flags_hw(const float* region, int C, int Y, int X, int y0, int x0, int Th, int Tw, int gy,
+                                        int gx, int32_t* flags, void* stream);
+/* out[slot] (Th x Tw) = candidate tile src_tile[slot]; slot = n*C + c of the (N,C,Th,Tw) result                */
+SRES_API int sres_tiles_gather_hw(const float* region, int C, int Y, int X, int y0, int x0, int Th, int Tw, int gy, int gx,
+                                  const int32_t* src_tile, int nslots, float* out, void* stream);
+/* in: nplanes Th x Tw planes.  Flips 0-3 write Th x Tw planes, out[r][c] = in[fy(r)][fx(c)]; flips 4-7 write
+ * Tw x Th planes, out[r][c] = in[fy(c)][fx(r)] (the reference flips x, then y, then swapaxes(-1,-2);
+ * source/batch.py:37-49), with fy(j) = (flip & 2) ? Th-1-j : j and fx(i) = (flip & 1) ? Tw-1-i : i.
+ * Statistics as sres_tiles_lnorm.  In-place only with flip_index 0.                                           */
+SRES_API int sres_tiles_lnorm_hw(const float* in, int nplanes, int Th, int Tw, int flip_index, float* out, float* mean,
+                                 float* std_, void* stream);
+/* tiles (N,C,th,tw) -> image (gy*th, gx*tw) of variable ivar; tile cell_to_tile[cy*gx+cx] lands at rows
+ * [cy*th, (cy+1)*th) and columns [cx*tw, (cx+1)*tw) (dual_trainer.py:449-480), NaN when < 0                   */
+SRES_API int sres_tiles_stitch_hw(const float* tiles, int C, int ivar, int th, int tw, int gy, int gx,
+                                  const int32_t* cell_to_tile, const float* mean, const float* std_, float* out,
+                                  void* stream);
+
 /* ------------------------------------------------------------------------------------------ */
 /* Raw LLC4320 fields -> region of interest (the reference's file reader, SURVEY.md 8f rank 4)  */
 /*   sres/base/source/swot/raw.py:133-145 load_file: big-endian f4 ocean-only ("shrunk") file,  */

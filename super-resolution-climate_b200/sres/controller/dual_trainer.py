@@ -322,13 +322,14 @@ class ModelTrainer(object):
             for r in range(self.world):
                 rlo, rhi = shard_range(len(ctiles), r, self.world)
                 counts.append(sum(min(c["end"], ntiles) - c["start"] for c in ctiles[rlo:rhi]))
-            nch, hr = len(self.target_variables), int(timeslice.shape[2])
-            scale = int(np.prod(cfg().model.downscale_factors)) * int(cfg().task.get("data_downsample", 1.0))
+            nch, hr_y, hr_x = len(self.target_variables), int(timeslice.shape[2]), int(timeslice.shape[3])
+            dsample = int(cfg().task.get("data_downsample", 1.0))
+            scale = int(np.prod(cfg().model.downscale_factors)) * dsample
             merged = {}
             for k in ("input", "target", "interpolated", "model"):
-                side = hr // scale if k == "input" else hr // int(cfg().task.get("data_downsample", 1.0))
+                f = scale if k == "input" else dsample
                 local = torch.cat([denorm(bd[k], a).float() for bd, a in zip(batches, stats)], dim=0) if batches else None
-                merged[k] = gather_rows(local, counts, (nch, side, side), self.device)
+                merged[k] = gather_rows(local, counts, (nch, hr_y // f, hr_x // f), self.device)
             batches, stats = [merged], None
             dist.all_reduce(lsum)
         lsum = lsum.cpu()
@@ -365,15 +366,15 @@ class ModelTrainer(object):
         pending: Dict[str, Tensor] = {}
         for image_type in batches[0].keys():
             tiles = torch.cat([torch.as_tensor(b[image_type], device=self.device).detach().float() for b in batches], dim=0).contiguous()
-            n, Cc, t, _ = tiles.shape
+            n, Cc, th, tw = tiles.shape
             cell = np.full(gy * gx, -1, dtype=np.int32)
             cell[tile_ids[:n].astype(np.int64)] = np.arange(n, dtype=np.int32)   # (ids are unique: later == earlier)
             cell_d = torch.from_numpy(cell).to(self.device)
-            img = torch.empty(gy * t, gx * t, dtype=torch.float32, device=self.device)
+            img = torch.empty(gy * th, gx * tw, dtype=torch.float32, device=self.device)
             if mean is not None and mean.numel() != n * Cc:
                 raise ValueError(f"assemble_images: {mean.numel()} normalisation entries for {n} tiles x {Cc} channels")
-            L.check(lib.sres_tiles_stitch(L.ptr(tiles), Cc, ivar, t, gy, gx, L.ptr(cell_d), L.ptr(mean), L.ptr(std), L.ptr(img),
-                                          L.cur_stream()), "sres_tiles_stitch")
+            L.check(lib.sres_tiles_stitch_hw(L.ptr(tiles), Cc, ivar, th, tw, gy, gx, L.ptr(cell_d), L.ptr(mean), L.ptr(std),
+                                             L.ptr(img), L.cur_stream()), "sres_tiles_stitch_hw")
             dev_img = img.double() if (cell < 0).any() else img
             host = torch.empty(dev_img.shape, dtype=dev_img.dtype, pin_memory=True)
             host.copy_(dev_img, non_blocking=True)
@@ -435,6 +436,12 @@ class ModelTrainer(object):
                                 res[k].append(v.detach())
                     if self.time_index >= 0:
                         break
+        shapes = sorted({tuple(v.shape[2:]) for v in res["target"]})
+        if len(shapes) > 1:
+            # the reference's np.concatenate fails on the same batches
+            raise ValueError(f"evaluate(keep_results=True): the batches come in tile shapes {shapes} (rectangular tiles with "
+                             "task.xyflip transpose some of them) and cannot be concatenated; use keep_results=False or "
+                             "turn xyflip off")
         results = {k: (torch.cat(v).cpu().numpy() if v else None) for k, v in res.items()}
         losses = dict(model=float(np.mean(ml)) if ml else float("nan"), interpolated=float(np.mean(il)) if il else float("nan"))
         if tset == TSet.Validation and ml and self.time_index < 0:

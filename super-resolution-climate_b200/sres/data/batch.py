@@ -65,7 +65,7 @@ def synthetic_region(C_: int, Y: int, X: int, seed: int, nan_fraction: float = 0
 
 
 def source_table(flags: np.ndarray, C_: int, ncand: int, order: str):
-    """Which candidate tile feeds slot (n, c) of the (N,C,T,T) result, and the tile-id coordinate.
+    """Which candidate tile feeds slot (n, c) of the (N,C,Th,Tw) result, and the tile-id coordinate.
 
     order == 'reference': bit-exact restatement of raw.py:225-233 -- survivors of the channel-major
     flat list are re-chunked C at a time (so for C > 1 a slot pairs consecutive flat tiles, SURVEY.md 8a)
@@ -131,9 +131,7 @@ class BatchDataset(object):
         """(C,Y,X) device region -> TileArray(tiles, channels, y, x), raw.py:216-233 on the GPU."""
         C_, Y, X = region.shape
         ts = self.tile_grid.get_full_tile_size()
-        if ts["x"] != ts["y"]:
-            raise NotImplementedError("square tiles only")
-        T = ts["y"]
+        Th, Tw = ts["y"], ts["x"]
         gs = self.tile_grid.get_grid_shape(image_shape=dict(c=C_, y=Y, x=X))
         roi = self.tile_grid.get_active_region(image_shape=dict(c=C_, y=Y, x=X))
         gy, gx, y0, x0 = gs["y"], gs["x"], roi["y"][0], roi["x"][0]
@@ -141,15 +139,15 @@ class BatchDataset(object):
         dev = region.device
         flags = torch.empty(C_ * ncand, dtype=torch.int32, device=dev)
         st = L.cur_stream()
-        L.check(self.lib.sres_tiles_finite_flags(L.ptr(region), C_, Y, X, y0, x0, T, gy, gx, L.ptr(flags), st),
-                "sres_tiles_finite_flags")
+        L.check(self.lib.sres_tiles_finite_flags_hw(L.ptr(region), C_, Y, X, y0, x0, Th, Tw, gy, gx, L.ptr(flags), st),
+                "sres_tiles_finite_flags_hw")
         src, ids = source_table(flags.cpu().numpy(), C_, ncand, self.task.get("tile_order", "reference"))
         n = src.size // C_
-        out = torch.empty(n, C_, T, T, dtype=torch.float32, device=dev)
+        out = torch.empty(n, C_, Th, Tw, dtype=torch.float32, device=dev)
         if n > 0:
             src_d = torch.from_numpy(src).to(dev)
-            L.check(self.lib.sres_tiles_gather(L.ptr(region), C_, Y, X, y0, x0, T, gy, gx, L.ptr(src_d), n * C_, L.ptr(out), st),
-                    "sres_tiles_gather")
+            L.check(self.lib.sres_tiles_gather_hw(L.ptr(region), C_, Y, X, y0, x0, Th, Tw, gy, gx, L.ptr(src_d), n * C_,
+                                                  L.ptr(out), st), "sres_tiles_gather_hw")
         return TileArray(out, ["tiles", "channels", "y", "x"], coords=dict(tiles=ids, channels=self.varnames),
                          attrs=dict(grid_shape=dict(gs)))
 
@@ -198,13 +196,14 @@ class BatchDataset(object):
         ntype = self.task.norm
         if ntype != "lnorm":
             raise NotImplementedError(f"sres (B200 build): norm '{ntype}' has no CUDA kernel (lnorm only)")
-        B, C_, T, _ = raw.shape
+        B, C_, Th, Tw = raw.shape
         raw = raw.contiguous()
-        out = torch.empty_like(raw)
+        # flips 4-7 end with swapaxes(-1, -2) (source/batch.py:37-49): a (Th, Tw) tile comes out (Tw, Th)
+        out = torch.empty((B, C_, Tw, Th) if int(flip_index) & 4 else (B, C_, Th, Tw), dtype=raw.dtype, device=raw.device)
         mean = torch.empty(B, C_, 1, 1, dtype=torch.float32, device=raw.device)
         std = torch.empty_like(mean)
-        L.check(self.lib.sres_tiles_lnorm(L.ptr(raw), B * C_, T, int(flip_index), L.ptr(out), L.ptr(mean), L.ptr(std),
-                                          L.cur_stream()), "sres_tiles_lnorm")
+        L.check(self.lib.sres_tiles_lnorm_hw(L.ptr(raw), B * C_, Th, Tw, int(flip_index), L.ptr(out), L.ptr(mean), L.ptr(std),
+                                             L.cur_stream()), "sres_tiles_lnorm_hw")
         return TileArray(out, ["tiles", "channels", "y", "x"],
                          coords=dict(tiles=self.timeslice.coords["tiles"][tile_range[0]:tile_range[1]], channels=self.varnames),
                          attrs=dict(mean=mean, std=std, xyflip=int(flip_index)))

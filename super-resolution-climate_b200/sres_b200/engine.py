@@ -154,23 +154,36 @@ class RcanEngine:
         d.res_scale = self.res_scale
         return d
 
-    MAX_SHAPES = 4   # workspaces (and their CUDA graphs) kept per engine; the least recently used shape is dropped
+    MAX_SHAPES = 4   # shape entries (workspaces and their CUDA graphs) kept per engine; the least recently used is dropped
+
+    @staticmethod
+    def _shape_entry(key):
+        """(B, H, W, training) and (B, W, H, training) are one cache entry: with rectangular tiles and xyflip a training
+        epoch alternates between the two orientations, so they are kept and evicted together.  Each orientation still
+        has its own workspace (the never-written padding rows of the gradient buffers differ between them)."""
+        B, H, W, training = key
+        return (B, min(H, W), max(H, W), training)
 
     def _evict_shapes(self, keep):
-        """Ragged last batches and new inference shapes each need a multi-GB workspace: keep the MAX_SHAPES most recent."""
-        while len(self._ws) >= self.MAX_SHAPES:
-            old = next(k for k in self._ws if k != keep)
+        """Ragged last batches and new inference shapes each need a multi-GB workspace: keep the MAX_SHAPES most recent
+        shape entries."""
+        keep_entry = self._shape_entry(keep)
+        while len({self._shape_entry(k) for k in self._ws} | {keep_entry}) > self.MAX_SHAPES:
+            old_entry = next(self._shape_entry(k) for k in self._ws if self._shape_entry(k) != keep_entry)
             torch.cuda.synchronize(self.device)
-            for gk in [g for g in self._graphs if (g[1] == old if isinstance(g, tuple) and len(g) > 1 else False)]:
-                del self._graphs[gk]
-            del self._ws[old]
-            self._packed_version.pop(old, None)
+            for old in [k for k in self._ws if self._shape_entry(k) == old_entry]:
+                for gk in [g for g in self._graphs if (g[1] == old if isinstance(g, tuple) and len(g) > 1 else False)]:
+                    del self._graphs[gk]
+                del self._ws[old]
+                self._packed_version.pop(old, None)
 
     def workspace(self, B: int, H: int, W: int, training: bool) -> torch.Tensor:
         key = (B, H, W, training)
         ws = self._ws.get(key)
         if ws is not None:
-            self._ws[key] = self._ws.pop(key)   # most recently used last
+            # most recently used last, together with the other orientation of its shape entry
+            for k in [k for k in self._ws if self._shape_entry(k) == self._shape_entry(key)]:
+                self._ws[k] = self._ws.pop(k)
         if ws is None:
             self._evict_shapes(key)
             nbytes = C.c_size_t(0)
